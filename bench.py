@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BGZF compress & inflate GB/s (uncompressed) on B200, next to the reference's CPU path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--mib M] [--level L] [--kind fastq|sam]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--mib M] [--level L] [--kind fastq|sam] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...     (N > 1)
   python bench.py --impl reference ...      the reference's own CPU implementation (oracle/_ref), all host threads
   python bench.py --workload config3 [--gib 64] ...   BASELINE config 3: ONE 64 GiB SAM-like input, block ranges sharded over
@@ -17,6 +17,10 @@ reduction of the timing.
   inflate    the same two numbers for BGZF inflate of the stream just produced
   roofline   algorithmic bytes (payload read + stream written, SURVEY 8d) / device time, against the measured HBM peak
   cpu_baseline  the reference (oracle/_ref: the unmodified 7bgzf hook + libdeflate) on this box's host cores
+
+--dump-outputs DIR writes, after the timed steps, what the last step of each timed leg handed its caller (see
+dump_outputs).  The input is generated from a fixed seed, so two builds run with the same arguments can be compared
+output for output.
 """
 import argparse
 import ctypes
@@ -191,20 +195,68 @@ def container_lines(codec, h_in, n, h_out, h_back):
     return res
 
 
+DUMP_SAMPLE = 2 << 20          # bytes kept of each byte output; 4 of them as float32 plus the member sizes stay under 64 MB
+DUMP_WINDOW = 4096
+
+
+def member_sizes(stream):
+    """compressed size of every member of a BGZF stream, by walking BSIZE (the EOF block included)"""
+    sizes, off = [], 0
+    while off + 18 <= len(stream):
+        size = int(stream[off + 16]) + (int(stream[off + 17]) << 8) + 1
+        sizes.append(size)
+        off += size
+    assert off == len(stream), "the BSIZE chain does not end at the end of the stream"
+    return sizes
+
+
+def dump_outputs(path, outputs):
+    """Writes every (name, numpy array) as <path>/<name>.npy: byte arrays in float32, integer lists in float64.  A byte
+    array longer than DUMP_SAMPLE is reduced to DUMP_SAMPLE bytes: whole DUMP_WINDOW-byte windows at offsets drawn from a
+    fixed seed, in order, so that equal outputs give equal samples.  The bytes after the last whole window are not in the
+    sample; of the compressed stream, compress_member_bytes covers every member, the EOF block included."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in outputs:
+        if a.dtype == np.uint8:
+            if a.size > DUMP_SAMPLE:
+                rng = np.random.default_rng(0)
+                starts = np.sort(rng.choice(a.size // DUMP_WINDOW, DUMP_SAMPLE // DUMP_WINDOW, replace=False)) * DUMP_WINDOW
+                a = a[(starts[:, None] + np.arange(DUMP_WINDOW)).ravel()]
+            a = a.astype(np.float32)
+        else:
+            a = a.astype(np.float64)
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps of each leg (default: 5; config3: 1, each a pass over the whole input); "
+                                                            "the pageable-host legs run min(2, K) and report their own count; not for config5")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="config1", choices=["config1", "config3", "config5"])
     ap.add_argument("--mib", type=int, default=1024, help="payload MiB per rank (BASELINE: 1 GiB)")
-    ap.add_argument("--gib", type=int, default=64, help="config3: total GiB of the one sharded input (BASELINE: 64)")
+    ap.add_argument("--gib", type=int, default=None, help="config3: total GiB of the one sharded input (default 64, as BASELINE); "
+                                                           "config5: GiB streamed through the hook (default 16)")
     ap.add_argument("--level", type=int, default=6)
     ap.add_argument("--kind", default="fastq", choices=["fastq", "sam"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-containers", action="store_true", help="skip the extra lines for the other containers (SURVEY 8f)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the outputs of each timed leg's last step "
+                                                          "as DIR/<name>.npy (config1, --impl b200)")
     args = ap.parse_args()
+    if args.workload == "config5" and args.steps is not None:
+        ap.error("--steps is not for config5: it times one pass per caller count (three at 32 and 64 callers)")
+    if args.steps is None:
+        args.steps = 1 if args.workload == "config3" else 5
+    if args.gib is None:
+        args.gib = 16 if args.workload == "config5" else 64
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload != "config1" or args.impl != "b200"):
+        ap.error("--dump-outputs is for --workload config1 --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -344,6 +396,7 @@ def main():
             clen[0] = codec.compress_device(d_in.data_ptr(), nbytes, d_out.data_ptr(), bound, args.level, stream=stream.cuda_stream)
 
         t_dev, _, launches_c = run_timed(comp_dev, args.steps, args.warmup)
+        clen_dev = clen[0]
         # --- inflate, device resident (member index built on the device inside the timed call)
         def inf_dev():
             codec.inflate_device(d_out.data_ptr(), clen[0], d_back.data_ptr(), nbytes, stream=stream.cuda_stream)
@@ -354,6 +407,7 @@ def main():
             clen[0] = codec.compress_into(h_in.data_ptr(), nbytes, h_out.data_ptr(), bound, args.level)
 
         _, w_e2e, _ = run_timed(comp_e2e, args.steps, args.warmup)
+        clen_e2e = clen[0]
 
         def inf_e2e():
             codec.inflate_into(h_out.data_ptr(), clen[0], h_back.data_ptr(), nbytes)
@@ -382,6 +436,13 @@ def main():
         ok = ok and bool(np.array_equal(p_back, p_in))
         del p_in, p_out, p_back
 
+    if args.dump_outputs and rank == 0:
+        stream_dev = d_out[:clen_dev].cpu().numpy()
+        dump_outputs(args.dump_outputs, [("compress_stream", stream_dev),
+                                         ("compress_member_bytes", np.array(member_sizes(stream_dev))),
+                                         ("inflate_output", d_back.cpu().numpy()),
+                                         ("compress_e2e_stream", h_out.numpy()[:clen_e2e]),
+                                         ("inflate_e2e_output", h_back.numpy())])
     sha = hashlib.sha256(h_out.numpy()[: clen[0]]).hexdigest()          # the whole BGZF stream this rank produced (EOF included)
     shas = gather_strings(sha)
     steps = args.steps
@@ -449,7 +510,7 @@ def run_config5(args):
     by build/hook_mt (tools/hook_mt.c): N pthreads, each a synchronous bgzf_compress(dst, &dlen, src, <= 0xff00, level) call
     at a time over BAM-encoded records (tools/datagen.c kind 2: what htslib hands the hook when samtools writes BAM) —
     --gib GiB streamed as repeats of a 1 GiB buffer.  The same harness drives the reference's 7bgzf.so on the host cores."""
-    gib = args.gib if args.gib != 64 else 16
+    gib = args.gib
     path = "/dev/shm/b200bgzf_bam1g.bin"
     subprocess.run(f"{os.path.join(ROOT, 'build', 'datagen')} bam {1 << 30} 2 > {path}", shell=True, check=True)
     env = dict(os.environ, BGZF_METHOD=f"libdeflate{args.level}")
@@ -523,7 +584,7 @@ def run_config3(args, codec, gen, rank, local_rank, world, barrier, max_over_ran
     d_in = torch.empty(CH, dtype=torch.uint8, device="cuda")
     d_out = torch.empty(bound, dtype=torch.uint8, device="cuda")
     shard = np.empty(int(mine * 0.30) + (1 << 20), dtype=np.uint8)   # this rank's part of the stream (SAM-like text: ratio ~0.13)
-    steps = max(1, args.steps if args.steps != 5 else 1)              # default: one pass
+    steps = args.steps
     t_dev = t_e2e = 0.0
     launches = 0
     with ClockSampler(local_rank) as clk:

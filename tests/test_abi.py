@@ -1,10 +1,12 @@
 """CPU: the C-ABI boundary — the shared objects load, export exactly what include/b200bgzf.h declares (and
 nothing unprefixed besides bgzf_compress), and fail loudly without a GPU (no CPU fallback)."""
 import ctypes
+import glob
 import json
 import os
 import re
 import subprocess
+import sys
 
 import pytest
 
@@ -12,7 +14,7 @@ import b200bgzf
 import helpers as H
 
 ROOT = H.ROOT
-HAVE_GPU = os.path.exists("/dev/nvidia0")
+HAVE_GPU = bool(glob.glob("/dev/nvidia[0-9]*"))        # a machine may expose its GPU under any index, not only 0
 
 
 def _declared():
@@ -88,7 +90,7 @@ def test_no_cpu_fallback_without_gpu():
     code = ("import ctypes,sys; h=ctypes.CDLL(sys.argv[1]); d=ctypes.create_string_buffer(65536); n=ctypes.c_size_t(65536);"
             "h.bgzf_compress.argtypes=[ctypes.c_char_p,ctypes.POINTER(ctypes.c_size_t),ctypes.c_char_p,ctypes.c_size_t,ctypes.c_int];"
             "print(h.bgzf_compress(d,ctypes.byref(n),b'x'*1000,1000,6), n.value)")
-    r = subprocess.run(["python", "-c", code, b200bgzf.HOOK_PATH], capture_output=True, text=True, env=dict(os.environ, BGZF_METHOD="libdeflate6"))
+    r = subprocess.run([sys.executable, "-c", code, b200bgzf.HOOK_PATH], capture_output=True, text=True, env=dict(os.environ, BGZF_METHOD="libdeflate6"))
     assert r.stdout.split() == ["-1", "65536"]
 
 
