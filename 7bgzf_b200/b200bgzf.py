@@ -299,9 +299,9 @@ class Codec:
         self._check(self.lib.b200bgzf_inflate_device(self.h, d_in, nbytes, d_out, out_cap, ctypes.byref(n), flags, stream))
         return n.value
 
-    def profile(self, enable=True, reset=True):
-        arr = (ctypes.c_ulonglong * 32)()
-        self._check(self.lib.b200bgzf_profile(self.h, 1 if enable else 0, arr, 32, 1 if reset else 0))
+    def profile(self, enable=True, reset=True, slots=32):
+        arr = (ctypes.c_ulonglong * slots)()
+        self._check(self.lib.b200bgzf_profile(self.h, 1 if enable else 0, arr, slots, 1 if reset else 0))
         return list(arr)
 
     def launches(self):

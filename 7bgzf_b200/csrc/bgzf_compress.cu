@@ -85,13 +85,28 @@ __device__ __forceinline__ void fence_proxy_async()
 __device__ __forceinline__ unsigned hash_peers(uint32_t h, bool valid)
 {
     unsigned peers = __ballot_sync(0xffffffffu, valid);
+    /* per hash bit: the vote, the lane's bit as a mask (SEL) and peers &= ~(ballot ^ mask) in one LOP3; ptxas takes the
+     * predicates for 7 bits at a time from h with one R2P.  (Written in C, the same step compiles to six instructions.) */
 #pragma unroll
     for (int k = 0; k < BG_HASH_BITS; k++) {
-        const uint32_t bit = (h >> k) & 1u;
-        const unsigned b = __ballot_sync(0xffffffffu, bit != 0);
-        peers &= b ^ (bit - 1u);
+        asm volatile("{\n\t.reg .pred p;\n\t.reg .b32 b, t;\n\t"
+                     "and.b32 t, %1, %2;\n\t"
+                     "setp.ne.u32 p, t, 0;\n\t"
+                     "vote.sync.ballot.b32 b, p, 0xffffffff;\n\t"
+                     "selp.b32 t, -1, 0, p;\n\t"
+                     "lop3.b32 %0, %0, b, t, 0x90;\n\t}"
+                     : "+r"(peers)
+                     : "r"(h), "r"(1u << k));
     }
     return peers;
+}
+
+/* bg_hash for any window width without a branch: the second word contributes nothing for 3 and 4 bytes, its low byte for 5,
+ * all of it for 8 (the block is followed by zero bytes: the second word of a position near the end stays inside the buffer) */
+__device__ __forceinline__ uint32_t hash_any_width(const uint32_t *dataw, uint32_t p, uint32_t m0, uint32_t m1)
+{
+    const uint32_t v0 = bg_ld32(dataw, p) & m0, v1 = bg_ld32(dataw, p + 4u) & m1;
+    return ((v0 * 0x1E35A7BDu) ^ (v1 * 0x9E3779B1u)) >> (32 - BG_HASH_BITS);
 }
 
 /* notes layout: tile = 16 consecutive groups (512 positions); tile i holds 32 lanes x 16 bytes, so that in phase
@@ -102,9 +117,11 @@ __device__ __forceinline__ unsigned hash_peers(uint32_t h, bool valid)
  * ready (optional): one flag per tile in shared memory, raised when the tile's links and notes are out — the linking
  * relay (build_link_phase) runs at the same time on other warps and waits for it */
 __device__ __forceinline__ void build_peers_phase(const BgCtx &c, uint4 *notes, uint32_t lane, uint32_t warp, uint32_t nwarps, uint32_t first,
-                                                  uint32_t step, uint4 *xprev, volatile uint8_t *ready)
+                                                  uint32_t step, uint4 *xprev, volatile uint8_t *ready, unsigned long long *prof, long long t0)
 {
     const uint32_t n = c.n, hb = c.scal[BG_S_HBYTES];
+    const uint32_t m0 = hb == 3 ? 0xffffffu : 0xffffffffu, m1 = hb == 8 ? 0xffffffffu : hb == 5 ? 0xffu : 0u;
+    BG_ASSERT(hb == 3 || hb == 4 || hb == 5 || hb == 8);
     const unsigned lt = (1u << lane) - 1u;
     const uint32_t ntiles = (n + 511u) >> 9;
     for (uint32_t tile = first + step * warp; tile < ntiles; tile += step * nwarps) {
@@ -116,7 +133,7 @@ __device__ __forceinline__ void build_peers_phase(const BgCtx &c, uint4 *notes, 
             const uint32_t p = base + lane;
             /* (the hash phase proper is folded in: a position's hash goes straight from the multiply into the ballots) */
             const bool valid = p + hb <= n;
-            const uint32_t h = valid ? bg_hash(c.dataw, p, hb) : BG_NOPOS;
+            const uint32_t h = valid ? hash_any_width(c.dataw, p, m0, m1) : BG_NOPOS;
             const unsigned peers = hash_peers(h, valid);
             uint32_t link = h;                                            /* a leader keeps its hash for the relay; no hash window: BG_NOPOS */
             if (valid) {
@@ -141,6 +158,7 @@ __device__ __forceinline__ void build_peers_phase(const BgCtx &c, uint4 *notes, 
             __threadfence_block();
             __syncwarp();
             if (lane == 0) ready[tile] = 1;
+            if (prof && lane == 0) atomicAdd(&prof[BGZF_PROF_READY + tile], (unsigned long long)(clock64() - t0));
         }
     }
 }
@@ -158,47 +176,73 @@ __device__ __forceinline__ void import_peer_tiles(const BgCtx &c, const uint4 *x
  * must run in tile order (and inside it, group order: shared-memory instructions of one warp execute in program order,
  * the accesses are volatile so the compiler keeps that order); it is entered when the `turn` word in shared memory
  * reaches the tile and hands the turn on as soon as its last head update is out.  Fetching the notes and the
- * leaders' hashes before, and storing the links after, overlap with the other warps' turns.  head[] reads and
- * writes go out back to back; the links they return are parked in registers until the turn has been passed on. */
+ * leaders' hashes before, and storing the links after, overlap with the other warps' turns.
+ * The ordered section was the critical path of the chain build (profiles/r03_link_split.txt: the relay handed on its
+ * last turn 28 k cycles after the last producer was done) and it competes for issue slots with 28 producer warps, so it
+ * is kept to three instructions per group: every access is prepared before the turn as one word, head byte offset << 16 |
+ * new head, and lanes without a leader go to a sink word instead of being predicated.  The turn is handed on with a
+ * release store and taken with an acquire load (one MEMBAR.ALL.CTA by the passing lane instead of two MEMBAR.SC.CTA
+ * per lane). */
 #define BG_LINKERS 4u
+#define BG_LINK_SINK (SM_SCAN + 4u * 33u - SM_REGB)   /* byte offset from head[] of a u16 nobody reads (scan scratch word 33) */
+__device__ __forceinline__ uint32_t ld_acquire_cta(const volatile uint32_t *p)
+{
+    uint32_t v;
+    asm volatile("ld.acquire.cta.shared::cta.u32 %0, [%1];" : "=r"(v) : "r"(smem_u32((const void *)p)) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_release_cta(volatile uint32_t *p, uint32_t v)
+{
+    asm volatile("st.release.cta.shared::cta.u32 [%0], %1;" ::"r"(smem_u32((const void *)p)), "r"(v) : "memory");
+}
+/* prof (optional): cycles since t0 at which each tile's turn is taken; the relay's waits on ready[] and on `turn` */
 __device__ __forceinline__ void build_link_phase(const BgCtx &c, const uint4 *notes, uint32_t warp, uint32_t lane, volatile uint32_t *turn,
-                                                 volatile uint8_t *ready)
+                                                 volatile uint8_t *ready, unsigned long long *prof, long long t0)
 {
     const uint32_t n = c.n;
     const uint32_t ntiles = (n + 511u) >> 9;
-    volatile uint16_t *vhead = c.head;
+    volatile uint8_t *vhead = (volatile uint8_t *)c.head;
+    static_assert(BG_LINK_SINK >= 2u * BG_HASH_SIZE && BG_LINK_SINK < 65536u, "the sink lies outside head[] and within 16 bits");
     for (uint32_t tile = warp; tile < ntiles; tile += BG_LINKERS) {
+        BG_ASSERT(tile < 128u);
+        const long long w0 = prof ? clock64() : 0;
         if (ready) {
             while (!ready[tile]) __nanosleep(40);
             __threadfence_block();
         }
+        const long long w1 = prof ? clock64() : 0;
         const uint4 cur = __ldcg(notes + tile * 32u + lane);
         const uint32_t w[4] = { cur.x, cur.y, cur.z, cur.w };
         /* the hash slots of this tile's leaders are untouched until their links are stored below: fetch them all now */
-        uint32_t hs[16];
+        uint32_t op[16];
 #pragma unroll
         for (uint32_t g = 0; g < 16; g++) {
             const uint32_t note = (w[g >> 2] >> (8 * (g & 3))) & 0xffu;
-            hs[g] = note != 0xffu ? (uint32_t)c.prev[tile * 512u + g * 32u + lane] : 0xffffffffu;
+            const uint32_t h = c.prev[tile * 512u + g * 32u + lane];
+            BG_ASSERT(note == 0xffu || h < BG_HASH_SIZE);
+            op[g] = note != 0xffu ? (h << 17) | (tile * 512u + g * 32u + note) : BG_LINK_SINK << 16;
         }
-        while (*turn != tile) {}
-        __threadfence_block();
-        uint16_t old[16];
+        const long long w2 = prof ? clock64() : 0;
+        while (ld_acquire_cta(turn) != tile) {}
+        const long long w3 = prof ? clock64() : 0;
+        uint32_t old[16];
 #pragma unroll
         for (uint32_t g = 0; g < 16; g++) {
-            const uint32_t h = hs[g];
-            if (h != 0xffffffffu) {
-                const uint32_t note = (w[g >> 2] >> (8 * (g & 3))) & 31u;
-                old[g] = vhead[h];
-                vhead[h] = (uint16_t)(tile * 512u + g * 32u + note);
-            }
+            volatile uint16_t *slot = (volatile uint16_t *)(vhead + (op[g] >> 16));
+            old[g] = *slot;
+            *slot = (uint16_t)op[g];
         }
-        __threadfence_block();
         __syncwarp();
-        if (lane == 0) *turn = tile + 1;
+        if (lane == 0) st_release_cta(turn, tile + 1);
+        if (prof && lane == 0) {
+            atomicAdd(&prof[23], (unsigned long long)(w1 - w0));
+            atomicAdd(&prof[24], (unsigned long long)(w3 - w2));
+            atomicAdd(&prof[BGZF_PROF_TURN + tile], (unsigned long long)(w3 - t0));
+            if (tile + 1 == ntiles) atomicAdd(&prof[25], (unsigned long long)(clock64() - t0));
+        }
 #pragma unroll
         for (uint32_t g = 0; g < 16; g++)
-            if (hs[g] != 0xffffffffu) c.prev[tile * 512u + g * 32u + lane] = old[g];
+            if ((op[g] >> 16) != BG_LINK_SINK) c.prev[tile * 512u + g * 32u + lane] = (uint16_t)old[g];
     }
 }
 
@@ -813,6 +857,7 @@ __device__ __forceinline__ void compress_blocks(BgzfCompressArgs &a)
     uint32_t *scan_scratch = (uint32_t *)(smem + SM_SCAN);
     unsigned long long *prof = a.prof;
     long long tprev_ = prof ? clock64() : 0;
+    uint32_t *const pscr = scan_scratch;                  /* profiling only: last producer, slowest / fastest pass-1 warp */
 
     BgCtx c;
     c.dataw = (uint32_t *)(smem + SM_DATA);
@@ -906,20 +951,26 @@ __device__ __forceinline__ void compress_blocks(BgzfCompressArgs &a)
         if (SPLIT) {
             /* every CTA has the same hashes; each finds the peers of its share of the tiles, the links travel through L2 */
             uint4 *xprev = (uint4 *)(unit_scratch + BGZF_SCRATCH_WORDS);
-            build_peers_phase(c, hi, t & 31u, t >> 5, BG_THREADS / 32u, crank, csize, xprev, nullptr);
+            build_peers_phase(c, hi, t & 31u, t >> 5, BG_THREADS / 32u, crank, csize, xprev, nullptr, nullptr, 0);
             cluster_sync();
             import_peer_tiles(c, xprev, t, crank, csize);
             __syncthreads();
             PROF_MARK(3);
-            if (t < 32u * BG_LINKERS) build_link_phase(c, hi, t >> 5, t & 31u, &c.scal[BG_S_WLIST], nullptr);   /* the other warps wait at the barrier */
+            if (t < 32u * BG_LINKERS) build_link_phase(c, hi, t >> 5, t & 31u, &c.scal[BG_S_WLIST], nullptr, nullptr, 0);   /* the other warps wait at the barrier */
         } else {
             /* peers and links at the same time: warps 0..3 are the linking relay, the other 28 find the peers tile by tile
              * and raise a flag per tile; the relay's ordered head-table section hides behind the ballots of the producers */
             volatile uint8_t *ready = (volatile uint8_t *)(smem + SM_READY);
             if (t < 128u) ready[t] = 0;
+            if (prof && t == 0) { pscr[0] = 0; pscr[1] = 0; pscr[2] = 0xffffffffu; }
             __syncthreads();
-            if (t < 32u * BG_LINKERS) build_link_phase(c, hi, t >> 5, t & 31u, &c.scal[BG_S_WLIST], ready);
-            else build_peers_phase(c, hi, t & 31u, (t >> 5) - BG_LINKERS, BG_THREADS / 32u - BG_LINKERS, 0u, 1u, nullptr, ready);
+            const long long t0 = prof ? clock64() : 0;
+            if (t < 32u * BG_LINKERS) {
+                build_link_phase(c, hi, t >> 5, t & 31u, &c.scal[BG_S_WLIST], ready, prof, t0);
+            } else {
+                build_peers_phase(c, hi, t & 31u, (t >> 5) - BG_LINKERS, BG_THREADS / 32u - BG_LINKERS, 0u, 1u, nullptr, ready, prof, t0);
+                if (prof && (t & 31u) == 0) atomicMax(&pscr[0], (uint32_t)(clock64() - t0));
+            }
         }
         __syncthreads();
         PROF_MARK(10);
@@ -927,9 +978,20 @@ __device__ __forceinline__ void compress_blocks(BgzfCompressArgs &a)
             bg_phase_search_clear(c, t, T);
             if (SPLIT) cluster_sync();                           /* every CTA's bitmap is clear before anyone's marks arrive */
             else __syncthreads();
+            const long long t1 = prof ? clock64() : 0;
             search_nearest<SPLIT>(c, t, crank, csize);
+            if (!SPLIT && prof && (t & 31u) == 0) {              /* pass 1: when the slowest and the fastest warp finish */
+                const uint32_t d = (uint32_t)(clock64() - t1);
+                atomicMax(&pscr[1], d);
+                atomicMin(&pscr[2], d);
+            }
             if (SPLIT) cluster_sync();                           /* ... and complete before it is read */
             else __syncthreads();
+            if (!SPLIT && prof && t == 0) {
+                atomicAdd(&prof[22], (unsigned long long)pscr[0]);
+                atomicAdd(&prof[26], (unsigned long long)pscr[1]);
+                atomicAdd(&prof[27], (unsigned long long)pscr[2]);
+            }
             PROF_MARK(21);
             if (c.scal[BG_S_DEPTH] > 1) {                        /* (uniform for the CTA) */
                 bg_phase_search_todo(c, t, T, crank, csize);

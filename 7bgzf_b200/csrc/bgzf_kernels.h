@@ -9,7 +9,9 @@
 #define BGZF_SCRATCH_WORDS (65536u + 32u + 16384u + 32u)   /* per-CTA scratch: u32 match per position + u8 build notes */
 #define BGZF_SPLIT_EXTRA_WORDS 32768u                       /* split launch: the chain links of every tile, exchanged between the CTAs */
 #define BGZF_SPLIT_MAX 8                                    /* largest cluster bgzf_launch_compress_split takes */
-#define BGZF_PROF_SLOTS 32
+#define BGZF_PROF_SLOTS 288                                 /* 32 phase counters, then per tile of the chain build: relay turn, ready flag */
+#define BGZF_PROF_TURN 32
+#define BGZF_PROF_READY 160
 
 struct BgzfCompressArgs {
     const uint8_t *in;         /* device: payload bytes */

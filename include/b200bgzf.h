@@ -244,7 +244,8 @@ int b200bgzf_container_inflate_size(int kind, const void *in, size_t in_bytes, s
 void *b200bgzf_host_alloc(size_t bytes);
 void b200bgzf_host_free(void *p);
 
-/* Per-phase cycle counters of the compress kernel (development aid; n <= 16). Resets them when reset != 0. */
+/* Per-phase cycle counters of the compress kernel (development aid; n <= 288: 32 phase counters, then per-tile
+ * timings of the chain build, see tools/link_split.py). Resets them when reset != 0. */
 int b200bgzf_profile(b200bgzf_ctx *ctx, int enable, unsigned long long *cycles, int n, int reset);
 /* number of kernel launches issued by this context so far */
 unsigned long long b200bgzf_launch_count(const b200bgzf_ctx *ctx);
