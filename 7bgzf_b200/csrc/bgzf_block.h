@@ -6,7 +6,7 @@
  * the phases with t = threadIdx.x and a __syncthreads() between them, and the development emulator
  * (tests/model/emul.cpp) calls the very same functions in a loop over t — in forward, reverse and shuffled
  * order, which doubles as a race detector: a phase may only read what an earlier phase wrote.
- * Warp-collective pieces (chain build with __match_any_sync, bitonic sort, block scan, TMA load) live in the
+ * Warp-collective pieces (chain build, litlen key ranking, block scan, TMA load) live in the
  * .cu file and have plain sequential twins in the emulator; their results are order-independent by
  * construction, so GPU output == emulator output, byte for byte.
  *
@@ -318,40 +318,66 @@ BG_HD void bg_phase_init(const BgCtx &c, uint32_t t, uint32_t T)
         c.scal[t] = 0;
 }
 
-/* phase 1: which literals occur (benign same-value stores) + CRC slice per thread */
-BG_HD void bg_phase_scan(const BgCtx &c, uint32_t t, uint32_t T)
+/* phase 1a: which literals occur (benign same-value stores) */
+BG_HD void bg_phase_census(const BgCtx &c, uint32_t t, uint32_t T)
 {
-    const uint32_t n = c.n;
-    for (uint32_t p = t; p < n; p += T)
+    for (uint32_t p = t; p < c.n; p += T)
         c.litflag[bg_ld8(c.dataw, p)] = 1;
-    /* CRC over the first m = n/4 words (of the payload: hw history words come first), slices right-aligned so the combine
-     * exponents are constants */
+}
+
+/* CRC over the first m = n/4 words of the payload (hw history words come first), cut into BG_THREADS slices of BG_CRC_WORDS
+ * words, right-aligned: slice k ends k slices before word m, so its combine factor is the constant crcpow[k].  Thread u of
+ * U takes slices u, u + U, u + 2U, ...: two at a time, as two independent lookup chains.  Each thread's share is XORed into
+ * scal[BG_S_CRC], which must start at 0; bg_crc_finish() adds the ragged tail once every share is in. */
+BG_HD void bg_crc_slices(const BgCtx &c, uint32_t u, uint32_t U)
+{
     const uint32_t hw = bg_f_hist(c) >> 2;
-    const uint32_t m = (n >> 2) - hw;
-    const uint32_t k = T - 1 - t;                 /* slices after mine */
-    const uint32_t endw = m >= BG_CRC_WORDS * k ? m - BG_CRC_WORDS * k : 0;
-    const uint32_t begw = endw >= BG_CRC_WORDS ? endw - BG_CRC_WORDS : 0;
-    uint32_t r = 0;
-    if (endw > begw) {
-        r = begw == 0 ? 0xFFFFFFFFu : 0u;
-        for (uint32_t w = begw; w < endw; w++) {
-            uint32_t v = c.dataw[hw + w];
-            r = bg_crc_byte(c.crctab, r, v & 0xff);
-            r = bg_crc_byte(c.crctab, r, (v >> 8) & 0xff);
-            r = bg_crc_byte(c.crctab, r, (v >> 16) & 0xff);
-            r = bg_crc_byte(c.crctab, r, v >> 24);
+    const uint32_t m = (c.n >> 2) - hw;
+    const uint32_t *d = c.dataw + hw;
+    uint32_t acc = 0;
+    for (uint32_t k0 = u; k0 < BG_THREADS; k0 += 2 * U) {
+        const uint32_t k1 = k0 + U;                                   /* (k1 >= BG_THREADS: an empty slice) */
+        const uint32_t e0 = m >= BG_CRC_WORDS * k0 ? m - BG_CRC_WORDS * k0 : 0;
+        const uint32_t e1 = k1 < BG_THREADS && m >= BG_CRC_WORDS * k1 ? m - BG_CRC_WORDS * k1 : 0;
+        const uint32_t b0 = e0 >= BG_CRC_WORDS ? e0 - BG_CRC_WORDS : 0, b1 = e1 >= BG_CRC_WORDS ? e1 - BG_CRC_WORDS : 0;
+        if (e0 == b0) break;                                          /* (slices further left are empty too) */
+        uint32_t r0 = b0 == 0 ? 0xFFFFFFFFu : 0u, r1 = b1 == 0 ? 0xFFFFFFFFu : 0u;
+        for (uint32_t i = 0; i < BG_CRC_WORDS; i++) {
+            if (b0 + i < e0) {
+                const uint32_t v = d[b0 + i];
+                r0 = bg_crc_byte(c.crctab, r0, v & 0xff);
+                r0 = bg_crc_byte(c.crctab, r0, (v >> 8) & 0xff);
+                r0 = bg_crc_byte(c.crctab, r0, (v >> 16) & 0xff);
+                r0 = bg_crc_byte(c.crctab, r0, v >> 24);
+            }
+            if (b1 + i < e1) {
+                const uint32_t v = d[b1 + i];
+                r1 = bg_crc_byte(c.crctab, r1, v & 0xff);
+                r1 = bg_crc_byte(c.crctab, r1, (v >> 8) & 0xff);
+                r1 = bg_crc_byte(c.crctab, r1, (v >> 16) & 0xff);
+                r1 = bg_crc_byte(c.crctab, r1, v >> 24);
+            }
         }
-        r = bg_crc_mul(r, c.crcpow[k]);
+        acc ^= bg_crc_mul(r0, c.crcpow[k0]);
+        if (e1 > b1) acc ^= bg_crc_mul(r1, c.crcpow[k1]);
     }
     /* XOR is order-independent: fold inside the warp, then one shared atomic per warp */
 #if defined(__CUDA_ARCH__)
-    for (int d = 16; d > 0; d >>= 1)
-        r ^= __shfl_xor_sync(0xffffffffu, r, d);
-    if ((t & 31u) == 0 && r)
-        atomicXor(&c.scal[BG_S_CRC], r);
+    for (int s = 16; s > 0; s >>= 1)
+        acc ^= __shfl_xor_sync(0xffffffffu, acc, s);
+    if ((u & 31u) == 0 && acc)
+        atomicXor(&c.scal[BG_S_CRC], acc);
 #else
-    c.scal[BG_S_CRC] ^= r;
+    c.scal[BG_S_CRC] ^= acc;
 #endif
+}
+
+/* phase 1: census and CRC slices, one slice per thread (the kernel runs the two apart: the census feeds the search, the
+ * CRC is read only by the trailer) */
+BG_HD void bg_phase_scan(const BgCtx &c, uint32_t t, uint32_t T)
+{
+    bg_phase_census(c, t, T);
+    bg_crc_slices(c, t, T);
 }
 
 /* phase 2: distinct-literal count (t < 256) */
@@ -377,17 +403,23 @@ BG_HD uint32_t bg_min_match_len(uint32_t nused, int depth, uint32_t n)
     return ml;
 }
 
-/* phase 3: finish CRC (thread 0), settle minlen/hash width (thread 0) */
-BG_HD void bg_phase_settle(const BgCtx &c, uint32_t t, uint32_t T)
+/* one thread, after every bg_crc_slices() share is in: the ragged tail bytes and the final complement */
+BG_HD void bg_crc_finish(const BgCtx &c)
 {
-    (void)T;
-    if (t != 0) return;
     const uint32_t n = c.n;
     uint32_t r = c.scal[BG_S_CRC];
     if (((n - bg_f_hist(c)) >> 2) == 0) r = 0xFFFFFFFFu;
     for (uint32_t p = n & ~3u; p < n; p++)
         r = bg_crc_byte(c.crctab, r, bg_ld8(c.dataw, p));
     c.scal[BG_S_CRC] = ~r;
+}
+
+/* phase 3a (thread 0): minlen, chain depth and hash width from the literal census */
+BG_HD void bg_phase_settle_census(const BgCtx &c, uint32_t t, uint32_t T)
+{
+    (void)T;
+    if (t != 0) return;
+    const uint32_t n = c.n;
     c.scal[BG_S_MINLEN] = bg_min_match_len(c.scal[BG_S_NUSED], c.prm.depth, n);
     /* binary-looking blocks (BAM records, executables: 80+ distinct byte values) get half as much chain depth again:
      * their matches are spread over more candidates than those of text, and the fixed depth that reaches the
@@ -401,6 +433,13 @@ BG_HD void bg_phase_settle(const BgCtx &c, uint32_t t, uint32_t T)
      * reaches every node a 4-byte window would have chained.  Measured at level 6: an ELF binary -3.0 % (it was 4 % behind
      * the reference), BAM-like records +-0.0 %; shallower walks (levels 2-5) lose on BAM-like data (+0.7 % at level 3): not done there. */
     if (c.scal[BG_S_MINLEN] == 3 && c.prm.depth >= 8) c.scal[BG_S_HBYTES] = 3;
+}
+
+/* phase 3 (thread 0): finish the CRC, settle minlen/hash width */
+BG_HD void bg_phase_settle(const BgCtx &c, uint32_t t, uint32_t T)
+{
+    if (t == 0) bg_crc_finish(c);
+    bg_phase_settle_census(c, t, T);
 }
 
 /* phase 4: hash every position that has a full hash window into prev[] */

@@ -9,7 +9,7 @@
  *       4. all-position chain search, 1024 positions at a time, results to an L2-resident scratch
  *          (levels 10-12: up to four matches per position, then min-cost-path passes, one warp per 1/32 of the block)
  *       5. local lazy rule -> step codes, per-chunk jump table, chunk-to-chunk walk
- *       6. histograms, length-limited Huffman (bitonic sort, two-queue merge, parallel depths), block type choice
+ *       6. histograms, length-limited Huffman (keys ranked by comparison, two-queue merge, parallel depths), block type choice
  *       7. per-chunk bit sizes, block-wide prefix sums, parallel bit packing, BGZF header/BSIZE/CRC/ISIZE
  *   bgzf_scan_kernel / bgzf_gather_kernel : exclusive scan of member sizes and compaction of the
  *       fixed-stride slots into one contiguous BGZF stream (+ the 28-byte EOF marker).
@@ -744,22 +744,136 @@ __device__ __forceinline__ void chunk_order_place(const BgCtx &c, uint32_t t, ui
     ((uint16_t *)(c.regb + BG_B_PERM))[cnt[cls * 32u + (t >> 5)] + rank] = (uint16_t)t;
 }
 
-/* ---- 512-key bitonic sort in shared memory (ascending); all threads call it ---- */
-__device__ __forceinline__ void bitonic_sort_512(uint32_t *keys, uint32_t t)
+/* ---- the litlen code's sort keys, ranked instead of sorted (the emulator's bg_phase_lkeys + std::sort + bg_phase_huff_prep).
+ * Keys (freq << 9 | sym) are distinct, so a used symbol's place in the ascending order is the number of smaller keys: each
+ * of threads 0..287 counts them over all 288 keys, 4 per broadcast load, with no block barrier in between.  Only the m used
+ * keys are placed (keys[m..) are never read).  Step 1 writes every symbol's key, ~0 for an unused one, to the parent-link
+ * array, which the tree merge fills only later. ---- */
+#define BG_B_RANKKEYS BG_B_TREEP         /* u32[288] (16-byte aligned) */
+
+__device__ __forceinline__ void litlen_keys(const BgCtx &c, uint32_t t)
 {
-    for (uint32_t k = 2; k <= 512; k <<= 1) {
-        for (uint32_t j = k >> 1; j > 0; j >>= 1) {
-            if (t < 512) {
-                uint32_t x = t ^ j;
-                if (x > t) {
-                    uint32_t a = keys[t], b = keys[x];
-                    bool up = (t & k) == 0;
-                    if ((a > b) == up) { keys[t] = b; keys[x] = a; }
-                }
+    const uint32_t *lfreq = (const uint32_t *)(c.regb + BG_B_LFREQ);
+    if (t < 288) {
+        const uint32_t f = lfreq[t];
+        ((uint32_t *)(c.regb + BG_B_RANKKEYS))[t] = f ? (f << 9) | t : 0xFFFFFFFFu;
+        if (f) atomicAdd(&c.scal[BG_S_HM], 1u);
+    }
+}
+
+/* step 2: place keys and leaf weights; what bg_phase_huff_prep clears; the distance alphabet's keys on the next warp */
+__device__ __forceinline__ void litlen_rank(const BgCtx &c, uint32_t t)
+{
+    uint8_t *rb = c.regb;
+    if (t < 288) {
+        const uint4 *all = (const uint4 *)(rb + BG_B_RANKKEYS);
+        const uint32_t k = ((const uint32_t *)all)[t];
+        rb[BG_B_LLEN + t] = 0;
+        if (k != 0xFFFFFFFFu) {
+            uint32_t rank = 0;
+#pragma unroll 8
+            for (uint32_t j = 0; j < 72; j++) {
+                const uint4 q = all[j];
+                rank += (q.x < k) + (q.y < k) + (q.z < k) + (q.w < k);
             }
-            __syncthreads();
+            ((uint32_t *)(rb + BG_B_KEYS))[rank] = k;
+            ((uint32_t *)(rb + BG_B_TREEW))[rank] = k >> 9;
+        }
+    } else if (t < 288 + 30) {
+        if (bg_rank_key((const uint32_t *)(rb + BG_B_DFREQ), 30, t - 288, (uint32_t *)(rb + BG_B_DKEYS))) atomicAdd(&c.scal[BG_S_DM], 1u);
+    } else if (t < 288 + 32 + 16) {
+        ((uint32_t *)(rb + BG_B_BLC))[t - 320] = 0;
+        if (t == 320) c.scal[BG_S_HOVF] = 0;
+    }
+}
+
+/* ---- a small alphabet's code lengths on one warp: bg_huff_lengths() split as for litlen (one lane merges, the warp takes
+ * the depths, lane 0 repairs the overflow, the warp assigns the lengths), handed on with __syncwarp().  Same lengths: a node
+ * deeper than maxbits counts as one overflow here as it does in the sequential depth pass.  keys: m ascending keys (m <= 32);
+ * w, par: 2m node slots; blc: u32[16]; lens[0..nzero) is cleared first.  All 32 lanes call it. ---- */
+__device__ __forceinline__ void warp_huff_lengths(const uint32_t *keys, uint32_t m, uint32_t maxbits, uint32_t nzero, uint32_t *w,
+                                                  uint16_t *par, uint32_t *blc, uint8_t *lens, uint32_t lane)
+{
+    if (lane < nzero) lens[lane] = 0;
+    if (lane < m) w[lane] = keys[lane] >> 9;
+    if (lane < 16) blc[lane] = 0;
+    __syncwarp();
+    if (m < 2) {                                                      /* (m is the same on every lane) */
+        if (lane == 0) {
+            const uint32_t s = m ? keys[0] & 511u : 0u;
+            lens[s] = 1;
+            lens[s ? 0 : 1] = 1;
+        }
+        return;
+    }
+    if (lane == 0) bg_huff_merge(m, w, par);
+    __syncwarp();
+    const uint32_t root = 2 * m - 2;
+    uint32_t ovf = 0;
+    for (uint32_t i = lane; i < root; i += 32) {
+        uint32_t d = 0;
+        for (uint32_t x = i; x != root && d < 64; x = par[x]) d++;
+        if (d > maxbits) { d = maxbits; ovf++; }
+        if (i < m) atomicAdd(&blc[d], 1u);
+    }
+    int overflow = (int)__reduce_add_sync(0xffffffffu, ovf);
+    __syncwarp();
+    if (lane == 0) {
+        while (overflow > 0) {
+            uint32_t bits = maxbits - 1;
+            while (bits > 1 && blc[bits] == 0) bits--;
+            blc[bits]--;
+            blc[bits + 1] += 2;
+            blc[maxbits]--;
+            overflow -= 2;
         }
     }
+    __syncwarp();
+    for (uint32_t i = lane; i < m; i += 32) {
+        uint32_t bits = maxbits, cum = blc[maxbits];
+        while (cum <= i && bits > 1) cum += blc[--bits];
+        lens[keys[i] & 511u] = (uint8_t)bits;
+    }
+}
+
+/* the distance code on warp 1 (the slots bg_phase_huff's thread 32 uses) */
+__device__ __forceinline__ void dist_tree_warp(const BgCtx &c, uint32_t lane)
+{
+    uint8_t *rb = c.regb;
+    warp_huff_lengths((const uint32_t *)(rb + BG_B_DKEYS), c.scal[BG_S_DM], 15, 32, (uint32_t *)(rb + BG_B_DTREEW),
+                      (uint16_t *)(rb + BG_B_DTREEP), (uint32_t *)(rb + BG_B_SCRATCH) + 32, rb + BG_B_DLEN, lane);
+}
+
+/* bg_phase_hdr5 on warp 0: the precode lengths on the warp, then HCLEN by a ballot and the header bit count by a sum */
+__device__ __forceinline__ void precode_hdr_warp(const BgCtx &c, uint32_t lane, uint32_t nitems)
+{
+    uint8_t *rb = c.regb;
+    uint32_t nl, nd;
+    bg_hdr_dims(c, &nl, &nd);
+    const uint32_t *pfreq = (const uint32_t *)(rb + BG_B_PFREQ);
+    uint8_t *plen = rb + BG_B_PLEN;
+    warp_huff_lengths((const uint32_t *)(rb + BG_B_PKEYS), c.scal[BG_S_PM], 7, 19, (uint32_t *)(rb + BG_B_DTREEW),
+                      (uint16_t *)(rb + BG_B_DTREEP), (uint32_t *)(rb + BG_B_SCRATCH) + 16, plen, lane);
+    __syncwarp();
+    const unsigned used = __ballot_sync(0xffffffffu, lane < 19 && plen[bg_precode_order(lane)] != 0);
+    uint32_t np = used ? 32u - (uint32_t)__clz(used) : 0u;            /* one past the last length HCLEN must carry, at least 4 */
+    if (np < 4) np = 4;
+    const uint32_t bits = lane < 19 ? pfreq[lane] * (plen[lane] + (lane == 16 ? 2u : lane == 17 ? 3u : lane == 18 ? 7u : 0u)) : 0u;
+    const uint32_t hdr = 3 + 5 + 5 + 4 + 3 * np + __reduce_add_sync(0xffffffffu, bits);
+    if (lane == 0) {
+        c.scal[BG_S_DYNHDR] = hdr;
+        c.scal[BG_S_NITEMS] = nitems;
+        c.scal[BG_S_NL] = nl;
+        c.scal[BG_S_ND] = nd;
+        c.scal[BG_S_NP] = np;
+    }
+}
+
+/* ---- named barrier of the tree warps (warps 0 .. BG_TREE_WARPS-1): the other warps run the CRC slices meanwhile ---- */
+#define BG_TREE_WARPS 4u
+__device__ __forceinline__ void tree_bar()
+{
+    asm volatile("bar.sync 1, %0;" :: "n"(BG_TREE_WARPS * 32) : "memory");
 }
 
 /* ---- exclusive prefix sum over 1024 u32 in shared memory; returns the grand total ---- */
@@ -939,11 +1053,13 @@ __device__ __forceinline__ void compress_blocks(BgzfCompressArgs &a)
         __syncthreads();
         PROF_MARK(0);
 
-        bg_phase_scan(c, t, T);
+        /* the literal census steers the search; the CRC is needed only by the trailer and runs on the warps the Huffman
+         * trees leave idle (below) */
+        bg_phase_census(c, t, T);
         __syncthreads();
         bg_phase_count(c, t, T);
         __syncthreads();
-        bg_phase_settle(c, t, T);
+        bg_phase_settle_census(c, t, T);
         __syncthreads();
         PROF_MARK(1);
         PROF_MARK(2);
@@ -1054,23 +1170,36 @@ __device__ __forceinline__ void compress_blocks(BgzfCompressArgs &a)
             PROF_MARK(6);
             bg_phase_tally(c, t, T);
             __syncthreads();
-            bg_phase_lkeys(c, t, T);
-            __syncthreads();
             PROF_MARK(7);
-            bitonic_sort_512((uint32_t *)(c.regb + BG_B_KEYS), t);
+            litlen_keys(c, t);
+            if (prof && t == 0) { pscr[3] = 0; pscr[4] = 0; }
+            __syncthreads();
+            litlen_rank(c, t);
+            __syncthreads();
             PROF_MARK(11);
-            bg_phase_huff_prep(c, t, T);
+            /* the trees on warps 0..3 (thread 0 merges the litlen tree, thread 32 builds the distance code), the CRC slices
+             * on the other 28 warps, once per block; everyone meets at the barrier after the trees */
+            const long long t2 = prof ? clock64() : 0;
+            if (t < 32u * BG_TREE_WARPS) {
+                const uint32_t TT = 32u * BG_TREE_WARPS;
+                if (t < 32u) bg_phase_huff(c, t, TT);                /* (thread 0: the litlen merge) */
+                else if (t < 64u) dist_tree_warp(c, t - 32u);
+                tree_bar();
+                bg_phase_huff_depth(c, t, TT);
+                tree_bar();
+                bg_phase_huff_fix(c, t, TT);
+                tree_bar();
+                bg_phase_huff_assign(c, t, TT);
+                if (prof && pass == 0 && (t & 31u) == 0) atomicMax(&pscr[3], (uint32_t)(clock64() - t2));
+            } else if (pass == 0) {
+                bg_crc_slices(c, t - 32u * BG_TREE_WARPS, T - 32u * BG_TREE_WARPS);
+                if (prof && (t & 31u) == 0) atomicMax(&pscr[4], (uint32_t)(clock64() - t2));
+            }
             __syncthreads();
-            bg_phase_huff(c, t, T);
-            __syncthreads();
-            bg_phase_huff_depth(c, t, T);
-            __syncthreads();
-            bg_phase_huff_fix(c, t, T);
-            __syncthreads();
-            bg_phase_huff_assign(c, t, T);
-            __syncthreads();
+            if (prof && pass == 0 && t == 0 && pscr[4] > pscr[3]) atomicAdd(&prof[28], (unsigned long long)(pscr[4] - pscr[3]));
             PROF_MARK(12);
         }
+        if (t == 0) bg_crc_finish(c);                            /* (every slice is in; the trailer is written by the emit) */
         bg_phase_hdr1(c, t, T);
         __syncthreads();
         bg_phase_hdr2(c, t, T);
@@ -1080,9 +1209,11 @@ __device__ __forceinline__ void compress_blocks(BgzfCompressArgs &a)
         const uint32_t nitems = block_exclusive_scan_1024((uint32_t *)(c.regb + BG_B_CBITS), scan_scratch, t);
         bg_phase_hdr4(c, t, T);
         __syncthreads();
-        bg_phase_hdr4b(c, t, T);
-        __syncthreads();
-        bg_phase_hdr5(c, t, T, nitems);
+        if (t < 32u) {                                           /* the precode keys and lengths are warp 0's work */
+            bg_phase_hdr4b(c, t, 32u);
+            __syncwarp();
+            precode_hdr_warp(c, t, nitems);
+        }
         __syncthreads();
         PROF_MARK(13);
         bg_phase_decide_b(c, t, T);
