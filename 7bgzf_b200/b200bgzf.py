@@ -16,6 +16,7 @@ MAX_BLOCK_SIZE = 0x10000
 APPEND_EOF = 1
 VERIFY = 2
 FRAME_MIGZ = 4
+RANGE_VOFFSET = 8
 E_NOFIT, E_ARG, E_CUDA, E_FORMAT, E_NOSPACE, E_CRC = 1, -1, -2, -3, -4, -5
 EOF_BLOCK = bytes.fromhex("1f8b08040000000000ff0600424302001b0003000000000000000000")
 
@@ -30,6 +31,7 @@ EXPORTS = [
     "b200bgzf_container_head", "b200bgzf_container_bound", "b200bgzf_container_frame", "b200bgzf_container_compress_host",
     "b200bgzf_inflate_units_host", "b200bgzf_container_units", "b200bgzf_units_free", "b200bgzf_container_inflate_host",
     "b200bgzf_multi_container_bound", "b200bgzf_multi_container_compress_host", "b200bgzf_container_inflate_size",
+    "b200bgzf_index_host", "b200bgzf_gzi_parse", "b200bgzf_inflate_ranges_host", "b200bgzf_inflate_ranges_device",
 ]
 CONTAINER_GZIP, CONTAINER_MIGZ, CONTAINER_GZINGA, CONTAINER_DICTZIP, CONTAINER_RAZF = 1, 2, 3, 4, 5
 
@@ -41,6 +43,10 @@ class Unit(ctypes.Structure):
 class PieceSpec(ctypes.Structure):
     _fields_ = [("member_blocks", ctypes.c_uint32), ("head_gap", ctypes.c_uint32), ("tail_gap", ctypes.c_uint32), ("no_final", ctypes.c_uint32),
                 ("piece_base", ctypes.c_uint64), ("piece_total", ctypes.c_uint64), ("history", ctypes.c_uint32), ("reserved", ctypes.c_uint32)]
+
+
+class Range(ctypes.Structure):
+    _fields_ = [("beg", ctypes.c_uint64), ("end", ctypes.c_uint64)]
 
 
 class B200BgzfError(RuntimeError):
@@ -116,6 +122,11 @@ def load(path=LIB_PATH):
     lib.b200bgzf_multi_container_bound.argtypes = [vp, i32, u32, sz]
     lib.b200bgzf_multi_container_bound.restype = sz
     lib.b200bgzf_multi_container_compress_host.argtypes = [vp, i32, u32, vp, sz, i32, vp, sz, psz]
+    lib.b200bgzf_index_host.argtypes = [vp, sz, pu64, pu64, sz, psz]
+    lib.b200bgzf_gzi_parse.argtypes = [vp, sz, pu64, pu64, sz, psz]
+    prange = ctypes.POINTER(Range)
+    lib.b200bgzf_inflate_ranges_host.argtypes = [vp, vp, sz, pu64, pu64, sz, prange, sz, vp, sz, psz, pu64, ctypes.c_uint]
+    lib.b200bgzf_inflate_ranges_device.argtypes = [vp, vp, sz, prange, sz, vp, sz, psz, pu64, ctypes.c_uint, vp]
     return lib
 
 
@@ -299,6 +310,37 @@ class Codec:
         self._check(self.lib.b200bgzf_inflate_device(self.h, d_in, nbytes, d_out, out_cap, ctypes.byref(n), flags, stream))
         return n.value
 
+    # ---- random access ----
+    def inflate_ranges(self, blob, ranges, index=None, voffsets=False, flags=0):
+        """(the ranges' bytes back to back, where each range starts) — b200bgzf_inflate_ranges_host.  ranges: [(beg, end)] of
+        the decoded stream, or of BGZF virtual offsets with voffsets=True; index: (caddr, uaddr) as index() / gzi_parse()
+        give them, or None (header walk)"""
+        n = len(ranges)
+        arr = (Range * max(n, 1))(*[Range(b, e) for b, e in ranges])
+        ca = ua = None
+        ni = 0
+        if index is not None:
+            ni = len(index[0])
+            ca, ua = (ctypes.c_uint64 * max(ni, 1))(*index[0]), (ctypes.c_uint64 * max(ni, 1))(*index[1])
+        fl = flags | (RANGE_VOFFSET if voffsets else 0)
+        need, off = ctypes.c_size_t(), (ctypes.c_uint64 * max(n, 1))()
+        rc = self.lib.b200bgzf_inflate_ranges_host(self.h, _addr(blob), len(blob), ca, ua, ni, arr, n, None, 0, ctypes.byref(need), off, fl)
+        self._check(rc, ok=(0, E_NOSPACE))
+        out = bytearray(max(need.value, 1))
+        got = ctypes.c_size_t()
+        self._check(self.lib.b200bgzf_inflate_ranges_host(self.h, _addr(blob), len(blob), ca, ua, ni, arr, n, _addr(out), len(out),
+                                                          ctypes.byref(got), off, fl))
+        return bytes(out[: got.value]), list(off[:n])
+
+    def inflate_ranges_device(self, d_in, nbytes, ranges, d_out, out_cap, voffsets=False, flags=0, stream=None):
+        """(output bytes, where each range starts) — b200bgzf_inflate_ranges_device (device addresses in and out)"""
+        n = len(ranges)
+        arr = (Range * max(n, 1))(*[Range(b, e) for b, e in ranges])
+        got, off = ctypes.c_size_t(), (ctypes.c_uint64 * max(n, 1))()
+        self._check(self.lib.b200bgzf_inflate_ranges_device(self.h, d_in, nbytes, arr, n, d_out, out_cap, ctypes.byref(got), off,
+                                                            flags | (RANGE_VOFFSET if voffsets else 0), stream))
+        return got.value, list(off[:n])
+
     def profile(self, enable=True, reset=True, slots=32):
         arr = (ctypes.c_ulonglong * slots)()
         self._check(self.lib.b200bgzf_profile(self.h, 1 if enable else 0, arr, slots, 1 if reset else 0))
@@ -390,3 +432,27 @@ def gzi_format(caddr, uaddr, lib=None):
     buf = bytearray(8 + 16 * max(n - 1, 0))
     w = lib.b200bgzf_gzi_format(ca, ua, n, _addr(buf), len(buf))
     return bytes(buf[:w])
+
+
+def _pairs(fn, blob, what, lib):
+    n = ctypes.c_size_t()
+    rc = fn(_addr(blob), len(blob), None, None, 0, ctypes.byref(n))
+    if rc not in (0, E_NOSPACE):
+        raise B200BgzfError(rc, what)
+    ca, ua = (ctypes.c_uint64 * max(n.value, 1))(), (ctypes.c_uint64 * max(n.value, 1))()
+    rc = fn(_addr(blob), len(blob), ca, ua, n.value, ctypes.byref(n))
+    if rc != 0:
+        raise B200BgzfError(rc, what)
+    return list(ca[: n.value]), list(ua[: n.value])
+
+
+def index(blob, lib=None):
+    """(caddr, uaddr): start of every member (EOF marker included) in the stream and in its decoded bytes — b200bgzf_index_host"""
+    lib = lib or load()
+    return _pairs(lib.b200bgzf_index_host, blob, "member index", lib)
+
+
+def gzi_parse(data, lib=None):
+    """(caddr, uaddr) of a .gzi, the implicit (0, 0) entry first — b200bgzf_gzi_parse"""
+    lib = lib or load()
+    return _pairs(lib.b200bgzf_gzi_parse, data, ".gzi", lib)

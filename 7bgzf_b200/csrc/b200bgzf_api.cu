@@ -64,6 +64,9 @@ struct Lane {
     volatile uint32_t *h_flag = nullptr;   /* pinned: set by a 4-byte copy queued behind the member's copy (no driver call needed to see it) */
     uint32_t *d_one = nullptr;             /* device word holding 1: the source of that copy */
     uint8_t *one_dev = nullptr, *one_host = nullptr;   /* one-block fast path: everything it needs in one device and one pinned slab */
+    uint8_t *d_rdec = nullptr;                  /* range reads: decoded members of a group, then the group's output */
+    uint64_t *d_rmeta = nullptr;                /* range reads: the group's gather lists */
+    size_t rdec_cap = 0, rmeta_cap = 0;
 };
 
 /* ---- the hook's combiner: many synchronous one-block callers, ONE submitter --------------------------------------
@@ -127,6 +130,10 @@ struct b200bgzf_ctx {
     uint32_t *d_idx_jump = nullptr, *d_idx_jump2 = nullptr, *d_idx_reach = nullptr;
     size_t idx_cap = 0, idx_tiles = 0;
     uint64_t *h_idx = nullptr;
+    /* device-resident range reads: per-member and per-range workspaces, the scratch of decoded members, pinned staging */
+    uint64_t *d_rng_mem = nullptr, *d_rng_rw = nullptr, *d_rng_counts = nullptr, *h_rng = nullptr, *h_rng_soff = nullptr;
+    uint8_t *d_rng_scratch = nullptr;
+    size_t rng_mem_cap = 0, rng_rw_cap = 0, rng_scratch_cap = 0, h_rng_cap = 0, h_rng_soff_cap = 0;
     /* Completion thread (hook callers beyond the host's core count): callers neither spin nor poll, they sleep on their
      * lane's futex word; this one thread polls the events of the lanes in flight and wakes each caller as its member is back */
     std::thread waiter;
@@ -221,6 +228,7 @@ void lane_free(Lane &l)
     if (l.done) cudaEventDestroy(l.done);
     cudaFree(l.one_dev);
     if (l.one_host) cudaFreeHost(l.one_host);
+    cudaFree(l.d_rdec); cudaFree(l.d_rmeta);
     if (l.stream) cudaStreamDestroy(l.stream);
     l.~Lane();
     new (&l) Lane();
@@ -425,6 +433,9 @@ extern "C" void b200bgzf_destroy(b200bgzf_ctx *ctx)
         cudaFree(ctx->d_idx_tilecount); cudaFree(ctx->d_idx_isize); cudaFree(ctx->d_idx_status); cudaFree(ctx->d_inf_status);
         cudaFree(ctx->d_idx_cand); cudaFree(ctx->d_idx_pick); cudaFree(ctx->d_idx_jump); cudaFree(ctx->d_idx_jump2); cudaFree(ctx->d_idx_reach);
         if (ctx->h_idx) cudaFreeHost(ctx->h_idx);
+        cudaFree(ctx->d_rng_mem); cudaFree(ctx->d_rng_rw); cudaFree(ctx->d_rng_counts); cudaFree(ctx->d_rng_scratch);
+        if (ctx->h_rng) cudaFreeHost(ctx->h_rng);
+        if (ctx->h_rng_soff) cudaFreeHost(ctx->h_rng_soff);
     }
     delete ctx;
 }
@@ -1173,16 +1184,10 @@ extern "C" int b200bgzf_inflate_size_host(const void *in, size_t in_bytes, size_
     return B200BGZF_OK;
 }
 
-extern "C" int b200bgzf_inflate_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, void *d_out, size_t out_cap,
-                                       size_t *out_bytes, unsigned flags, void *stream_)
+namespace {
+/* the member index of a device-resident BGZF stream (ctx->d_idx_*): member count and decoded size to the host */
+int device_index(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, cudaStream_t stream, uint64_t *nmembers, uint64_t *total)
 {
-    if (!ctx || !d_in || !out_bytes || in_bytes < 28) return B200BGZF_E_ARG;
-    DeviceGuard g(ctx->device);
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    Lane &l = ctx->lanes[0];
-    int r = lane_reserve(ctx, l, 1, 0, 0, false);
-    if (r) return r;
-    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : l.stream;
     const size_t tiles = bgzf_index_tiles(in_bytes);
     if (!ctx->h_idx) CK(cudaMallocHost((void **)&ctx->h_idx, 8 * sizeof(uint64_t)));
     if (!ctx->d_idx_counts) {
@@ -1234,7 +1239,24 @@ extern "C" int b200bgzf_inflate_device(b200bgzf_ctx *ctx, const void *d_in, size
         break;
     }
     if ((uint32_t)ctx->h_idx[2]) return B200BGZF_E_FORMAT;
-    const uint64_t nm = ctx->h_idx[0], total = ctx->h_idx[1];
+    *nmembers = ctx->h_idx[0];
+    *total = ctx->h_idx[1];
+    return B200BGZF_OK;
+}
+}  // namespace
+
+extern "C" int b200bgzf_inflate_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, void *d_out, size_t out_cap,
+                                       size_t *out_bytes, unsigned flags, void *stream_)
+{
+    if (!ctx || !d_in || !out_bytes || in_bytes < 28) return B200BGZF_E_ARG;
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    int r = lane_reserve(ctx, l, 1, 0, 0, false);
+    if (r) return r;
+    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : l.stream;
+    uint64_t nm = 0, total = 0;
+    if ((r = device_index(ctx, d_in, in_bytes, stream, &nm, &total))) return r;
     *out_bytes = (size_t)total;
     if (total > out_cap || (!d_out && total)) return B200BGZF_E_NOSPACE;
     BgzfInflateArgs a;
@@ -1401,4 +1423,407 @@ extern "C" int b200bgzf_inflate_units_host(b200bgzf_ctx *ctx, const void *in, si
         return out_bytes ? B200BGZF_OK : B200BGZF_E_ARG;
     }
     return inflate_host_impl(ctx, in, in_bytes, units, nunits, out, out_cap, out_bytes, flags, unit_crc);
+}
+
+/* ------------------------------------------------------------------------------------------------ */
+/* random access                                                                                    */
+
+namespace {
+
+/* Device bytes a range call may hold for decoded members: the device variant's scratch; a host-variant group (decoded
+ * members + output) takes a quarter, and a range is cut into pieces of a sixteenth.  B200BGZF_RANGE_BUDGET (bytes, at least
+ * 1 MiB) lowers it, so that the multi-pass paths can be exercised on small inputs. */
+uint64_t range_budget()
+{
+    static const uint64_t b = [] {
+        const char *e = getenv("B200BGZF_RANGE_BUDGET");
+        const unsigned long long v = e && *e ? strtoull(e, nullptr, 10) : 0ull;
+        return v >= (1ull << 20) ? (uint64_t)v : (uint64_t)1 << 30;
+    }();
+    return b;
+}
+
+/* largest i in [0, n) with a[i] <= x (a ascending, a[0] <= x) */
+size_t last_le(const uint64_t *a, size_t n, uint64_t x) { return (size_t)(std::upper_bound(a, a + n, x) - a) - 1; }
+
+/* every member start (EOF marker included) by a header walk */
+int walk_index(const uint8_t *p, size_t in_bytes, std::vector<uint64_t> &c, std::vector<uint64_t> &u)
+{
+    uint64_t off = 0, pos = 0;
+    while (off < in_bytes) {
+        uint64_t sz = 0;
+        if (!member_parse(p + off, in_bytes - off, &sz)) return B200BGZF_E_FORMAT;
+        c.push_back(off);
+        u.push_back(pos);
+        pos += rd32(p + off + sz - 4);
+        off += sz;
+    }
+    return B200BGZF_OK;
+}
+
+}  // namespace
+
+extern "C" int b200bgzf_index_host(const void *in, size_t in_bytes, uint64_t *caddr, uint64_t *uaddr, size_t cap, size_t *nmembers)
+{
+    if ((!in && in_bytes) || !nmembers || (cap && (!caddr || !uaddr))) return B200BGZF_E_ARG;
+    std::vector<uint64_t> c, u;
+    const int r = walk_index((const uint8_t *)in, in_bytes, c, u);
+    if (r) return r;
+    *nmembers = c.size();
+    const size_t n = std::min(cap, c.size());
+    if (n) { memcpy(caddr, c.data(), n * 8); memcpy(uaddr, u.data(), n * 8); }
+    return c.size() > cap ? B200BGZF_E_NOSPACE : B200BGZF_OK;
+}
+
+extern "C" int b200bgzf_gzi_parse(const void *gzi, size_t gzi_bytes, uint64_t *caddr, uint64_t *uaddr, size_t cap, size_t *nmembers)
+{
+    if (!gzi || !nmembers || (cap && (!caddr || !uaddr))) return B200BGZF_E_ARG;
+    const uint8_t *p = (const uint8_t *)gzi;
+    auto get = [&](size_t at) { uint64_t v = 0; for (int k = 7; k >= 0; k--) v = v << 8 | p[at + k]; return v; };
+    if (gzi_bytes < 8) return B200BGZF_E_FORMAT;
+    const uint64_t entries = get(0);
+    if (entries > (gzi_bytes - 8) / 16 || gzi_bytes != 8 + 16 * entries) return B200BGZF_E_FORMAT;
+    uint64_t pc = 0, pu = 0;
+    for (uint64_t i = 0; i < entries; i++) {
+        const uint64_t c = get(8 + 16 * i), u = get(16 + 16 * i);
+        if (c <= pc || u < pu) return B200BGZF_E_FORMAT;
+        pc = c;
+        pu = u;
+    }
+    *nmembers = (size_t)entries + 1;
+    const size_t n = std::min<size_t>(cap, entries + 1);
+    for (size_t i = 0; i < n; i++) {
+        caddr[i] = i ? get(8 + 16 * (i - 1)) : 0;
+        uaddr[i] = i ? get(16 + 16 * (i - 1)) : 0;
+    }
+    return entries + 1 > cap ? B200BGZF_E_NOSPACE : B200BGZF_OK;
+}
+
+extern "C" int b200bgzf_inflate_ranges_host(b200bgzf_ctx *ctx, const void *in, size_t in_bytes, const uint64_t *caddr, const uint64_t *uaddr,
+                                            size_t nindex, const b200bgzf_range *ranges, size_t nranges, void *out, size_t out_cap,
+                                            size_t *out_bytes, uint64_t *range_off, unsigned flags)
+{
+    if (!ctx || !out_bytes || (!in && in_bytes) || (!ranges && nranges) || (!caddr != !uaddr) || (caddr && !nindex)) return B200BGZF_E_ARG;
+    const uint8_t *p = (const uint8_t *)in;
+    /* ---- plan on the host: the index, every range as [beg, end) of the decoded stream, the output layout ---- */
+    std::vector<uint64_t> wc, wu;
+    if (!caddr) {
+        const int r = walk_index(p, in_bytes, wc, wu);
+        if (r) return r;
+        caddr = wc.data();
+        uaddr = wu.data();
+        nindex = wc.size();
+    }
+    const size_t n = nindex;
+    for (size_t m = 0; m < n; m++)
+        if (caddr[m] >= in_bytes || (m && (caddr[m] <= caddr[m - 1] || uaddr[m] < uaddr[m - 1])) || (m == 0 && uaddr[0] != 0)) return B200BGZF_E_ARG;
+    uint64_t total = 0;
+    if (n) {                                            /* the decoded size: the last listed member's ISIZE */
+        uint64_t sz = 0;
+        if (!member_parse(p + caddr[n - 1], in_bytes - caddr[n - 1], &sz)) return B200BGZF_E_FORMAT;
+        total = uaddr[n - 1] + rd32(p + caddr[n - 1] + sz - 4);
+    }
+    auto uend = [&](size_t m) { return m + 1 < n ? uaddr[m + 1] : total; };
+    auto cend = [&](size_t m) { return m + 1 < n ? caddr[m + 1] : (uint64_t)in_bytes; };
+    auto resolve = [&](uint64_t v, uint64_t *pos) {
+        const uint64_t c = v >> 16, u = v & 0xffffu;
+        if (c == in_bytes) { *pos = total; return u == 0; }
+        if (!n || c < caddr[0]) return false;
+        const size_t m = last_le(caddr, n, c);
+        if (caddr[m] != c || u > uend(m) - uaddr[m]) return false;
+        *pos = uaddr[m] + u;
+        return true;
+    };
+    std::vector<uint64_t> rb(nranges), re(nranges);
+    uint64_t out_total = 0;
+    for (size_t i = 0; i < nranges; i++) {
+        uint64_t b = ranges[i].beg, e = ranges[i].end;
+        if ((flags & B200BGZF_RANGE_VOFFSET) && !(resolve(b, &b) && resolve(e, &e))) return B200BGZF_E_ARG;
+        if (b > e || e > total) return B200BGZF_E_ARG;
+        rb[i] = b;
+        re[i] = e;
+        if (range_off) range_off[i] = out_total;
+        out_total += e - b;
+    }
+    *out_bytes = (size_t)out_total;
+    if (out_total > out_cap || (!out && out_total)) return B200BGZF_E_NOSPACE;
+    if (out_total == 0) return B200BGZF_OK;
+
+    /* ---- groups of consecutive pieces of ranges, pipelined over the lanes ---- */
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    PendingGuard pg(ctx->lanes, kLanes);
+    const uint64_t group_cap = range_budget() / 4, piece_cap = range_budget() / 16;
+    const bool verify = (flags & B200BGZF_VERIFY) != 0;
+    struct Piece { uint64_t beg, len, out; size_t first; };
+    std::vector<uint64_t> stamp(n, ~0ull), msoff(n);
+    std::vector<size_t> gm;                             /* the group's touched members */
+    std::vector<Piece> gp;
+    uint64_t gdec = 0, gout = 0, gout0 = 0, out_pos = 0, gid = 0;
+    bool bad = false, badcrc = false;
+    int r, lane_i = 0;
+    auto complete = [&](Lane &l) -> int {
+        CK(cudaStreamSynchronize(l.stream));
+        if (l.h_total[1] & 1u) bad = true;
+        if (l.h_total[1] & 2u) badcrc = true;
+        l.pending = false;
+        return 0;
+    };
+    auto submit = [&]() -> int {
+        Lane &l = ctx->lanes[lane_i++ % kInflateLanes];
+        if (l.pending && (r = complete(l))) return r;
+        std::sort(gm.begin(), gm.end());
+        const size_t M = gm.size(), P = gp.size();
+        uint64_t cbytes = 0;
+        for (size_t k = 0; k < M; k++)
+            if (k + 1 == M || gm[k + 1] != gm[k] + 1) {                       /* end of a run of consecutive members */
+                size_t k0 = k;
+                while (k0 > 0 && gm[k0 - 1] + 1 == gm[k0]) k0--;
+                cbytes += cend(gm[k]) - caddr[gm[k0]];
+            }
+        if ((r = lane_reserve(ctx, l, (uint32_t)std::max<size_t>(M, kInflateBatch), cbytes + 256, 0, false))) return r;
+        const uint64_t obase = (gdec + 64 + 255) & ~(uint64_t)255;             /* the group's output behind its decoded members */
+        CK(grow(&l.d_rdec, &l.rdec_cap, obase + gout + 64));
+        CK(grow(&l.d_rmeta, &l.rmeta_cap, 4 * P));
+        CK(grow(&l.h_in, &l.host_in_cap, cbytes + 16, true));
+        CK(grow(&l.h_meta, &l.meta_cap, 3 * M + 4 * P, true));
+        uint64_t *h_inoff = l.h_meta, *h_outoff = l.h_meta + M, *h_rm = l.h_meta + 3 * M;
+        uint32_t *h_hdr = (uint32_t *)(l.h_meta + 2 * M), *h_msz = h_hdr + M;
+        /* the compressed bytes of every run of touched members, packed; nothing else of the input is read */
+        uint64_t pos = 0, soff = 0;
+        for (size_t k0 = 0; k0 < M;) {
+            size_t k1 = k0 + 1;
+            while (k1 < M && gm[k1] == gm[k1 - 1] + 1) k1++;
+            const uint64_t cs = caddr[gm[k0]], ce = cend(gm[k1 - 1]);
+            memcpy(l.h_in + pos, p + cs, ce - cs);
+            for (size_t k = k0; k < k1; k++) {
+                const size_t m = gm[k];
+                uint64_t sz = 0;
+                const uint32_t hl = member_parse(p + caddr[m], cend(m) - caddr[m], &sz);
+                if (!hl) return B200BGZF_E_FORMAT;
+                const uint32_t isz = rd32(p + caddr[m] + sz - 4);
+                if (isz != uend(m) - uaddr[m] || isz > 1032ull * (sz - hl) + 1032u) return B200BGZF_E_FORMAT;   /* (index and stream disagree) */
+                h_inoff[k] = pos + (caddr[m] - cs);
+                h_outoff[k] = soff;
+                h_hdr[k] = hl;
+                h_msz[k] = (uint32_t)sz;
+                msoff[m] = soff;
+                soff += isz;
+            }
+            pos += ce - cs;
+            k0 = k1;
+        }
+        /* gather lists: where each piece starts in the decoded members and in the group's output, its length, first tile */
+        uint64_t tiles = 0;
+        for (size_t j = 0; j < P; j++) {
+            const Piece &q = gp[j];
+            h_rm[j] = msoff[q.first] + (q.beg - uaddr[q.first]);
+            h_rm[P + j] = q.out - gout0;
+            h_rm[2 * P + j] = q.len;
+            h_rm[3 * P + j] = tiles;
+            tiles += (q.len + BGZF_GATHER_TILE - 1) / BGZF_GATHER_TILE;
+        }
+        CK(cudaMemcpyAsync(l.d_in, l.h_in, pos, cudaMemcpyHostToDevice, l.stream));
+        CK(cudaMemcpyAsync(l.d_inoff, h_inoff, M * sizeof(uint64_t), cudaMemcpyHostToDevice, l.stream));
+        CK(cudaMemcpyAsync(l.d_outoff, h_outoff, M * sizeof(uint64_t), cudaMemcpyHostToDevice, l.stream));
+        CK(cudaMemcpyAsync(l.d_inlen, h_hdr, M * sizeof(uint32_t), cudaMemcpyHostToDevice, l.stream));
+        CK(cudaMemcpyAsync(l.d_len, h_msz, M * sizeof(uint32_t), cudaMemcpyHostToDevice, l.stream));
+        CK(cudaMemcpyAsync(l.d_rmeta, h_rm, 4 * P * sizeof(uint64_t), cudaMemcpyHostToDevice, l.stream));
+        CK(cudaMemsetAsync(l.d_total, 0, 4 * sizeof(uint64_t), l.stream));
+        BgzfInflateArgs a;
+        memset(&a, 0, sizeof a);
+        a.in = l.d_in;
+        a.in_off = l.d_inoff;
+        a.out_off = l.d_outoff;
+        a.hdr_len = l.d_inlen;
+        a.msize = l.d_len;
+        a.nblocks = (uint32_t)M;
+        a.out = l.d_rdec;
+        a.status = l.d_status;
+        a.err_flag = (uint32_t *)(l.d_total + 1);
+        a.crctab = ctx->d_crctab;
+        a.crcpow = ctx->d_crcpow;
+        a.verify_crc = verify ? 1 : 0;
+        CK(bgzf_launch_inflate(&a, l.stream));
+        BgzfRangeGatherArgs ga;
+        ga.scratch = l.d_rdec;
+        ga.win_lo = 0;
+        ga.win_hi = ~0ull;
+        ga.out = l.d_rdec + obase;
+        ga.src = l.d_rmeta;
+        ga.range_off = l.d_rmeta + P;
+        ga.len = l.d_rmeta + 2 * P;
+        ga.tile_off = l.d_rmeta + 3 * P;
+        ga.nranges = (uint32_t)P;
+        CK(bgzf_launch_range_gather(&ga, tiles, l.stream));
+        ctx->launches += 2 + a.verify_crc;
+        CK(cudaMemcpyAsync((uint8_t *)out + gout0, l.d_rdec + obase, gout, cudaMemcpyDeviceToHost, l.stream));
+        CK(cudaMemcpyAsync(l.h_total, l.d_total, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, l.stream));
+        l.pending = true;
+        gid++;
+        gm.clear();
+        gp.clear();
+        gout0 += gout;
+        gdec = gout = 0;
+        return 0;
+    };
+    for (size_t i = 0; i < nranges; i++) {
+        for (uint64_t b = rb[i]; b < re[i];) {
+            const uint64_t len = std::min(piece_cap, re[i] - b);
+            const size_t f = last_le(uaddr, n, b), l = last_le(uaddr, n, b + len - 1);
+            uint64_t add = 0;
+            for (size_t m = f; m <= l; m++)
+                if (stamp[m] != gid) add += uend(m) - uaddr[m];
+            if (!gp.empty() && gdec + add + gout + len > group_cap) {
+                if ((r = submit())) return r;
+                add = uaddr[l] - uaddr[f] + (uend(l) - uaddr[l]);
+            }
+            if (gp.size() >= 0xffffffffu) return B200BGZF_E_ARG;
+            for (size_t m = f; m <= l; m++)
+                if (stamp[m] != gid) { stamp[m] = gid; gm.push_back(m); }
+            gdec += add;
+            gout += len;
+            gp.push_back({ b, len, out_pos, f });
+            out_pos += len;
+            b += len;
+        }
+    }
+    if (!gp.empty() && (r = submit())) return r;
+    for (auto &l : ctx->lanes)
+        if (l.pending && (r = complete(l))) return r;
+    return bad ? B200BGZF_E_FORMAT : badcrc ? B200BGZF_E_CRC : B200BGZF_OK;
+}
+
+extern "C" int b200bgzf_inflate_ranges_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, const b200bgzf_range *ranges, size_t nranges,
+                                              void *d_out, size_t out_cap, size_t *out_bytes, uint64_t *range_off, unsigned flags, void *stream_)
+{
+    if (!ctx || !d_in || !out_bytes || in_bytes < 28 || (!ranges && nranges) || nranges > 0x7fffffffu) return B200BGZF_E_ARG;
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    int r = lane_reserve(ctx, l, 1, 0, 0, false);
+    if (r) return r;
+    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : l.stream;
+    uint64_t nm = 0, total = 0;
+    if ((r = device_index(ctx, d_in, in_bytes, stream, &nm, &total))) return r;
+    *out_bytes = 0;
+    if (nranges == 0) return B200BGZF_OK;
+    const size_t R = nranges;
+    /* workspaces: per member diff (i32, nm + 1), m_soff, t_in_off, t_soff; per range 2 (beg, end) + delta, len, src, range_off,
+     * tile_off + first (u32); pinned: 8 words of counts, the ranges, range_off */
+    CK(grow(&ctx->d_rng_mem, &ctx->rng_mem_cap, 3 * (size_t)ctx->idx_cap + ctx->idx_cap / 2 + 2));
+    CK(grow(&ctx->d_rng_rw, &ctx->rng_rw_cap, 7 * R + R / 2 + 1));
+    CK(grow(&ctx->h_rng, &ctx->h_rng_cap, 8 + 3 * R, true));
+    if (!ctx->d_rng_counts) CK(cudaMalloc((void **)&ctx->d_rng_counts, 8 * sizeof(uint64_t)));
+    uint64_t *m_soff = ctx->d_rng_mem, *t_in_off = m_soff + nm, *t_soff = t_in_off + nm;
+    int32_t *diff = (int32_t *)(t_soff + nm);
+    uint64_t *d_rng = ctx->d_rng_rw, *delta = d_rng + 2 * R, *len = delta + R, *src = len + R, *roff = src + R, *toff = roff + R;
+    uint32_t *first = (uint32_t *)(toff + R);
+    uint64_t *h_counts = ctx->h_rng, *h_rng = ctx->h_rng + 8, *h_roff = h_rng + 2 * R;
+    for (size_t i = 0; i < R; i++) { h_rng[2 * i] = ranges[i].beg; h_rng[2 * i + 1] = ranges[i].end; }
+    CK(cudaMemcpyAsync(d_rng, h_rng, 2 * R * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+    CK(cudaMemsetAsync(diff, 0, (nm + 1) * sizeof(int32_t), stream));
+    CK(cudaMemsetAsync(ctx->d_rng_counts, 0, 8 * sizeof(uint64_t), stream));
+    BgzfRangePlanArgs pa;
+    pa.ranges = d_rng;
+    pa.nranges = (uint32_t)R;
+    pa.voffsets = (flags & B200BGZF_RANGE_VOFFSET) ? 1 : 0;
+    pa.in_bytes = in_bytes;
+    pa.in_off = ctx->d_idx_inoff;
+    pa.out_off = ctx->d_idx_outoff;
+    pa.isize = ctx->d_idx_isize;
+    pa.nmembers = ctx->d_idx_counts;
+    pa.total = ctx->d_idx_counts + 1;
+    pa.diff = diff;
+    pa.first = first;
+    pa.delta = delta;
+    pa.len = len;
+    pa.status = (uint32_t *)(ctx->d_rng_counts + 4);
+    CK(bgzf_launch_range_plan(&pa, stream));
+    BgzfRangeTouchArgs ta;
+    ta.nmembers = (uint32_t)nm;
+    ta.nranges = (uint32_t)R;
+    ta.diff = diff;
+    ta.in_off = ctx->d_idx_inoff;
+    ta.isize = ctx->d_idx_isize;
+    ta.t_in_off = t_in_off;
+    ta.t_soff = t_soff;
+    ta.m_soff = m_soff;
+    ta.first = first;
+    ta.delta = delta;
+    ta.len = len;
+    ta.src = src;
+    ta.range_off = roff;
+    ta.tile_off = toff;
+    ta.counts = ctx->d_rng_counts;
+    CK(bgzf_launch_range_touch(&ta, stream));
+    ctx->launches += 2;
+    CK(cudaMemcpyAsync(h_counts, ctx->d_rng_counts, 8 * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaMemcpyAsync(h_roff, roff, R * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    if ((uint32_t)h_counts[4]) return B200BGZF_E_ARG;
+    const uint64_t nt = h_counts[0], sbytes = h_counts[1], obytes = h_counts[2], ntiles = h_counts[3];
+    *out_bytes = (size_t)obytes;
+    if (range_off) memcpy(range_off, h_roff, R * sizeof(uint64_t));
+    if (obytes > out_cap || (!d_out && obytes)) return B200BGZF_E_NOSPACE;
+    if (obytes == 0) return B200BGZF_OK;
+    /* passes over consecutive touched members whose decoded bytes fit the scratch (one pass unless they exceed the budget) */
+    const uint64_t budget = range_budget();
+    std::vector<uint64_t> cut{ 0 }, base{ 0 };          /* pass k: touched members [cut[k], cut[k+1]), scratch coordinates from base[k] */
+    if (sbytes <= budget) {
+        cut.push_back(nt);
+    } else {
+        CK(grow(&ctx->h_rng_soff, &ctx->h_rng_soff_cap, (size_t)nt, true));
+        uint64_t *h_soff = ctx->h_rng_soff;
+        CK(cudaMemcpyAsync(h_soff, t_soff, nt * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        for (uint64_t k0 = 0; k0 < nt;) {
+            uint64_t k1 = k0 + 1;
+            while (k1 < nt && (k1 + 1 < nt ? h_soff[k1 + 1] : sbytes) - h_soff[k0] <= budget) k1++;
+            cut.push_back(k1);
+            base.push_back(k1 < nt ? h_soff[k1] : sbytes);
+            k0 = k1;
+        }
+        base.pop_back();
+        for (size_t k = 0; k + 1 < cut.size(); k++)       /* scratch offsets relative to their pass */
+            for (uint64_t j = cut[k]; j < cut[k + 1]; j++) h_soff[j] -= base[k];
+        CK(cudaMemcpyAsync(t_soff, h_soff, nt * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+    }
+    uint64_t widest = 0;
+    for (size_t k = 0; k + 1 < cut.size(); k++) {
+        const uint64_t hi = k + 2 < cut.size() ? base[k + 1] : sbytes;
+        widest = std::max(widest, hi - base[k]);
+    }
+    CK(grow(&ctx->d_rng_scratch, &ctx->rng_scratch_cap, (size_t)widest + 64));
+    for (size_t k = 0; k + 1 < cut.size(); k++) {
+        BgzfInflateArgs a;
+        memset(&a, 0, sizeof a);
+        a.in = (const uint8_t *)d_in;
+        a.in_off = t_in_off + cut[k];
+        a.out_off = t_soff + cut[k];
+        a.nblocks = (uint32_t)(cut[k + 1] - cut[k]);
+        a.out = ctx->d_rng_scratch;
+        a.status = ctx->d_inf_status + cut[k];
+        a.err_flag = ctx->d_idx_status + 1;
+        a.crctab = ctx->d_crctab;
+        a.crcpow = ctx->d_crcpow;
+        a.verify_crc = (flags & B200BGZF_VERIFY) ? 1 : 0;
+        CK(bgzf_launch_inflate(&a, stream));
+        BgzfRangeGatherArgs ga;
+        ga.scratch = ctx->d_rng_scratch;
+        ga.win_lo = base[k];
+        ga.win_hi = k + 2 < cut.size() ? base[k + 1] : sbytes;
+        ga.out = (uint8_t *)d_out;
+        ga.src = src;
+        ga.range_off = roff;
+        ga.len = len;
+        ga.tile_off = toff;
+        ga.nranges = (uint32_t)R;
+        CK(bgzf_launch_range_gather(&ga, ntiles, stream));
+        ctx->launches += 2 + a.verify_crc;
+    }
+    CK(cudaMemcpyAsync(ctx->h_idx + 3, ctx->d_idx_status + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    const uint32_t ef = (uint32_t)ctx->h_idx[3];
+    return (ef & 1u) ? B200BGZF_E_FORMAT : (ef & 2u) ? B200BGZF_E_CRC : B200BGZF_OK;
 }

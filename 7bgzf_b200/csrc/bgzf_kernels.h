@@ -87,9 +87,50 @@ struct BgzfIndexWork {
     uint32_t *status;          /* bit 0: not a BGZF stream, bit 1: more candidates than max_blocks */
 };
 
+/* random access (bgzf_ranges.cu): requested ranges -> touched members -> scratch -> caller's output */
+#define BGZF_GATHER_TILE 32768u      /* bytes of one range copied by one gather CTA */
+
+struct BgzfRangePlanArgs {
+    const uint64_t *ranges;    /* device: [2 * nranges] beg, end (uncompressed offsets, or BGZF virtual offsets) */
+    uint32_t nranges;
+    int voffsets;
+    uint64_t in_bytes;         /* stream size: a virtual offset may name it (uoffset 0) as the end */
+    const uint64_t *in_off, *out_off;   /* device: the member index (bgzf_launch_index) */
+    const uint32_t *isize;
+    const uint64_t *nmembers, *total;   /* device: member count and decoded size */
+    int32_t *diff;             /* device [nmembers + 1], zeroed: +1 at a range's first member, -1 after its last */
+    uint32_t *first;           /* device [nranges] out: first member of every range */
+    uint64_t *delta, *len;     /* device [nranges] out: offset of the range in its first member, length */
+    uint32_t *status;          /* device: bit 0 set by a range that is out of bounds or names no member start */
+};
+
+struct BgzfRangeTouchArgs {
+    uint32_t nmembers, nranges;
+    const int32_t *diff;
+    const uint64_t *in_off;    /* device [nmembers] */
+    const uint32_t *isize;     /* device [nmembers] */
+    uint64_t *t_in_off, *t_soff;   /* device [nmembers] out: the touched members' input offsets and scratch offsets, in order */
+    uint64_t *m_soff;          /* device [nmembers] out: scratch offset of every touched member (by member number) */
+    const uint32_t *first;
+    const uint64_t *delta, *len;
+    uint64_t *src, *range_off, *tile_off;   /* device [nranges] out: where a range starts in scratch / in the output; its first tile */
+    uint64_t *counts;          /* device [4] out: touched members, scratch bytes, output bytes, gather tiles */
+};
+
+struct BgzfRangeGatherArgs {
+    const uint8_t *scratch;    /* device: decoded bytes [win_lo, win_hi) of the scratch coordinates (+ 64 bytes of pad) */
+    uint64_t win_lo, win_hi;
+    uint8_t *out;              /* device */
+    const uint64_t *src, *range_off, *len, *tile_off;   /* device [nranges] */
+    uint32_t nranges;
+};
+
 #ifdef __cplusplus
 extern "C" {
 #endif
+cudaError_t bgzf_launch_range_plan(const BgzfRangePlanArgs *a, cudaStream_t stream);
+cudaError_t bgzf_launch_range_touch(const BgzfRangeTouchArgs *a, cudaStream_t stream);
+cudaError_t bgzf_launch_range_gather(const BgzfRangeGatherArgs *a, uint64_t ntiles, cudaStream_t stream);
 size_t bgzf_compress_smem_bytes(void);
 cudaError_t bgzf_launch_compress(const BgzfCompressArgs *a, int grid, cudaStream_t stream);
 cudaError_t bgzf_launch_compress_split(const BgzfCompressArgs *a, int csize, cudaStream_t stream);

@@ -3,6 +3,8 @@
  *
  *   7bgzf -c -l6 [-@ N] < in > out.bgz        compress (stdin -> stdout only)
  *   7bgzf -d [-@ N] < in.bgz > out            decompress
+ *   7bgzf -d --offset=N [--size=M] [--gzi=F] < in.bgz > out    decompress bytes [N, N+M) only (bgzip -b N -s M)
+ *   7bgzf --reindex --gzi=F < in.bgz          write the .gzi of an existing stream (bgzip -r)
  *
  * Same flags as the reference's popt table (7bgzf.c:379-398): -l[N]/--libdeflate[=N] (1-12, default 6),
  * -z -m -s -S -n -C -i -K -T [N] and -Z N (the other method flags: each selects a level for the one GPU codec,
@@ -22,6 +24,7 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <sys/mman.h>
 #include <sys/stat.h>
 #include <sys/time.h>
 #include <unistd.h>
@@ -62,6 +65,9 @@ static void usage(const char *argv0)
             "  -@, --threads=threads     threads\n"
             "  -d, --decompress          decompress\n"
             "      --gzi=FILE            (extension) also write a bgzip-style .gzi index of the members to FILE\n"
+            "      --offset=N            (extension, with -d) decompress from byte N of the data on (read --gzi=FILE if given)\n"
+            "      --size=M              (extension, with --offset) at most M bytes\n"
+            "      --reindex             (extension) write the .gzi of the stream on stdin to --gzi=FILE, nothing to stdout\n"
             "      --devices=N           (extension) spread the blocks over N GPUs (contiguous block ranges, same output)\n"
             "      --independent         (extension, 7gzip) pieces without the 16 KiB of history before them: faster, 2-3 %% larger\n"
             "      --primed              (extension, 7migz) pieces of a member see the 32 KiB before them: slower, 2 %% smaller\n"
@@ -428,6 +434,141 @@ static int run_pipeline(int ndevices, int decompress, int level, uint32_t block,
     return ret;
 }
 
+/* ---- random access: the whole input in memory (a regular file is mapped: only the members a read touches are paged in) ---- */
+struct input_map {
+    unsigned char *p;
+    size_t n, map_len;
+    int mapped;
+};
+static int input_load(struct input_map *im)
+{
+    memset(im, 0, sizeof *im);
+    struct stat st;
+    const off_t pos = lseek(0, 0, SEEK_CUR);
+    if (fstat(0, &st) == 0 && S_ISREG(st.st_mode) && pos >= 0 && st.st_size > pos) {
+        void *m = mmap(NULL, (size_t)st.st_size, PROT_READ, MAP_PRIVATE, 0, 0);
+        if (m != MAP_FAILED) {
+            im->p = (unsigned char *)m + pos;
+            im->n = (size_t)(st.st_size - pos);
+            im->map_len = (size_t)st.st_size;
+            im->mapped = 1;
+            return 0;
+        }
+    }
+    size_t cap = (size_t)1 << 20;
+    im->p = (unsigned char *)malloc(cap);
+    for (;;) {
+        if (!im->p) return -1;
+        const ssize_t r = read(0, im->p + im->n, cap - im->n);
+        if (r < 0) return -1;
+        if (r == 0) return 0;
+        im->n += (size_t)r;
+        if (im->n == cap) im->p = (unsigned char *)realloc(im->p, cap *= 2);
+    }
+}
+static void input_free(struct input_map *im)
+{
+    if (im->mapped) munmap(im->p - (im->map_len - im->n), im->map_len);
+    else free(im->p);
+}
+
+/* (caddr, uaddr) of every member: from a .gzi, or by a header walk of the input */
+static int load_index(const struct input_map *im, const char *gzi_path, uint64_t **c, uint64_t **u, size_t *n)
+{
+    *c = *u = NULL;
+    *n = 0;
+    unsigned char *buf = NULL;
+    size_t len = 0;
+    if (gzi_path) {
+        FILE *f = fopen(gzi_path, "rb");
+        if (!f) { fprintf(stderr, "cannot read the index %s\n", gzi_path); return 1; }
+        size_t cap = 4096;
+        buf = (unsigned char *)malloc(cap);
+        for (size_t r; buf && (r = fread(buf + len, 1, cap - len, f)) > 0;)
+            if ((len += r) == cap) buf = (unsigned char *)realloc(buf, cap *= 2);
+        fclose(f);
+        if (!buf) { fprintf(stderr, "out of memory\n"); return 1; }
+    }
+    int r = gzi_path ? b200bgzf_gzi_parse(buf, len, NULL, NULL, 0, n) : b200bgzf_index_host(im->p, im->n, NULL, NULL, 0, n);
+    if (r == 0 || r == B200BGZF_E_NOSPACE) {
+        *c = (uint64_t *)malloc((*n + 1) * sizeof(uint64_t));
+        *u = (uint64_t *)malloc((*n + 1) * sizeof(uint64_t));
+        r = !*c || !*u ? B200BGZF_E_ARG
+                       : gzi_path ? b200bgzf_gzi_parse(buf, len, *c, *u, *n, n) : b200bgzf_index_host(im->p, im->n, *c, *u, *n, n);
+    }
+    free(buf);
+    if (r) fprintf(stderr, gzi_path ? "%s: not a .gzi index\n" : "not BGZF or corrupted\n", gzi_path);
+    return r ? 1 : 0;
+}
+
+/* decoded size: start of the last member + its ISIZE */
+static int stream_total(const struct input_map *im, const uint64_t *c, const uint64_t *u, size_t n, uint64_t *total)
+{
+    *total = 0;
+    if (!n) return 0;
+    uint64_t sz = 0;
+    if (c[n - 1] >= im->n || !b200bgzf_member_header(im->p + c[n - 1], im->n - c[n - 1], &sz)) return 1;
+    const unsigned char *t = im->p + c[n - 1] + sz - 4;
+    *total = u[n - 1] + ((uint64_t)t[0] | ((uint64_t)t[1] << 8) | ((uint64_t)t[2] << 16) | ((uint64_t)t[3] << 24));
+    return 0;
+}
+
+static int range_applet(uint64_t offset, uint64_t size, int have_size, const char *gzi_path)
+{
+    struct input_map im;
+    if (input_load(&im)) { fprintf(stderr, "cannot read stdin\n"); return 1; }
+    uint64_t *c = NULL, *u = NULL, total = 0;
+    size_t n = 0;
+    int ret = load_index(&im, gzi_path, &c, &u, &n);
+    if (!ret && stream_total(&im, c, u, n, &total)) { fprintf(stderr, "not BGZF or corrupted\n"); ret = 1; }
+    if (!ret && offset > total) { fprintf(stderr, "offset %llu is past the end of the data (%llu bytes)\n", (unsigned long long)offset, (unsigned long long)total); ret = 1; }
+    if (!ret) {
+        const uint64_t end = !have_size || size > total - offset ? total : offset + size;
+        b200bgzf_range rg = { offset, end };
+        unsigned char *out = (unsigned char *)malloc(end - offset + 1);
+        b200bgzf_ctx *ctx = NULL;
+        size_t got = 0;
+        const char *dev = getenv("B200BGZF_DEVICE");
+        int r = !out ? B200BGZF_E_ARG : b200bgzf_create(&ctx, dev && *dev ? atoi(dev) : -1);
+        if (r) fprintf(stderr, "b200bgzf: cannot initialise the GPU codec: %s\n", b200bgzf_strerror(r));
+        else if ((r = b200bgzf_inflate_ranges_host(ctx, im.p, im.n, c, u, n, &rg, 1, out, end - offset + 1, &got, NULL, 0)) != 0)
+            fprintf(stderr, "inflate %d\n", r);
+        if (!r && got && fwrite(out, 1, got, stdout) != got) r = 1;
+        ret = r ? 1 : 0;
+        b200bgzf_destroy(ctx);
+        free(out);
+    }
+    free(c);
+    free(u);
+    input_free(&im);
+    return ret;
+}
+
+/* bgzip -r: the .gzi of an existing stream (members that carry data; the first is implicit) */
+static int reindex_applet(const char *gzi_path)
+{
+    struct input_map im;
+    if (input_load(&im)) { fprintf(stderr, "cannot read stdin\n"); return 1; }
+    uint64_t *c = NULL, *u = NULL, total = 0;
+    size_t n = 0, k = 0;
+    int ret = load_index(&im, NULL, &c, &u, &n);
+    if (!ret && stream_total(&im, c, u, n, &total)) ret = 1;
+    if (!ret) {
+        for (size_t i = 0; i < n; i++)
+            if ((i + 1 < n ? u[i + 1] : total) > u[i]) { c[k] = c[i]; u[k++] = u[i]; }
+        struct gzi_acc g;
+        memset(&g, 0, sizeof g);
+        g.caddr = c;
+        g.uaddr = u;
+        g.n = k;
+        ret = gzi_write(&g, gzi_path);
+    }
+    free(c);
+    free(u);
+    input_free(&im);
+    return ret;
+}
+
 int container_applet(const char *name, int kind, int decompress, int level, unsigned param, int ndevices, int nfiles, char **files);   /* applet_containers.c */
 
 static const struct { const char *name; int kind; } k_personas[] = {
@@ -439,6 +580,8 @@ int main(int argc, char **argv)
 {
     int levels[NFLAGS];
     int decompress = 0, nthreads = 1, bad = 0, ndevices = 1, migz = 0, bsize = 0, extreme = 0, kind = 0;
+    int have_offset = 0, have_size = 0, reindex = 0;
+    unsigned long long range_offset = 0, range_size = 0;
     unsigned piece_flags = 0;    /* 7gzip --independent: pieces without dictionary priming; 7migz --primed: with it */
     const char *gzi_path = NULL, *persona = "7bgzf";
     memset(levels, 0, sizeof levels);
@@ -466,7 +609,8 @@ int main(int argc, char **argv)
         { "help", no_argument, 0, 'h' },         { "gzi", required_argument, 0, 1000 },
         { "devices", required_argument, 0, 1001 },  { "bsize", required_argument, 0, 'b' },
         { "extreme", no_argument, 0, 'X' },      { "independent", no_argument, 0, 1002 },
-        { "primed", no_argument, 0, 1003 },
+        { "primed", no_argument, 0, 1003 },      { "offset", required_argument, 0, 1004 },
+        { "size", required_argument, 0, 1005 },  { "reindex", no_argument, 0, 1006 },
         { 0, 0, 0, 0 },
     };
     int opt;
@@ -480,6 +624,14 @@ int main(int argc, char **argv)
         if (opt == 1000) { gzi_path = optarg; continue; }
         if (opt == 1001) { ndevices = atoi(optarg); if (ndevices < 1 || ndevices > 64) bad = 1; continue; }
         if (opt == 'b') { bsize = atoi(optarg); continue; }
+        if (opt == 1004 || opt == 1005) {
+            char *e = NULL;
+            const unsigned long long v = strtoull(optarg, &e, 10);
+            if (!*optarg || *e || *optarg == '-') bad = 1;
+            if (opt == 1004) { range_offset = v; have_offset = 1; } else { range_size = v; have_size = 1; }
+            continue;
+        }
+        if (opt == 1006) { reindex = 1; continue; }
         if (opt == 'h' || opt == '?') { bad = 1; continue; }
         for (size_t k = 0; k < NFLAGS; k++)
             if (k_flags[k].short_opt == opt)
@@ -488,6 +640,19 @@ int main(int argc, char **argv)
     int chosen = -1, nchosen = 0, level_sum = 0;
     for (size_t k = 0; k < NFLAGS; k++)
         if (levels[k]) { chosen = (int)k; nchosen++; level_sum += levels[k]; }
+    /* random access (7bgzf only): -d --offset [--size] [--gzi], and --reindex --gzi */
+    if ((have_offset || have_size || reindex) && !bad) {
+        if (kind || (reindex && (decompress || nchosen || have_offset || have_size || !gzi_path)) ||
+            (!reindex && (!decompress || nchosen || !have_offset))) {
+            usage(argv[0]);
+            return 1;
+        }
+        if (isatty(fileno(stdin)) || (!reindex && isatty(fileno(stdout)))) {
+            usage(argv[0]);
+            return -1;
+        }
+        return reindex ? reindex_applet(gzi_path) : range_applet(range_offset, range_size, have_size, gzi_path);
+    }
     if (bad || (!decompress && nchosen != 1) || (decompress && nchosen != 0)) {
         usage(argv[0]);
         return 1;

@@ -10,7 +10,7 @@ CSRC      := $(PKG)/csrc
 HOST      := $(PKG)/host
 OBJ       := build/obj
 
-CU_SRCS   := $(CSRC)/bgzf_compress.cu $(CSRC)/bgzf_inflate.cu $(CSRC)/b200bgzf_api.cu
+CU_SRCS   := $(CSRC)/bgzf_compress.cu $(CSRC)/bgzf_inflate.cu $(CSRC)/bgzf_ranges.cu $(CSRC)/b200bgzf_api.cu
 CU_OBJS   := $(patsubst $(CSRC)/%.cu,$(OBJ)/%.o,$(CU_SRCS))
 HDRS      := $(wildcard $(CSRC)/*.h) include/b200bgzf.h
 

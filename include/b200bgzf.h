@@ -111,6 +111,54 @@ int b200bgzf_inflate_host(b200bgzf_ctx *ctx, const void *in, size_t in_bytes, vo
                           unsigned flags);
 
 /*
+ * Random access (SURVEY §8(f) rank 2, the reading half of the index above): decode only the members that a list of byte
+ * ranges needs.  No GPU involved in the two index helpers.
+ *
+ * b200bgzf_index_host walks the member headers (any flavour b200bgzf_member_header accepts) and lists the start of every
+ * member, the EOF marker and other empty members included, as (compressed offset, uncompressed offset) pairs.
+ * b200bgzf_gzi_parse reads a .gzi (the inverse of b200bgzf_gzi_format) and puts back the implicit (0, 0) first entry; it
+ * refuses a file whose size does not match its entry count and entries that are not ascending (compressed offsets
+ * strictly, uncompressed offsets never going down).  Both store min(count, cap) pairs and set *nmembers to the count;
+ * with cap below the count (caddr / uaddr may then be NULL) they return B200BGZF_E_NOSPACE.
+ */
+#define B200BGZF_RANGE_VOFFSET 8u   /* ranges are [vbeg, vend) BGZF virtual offsets (coffset << 16 | uoffset), not uncompressed offsets */
+typedef struct b200bgzf_range {
+    uint64_t beg, end;
+} b200bgzf_range;
+int b200bgzf_index_host(const void *in, size_t in_bytes, uint64_t *caddr, uint64_t *uaddr, size_t cap, size_t *nmembers);
+int b200bgzf_gzi_parse(const void *gzi, size_t gzi_bytes, uint64_t *caddr, uint64_t *uaddr, size_t cap, size_t *nmembers);
+
+/*
+ * Decode byte ranges of a stream.
+ *   Output     the ranges' bytes back to back in the caller's order; range_off[i] (optional, nranges entries) = where range i
+ *              starts in `out`, *out_bytes = the total.  out_cap too small (or out NULL with a non-empty result): returns
+ *              B200BGZF_E_NOSPACE with *out_bytes = the size needed, before any member is decoded.
+ *   Ranges     any order, may overlap, may be empty.  A member that several ranges touch is decoded once per call (the host
+ *              variant cuts the call into groups of consecutive ranges of at most 256 MiB of decoded members + output each;
+ *              a member shared by two groups is decoded by both).
+ *   Offsets    uncompressed: beg <= end <= total decoded size, else B200BGZF_E_ARG.  B200BGZF_RANGE_VOFFSET: [vbeg, vend)
+ *              virtual offsets as a .bai / .csi query returns its chunks; vbeg <= vend, coffset a member start (listed in
+ *              the index when one is given) or in_bytes with uoffset 0 (the end), uoffset <= that member's ISIZE, else
+ *              B200BGZF_E_ARG.  An empty member (the EOF marker) never starts a range.
+ *   Index      host variant: caddr / uaddr (nindex entries, as b200bgzf_index_host or b200bgzf_gzi_parse give them) or NULL,
+ *              and the index is then built by a header walk.  With an index, the call reads only the compressed bytes of
+ *              the members it touches and the header and trailer of the last listed member (for the total size).
+ *   Verify     B200BGZF_VERIFY checks the CRC-32 of every decoded member (B200BGZF_E_CRC).  A corrupt member that is
+ *              touched gives B200BGZF_E_FORMAT; one that is not touched is never read.
+ *   Formats    host: what b200bgzf_inflate_host accepts.  Device: BGZF only (like b200bgzf_inflate_device, whose device
+ *              index it builds); the ranges and range_off are host arrays, d_in / d_out device memory, and the decoded
+ *              members go through a scratch buffer of at most 1 GiB in the context (more touched members: several
+ *              passes).  Synchronises before returning.
+ * One member decodes on one warp in 4-5 ms; these calls are built for batches of ranges (thousands of members side by
+ * side), not for the latency of one small query.
+ */
+int b200bgzf_inflate_ranges_host(b200bgzf_ctx *ctx, const void *in, size_t in_bytes, const uint64_t *caddr, const uint64_t *uaddr,
+                                 size_t nindex, const b200bgzf_range *ranges, size_t nranges, void *out, size_t out_cap,
+                                 size_t *out_bytes, uint64_t *range_off, unsigned flags);
+int b200bgzf_inflate_ranges_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, const b200bgzf_range *ranges, size_t nranges,
+                                   void *d_out, size_t out_cap, size_t *out_bytes, uint64_t *range_off, unsigned flags, void *stream);
+
+/*
  * Inflate a list of units found by the caller — what the readers of the indexed containers need (dictzip's chunk table,
  * RAZF's block index, GZinga's member index: applet/7dictzip.c:320-400, 7razf.c:293-384, 7gzinga.c:218-307).  A unit is either
  * a gzip member (piece = 0: hdr_len bytes of header, DEFLATE data, CRC32 + ISIZE; out_len is ignored, ISIZE counts) or a raw
