@@ -32,6 +32,7 @@ EXPORTS = [
     "b200bgzf_inflate_units_host", "b200bgzf_container_units", "b200bgzf_units_free", "b200bgzf_container_inflate_host",
     "b200bgzf_multi_container_bound", "b200bgzf_multi_container_compress_host", "b200bgzf_container_inflate_size",
     "b200bgzf_index_host", "b200bgzf_gzi_parse", "b200bgzf_inflate_ranges_host", "b200bgzf_inflate_ranges_device",
+    "b200bgzf_gzip_inflate_device",
 ]
 CONTAINER_GZIP, CONTAINER_MIGZ, CONTAINER_GZINGA, CONTAINER_DICTZIP, CONTAINER_RAZF = 1, 2, 3, 4, 5
 
@@ -80,6 +81,7 @@ def load(path=LIB_PATH):
     lib.b200bgzf_inflate_size_host.argtypes = [vp, sz, psz, psz]
     lib.b200bgzf_inflate_device.argtypes = [vp, vp, sz, vp, sz, psz, ctypes.c_uint, vp]
     lib.b200bgzf_inflate_host.argtypes = [vp, vp, sz, vp, sz, psz, ctypes.c_uint]
+    lib.b200bgzf_gzip_inflate_device.argtypes = [vp, vp, sz, vp, sz, psz, ctypes.c_uint, vp]
     lib.b200bgzf_profile.argtypes = [vp, i32, ctypes.POINTER(ctypes.c_ulonglong), i32, i32]
     lib.b200bgzf_launch_count.argtypes = [vp]
     lib.b200bgzf_launch_count.restype = ctypes.c_ulonglong
@@ -308,6 +310,12 @@ class Codec:
     def inflate_device(self, d_in, nbytes, d_out, out_cap, flags=0, stream=None):
         n = ctypes.c_size_t()
         self._check(self.lib.b200bgzf_inflate_device(self.h, d_in, nbytes, d_out, out_cap, ctypes.byref(n), flags, stream))
+        return n.value
+
+    def gzip_inflate_device(self, d_in, nbytes, d_out, out_cap, flags=0, stream=None):
+        """One whole-stream gzip member in device memory -> d_out; returns the decoded size (b200bgzf_gzip_inflate_device)."""
+        n = ctypes.c_size_t()
+        self._check(self.lib.b200bgzf_gzip_inflate_device(self.h, d_in, nbytes, d_out, out_cap, ctypes.byref(n), flags, stream))
         return n.value
 
     # ---- random access ----

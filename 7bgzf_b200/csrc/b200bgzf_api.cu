@@ -25,6 +25,7 @@
 
 #include "../../include/b200bgzf.h"
 #include "bgzf_block.h"
+#include "bgzf_gzip_route.h"
 #include "bgzf_kernels.h"
 #include "bgzf_tables.h"
 
@@ -110,6 +111,17 @@ struct Combiner {
     std::atomic<bool> stop{false}, sleeping{false};
 };
 
+/* whole-stream gzip: device workspaces of b200bgzf_gzip_inflate_device and the GZIP container reader (grown on demand) */
+struct GzWork {
+    uint32_t *tile_count = nullptr, *u32 = nullptr, *small32 = nullptr;
+    uint64_t *tile_off = nullptr, *u64 = nullptr, *small64 = nullptr, *h = nullptr;
+    uint16_t *scratch = nullptr;
+    uint8_t *d_in = nullptr, *d_out = nullptr;
+    size_t tiles_cap = 0, tileoff_cap = 0, u32_cap = 0, u64_cap = 0, scratch_cap = 0, in_cap = 0, out_cap = 0, h_cap = 0;
+    cudaStream_t copy = nullptr;      /* D2H of finished batches (host reader), behind the batch's event */
+    cudaEvent_t ev = nullptr;
+};
+
 }  // namespace
 
 struct b200bgzf_ctx {
@@ -134,6 +146,7 @@ struct b200bgzf_ctx {
     uint64_t *d_rng_mem = nullptr, *d_rng_rw = nullptr, *d_rng_counts = nullptr, *h_rng = nullptr, *h_rng_soff = nullptr;
     uint8_t *d_rng_scratch = nullptr;
     size_t rng_mem_cap = 0, rng_rw_cap = 0, rng_scratch_cap = 0, h_rng_cap = 0, h_rng_soff_cap = 0;
+    GzWork gz;
     /* Completion thread (hook callers beyond the host's core count): callers neither spin nor poll, they sleep on their
      * lane's futex word; this one thread polls the events of the lanes in flight and wakes each caller as its member is back */
     std::thread waiter;
@@ -436,6 +449,12 @@ extern "C" void b200bgzf_destroy(b200bgzf_ctx *ctx)
         cudaFree(ctx->d_rng_mem); cudaFree(ctx->d_rng_rw); cudaFree(ctx->d_rng_counts); cudaFree(ctx->d_rng_scratch);
         if (ctx->h_rng) cudaFreeHost(ctx->h_rng);
         if (ctx->h_rng_soff) cudaFreeHost(ctx->h_rng_soff);
+        GzWork &z = ctx->gz;
+        cudaFree(z.tile_count); cudaFree(z.u32); cudaFree(z.small32); cudaFree(z.tile_off); cudaFree(z.u64); cudaFree(z.small64);
+        cudaFree(z.scratch); cudaFree(z.d_in); cudaFree(z.d_out);
+        if (z.h) cudaFreeHost(z.h);
+        if (z.copy) cudaStreamDestroy(z.copy);
+        if (z.ev) cudaEventDestroy(z.ev);
     }
     delete ctx;
 }
@@ -1423,6 +1442,299 @@ extern "C" int b200bgzf_inflate_units_host(b200bgzf_ctx *ctx, const void *in, si
         return out_bytes ? B200BGZF_OK : B200BGZF_E_ARG;
     }
     return inflate_host_impl(ctx, in, in_bytes, units, nunits, out, out_cap, out_bytes, flags, unit_crc);
+}
+
+/* ------------------------------------------------------------------------------------------------ */
+/* whole-stream gzip: one member, inflated in parallel between its byte-aligned flush points (bgzf_gzip.cu)               */
+
+namespace {
+
+/* Scratch (2 bytes per output byte of the chunks in flight) stays under this; B200BGZF_GZIP_BUDGET (bytes, at least 1 MiB)
+ * lowers it, so that the multi-batch path can be exercised on small inputs. */
+uint64_t gzip_budget()
+{
+    static const uint64_t b = [] {
+        const char *e = getenv("B200BGZF_GZIP_BUDGET");
+        const unsigned long long v = e && *e ? strtoull(e, nullptr, 10) : 0ull;
+        return v >= (1ull << 20) && v < (1ull << 30) ? (uint64_t)v : (uint64_t)1 << 30;
+    }();
+    return b;
+}
+
+constexpr uint64_t kGzMaxChunkIn = 4ull << 20;   /* compressed bytes one chunk may span: bounds a false candidate's garbage decode */
+constexpr uint32_t kGzCrcPiece = 1u << 20;       /* B200BGZF_VERIFY: output bytes per CRC unit of bgzf_verify_kernel */
+
+/* Decodes the member d_in[0, in_bytes) (header of hlen bytes, trailer isize / want_crc) into d_out through its flush-point chain.
+ * Returns BGZF_GZIP_FALLBACK when the member has no complete chain (no flush point, a chunk over the caps, a chain that ends
+ * anywhere but at the trailer, a decode that differs from the boundary pass): the one-warp path then gives the outcome.
+ * on_batch(base, bytes) is called after the launches that write output [base, base + bytes). */
+template <typename F>
+int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, uint32_t hlen, uint32_t isize, uint32_t want_crc,
+                       uint8_t *d_out, size_t out_cap, size_t *total_out, unsigned flags, cudaStream_t stream, F on_batch)
+{
+    GzWork &z = ctx->gz;
+    const uint64_t data_len = in_bytes - hlen - 8;
+    if (data_len == 0) return BGZF_GZIP_FALLBACK;
+    const size_t tiles = bgzf_gzip_tiles(data_len);
+    CK(grow(&z.tile_count, &z.tiles_cap, tiles));
+    CK(grow(&z.tile_off, &z.tileoff_cap, tiles));
+    size_t c64 = z.small64 ? 8 : 0, c32 = z.small32 ? 8 : 0, hc = z.h_cap;
+    CK(grow(&z.small64, &c64, 8));
+    CK(grow(&z.small32, &c32, 8));
+    CK(grow(&z.h, &hc, 8, true));
+    z.h_cap = hc;
+    BgzfGzipArgs a;
+    memset(&a, 0, sizeof a);
+    a.data = d_in + hlen;
+    a.data_len = data_len;
+    a.max_in = kGzMaxChunkIn;
+    a.tile_count = z.tile_count;
+    a.tile_off = z.tile_off;
+    a.counts = z.small64;
+    a.ncand = z.small64 + 1;
+    a.nchunks = z.small64 + 2;
+    a.total = z.small64 + 3;
+    a.chain_status = z.small32;
+    a.err = z.small32 + 1;
+    a.out = d_out;
+    CK(cudaMemsetAsync(z.small64, 0, 8 * sizeof(uint64_t), stream));
+    CK(cudaMemsetAsync(z.small32, 0, 8 * sizeof(uint32_t), stream));
+    /* 1. flush points: count, then size the candidate arrays by it */
+    CK(bgzf_launch_gzip_count(&a, stream));
+    ctx->launches += 3;
+    CK(cudaMemcpyAsync(z.h, z.small64, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    const uint64_t nc = z.h[0] + 1;
+    if (nc < 2 || nc > 0xfffffff0ull) return BGZF_GZIP_FALLBACK;
+    /* u64: cand, end, pick, c_start, c_off; u32: olen, status, c_len, lastm, anchor, jump, jump2, reach */
+    CK(grow(&z.u64, &z.u64_cap, 5 * nc));
+    CK(grow(&z.u32, &z.u32_cap, 8 * (nc + 2)));
+    a.cand = z.u64; a.end = z.u64 + nc; a.pick = z.u64 + 2 * nc; a.c_start = z.u64 + 3 * nc; a.c_off = z.u64 + 4 * nc;
+    uint32_t *q = z.u32;
+    a.olen = q; a.status = q + nc; a.c_len = q + 2 * nc; a.lastm = q + 3 * nc; a.anchor = q + 4 * nc;
+    a.jump = q + 5 * nc; a.jump2 = q + 6 * nc + 2; a.reach = q + 7 * nc + 4;
+    /* 2. boundary pass, chain from the data start, chunk offsets */
+    CK(bgzf_launch_gzip_chain(&a, (uint32_t)nc, stream));
+    ctx->launches += BGZF_GZIP_CHAIN_LAUNCHES;
+    CK(cudaMemcpyAsync(z.h, z.small64, 4 * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaMemcpyAsync(z.h + 4, z.small32, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    if ((uint32_t)z.h[4] & 1u) return BGZF_GZIP_FALLBACK;
+    const uint64_t nchunks = z.h[2], total = z.h[3];
+    if (nchunks == 0 || nchunks > nc) return BGZF_GZIP_FALLBACK;
+    /* the chain is the sequential decoder's exact bit path: its length is what that decoder would produce */
+    *total_out = (size_t)total;
+    if ((uint32_t)total != isize) return B200BGZF_E_FORMAT;
+    if (total > out_cap || (!d_out && total)) return B200BGZF_E_NOSPACE;
+    /* 3. batches of chained chunks whose scratch fits the budget */
+    const uint64_t win = bgzf_gzip_window(), budget = gzip_budget();
+    std::vector<uint64_t> cut;                      /* batch boundaries (chunk indices) */
+    if (2 * (win + total) <= budget) {
+        cut = { 0, nchunks };
+    } else {
+        std::vector<uint64_t> off(nchunks + 1);
+        CK(cudaMemcpyAsync(off.data(), a.c_off, nchunks * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        off[nchunks] = total;
+        cut.push_back(0);
+        uint64_t j = 0;
+        while (j < nchunks) {
+            uint64_t j1 = j + 1;
+            if (2 * (win + off[j1] - off[j]) > budget) return BGZF_GZIP_FALLBACK;   /* one chunk alone is over the budget */
+            while (j1 < nchunks && 2 * (win + off[j1 + 1] - off[j]) <= budget) j1++;
+            cut.push_back(j1);
+            j = j1;
+        }
+    }
+    uint64_t most = 0;
+    std::vector<uint64_t> base(cut.size());
+    {
+        std::vector<uint64_t> off0(cut.size());
+        for (size_t i = 0; i < cut.size(); i++) {
+            if (cut[i] == nchunks) { off0[i] = total; continue; }
+            CK(cudaMemcpyAsync(&off0[i], a.c_off + cut[i], sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+        }
+        CK(cudaStreamSynchronize(stream));
+        for (size_t i = 0; i + 1 < cut.size(); i++) most = std::max(most, off0[i + 1] - off0[i]);
+        base = off0;
+    }
+    CK(grow(&z.scratch, &z.scratch_cap, win + most + 16));
+    a.scratch = z.scratch;
+    for (size_t i = 0; i + 1 < cut.size(); i++) {
+        CK(bgzf_launch_gzip_batch(&a, (uint32_t)cut[i], (uint32_t)cut[i + 1], base[i], base[i + 1] - base[i], stream));
+        ctx->launches += BGZF_GZIP_BATCH_LAUNCHES;
+        if (int r = on_batch(base[i], base[i + 1] - base[i])) return r;
+    }
+    /* 4. B200BGZF_VERIFY: CRC-32 of 1 MiB units of the output (bgzf_verify_kernel's tiles), combined here */
+    const bool verify = (flags & B200BGZF_VERIFY) != 0;
+    const uint64_t nu = verify ? (total + kGzCrcPiece - 1) / kGzCrcPiece : 0;
+    std::vector<uint32_t> hcrc(nu);
+    if (nu) {
+        /* u64: in_off (0), out_off; u32: hdr_len (0), msize (0), unit_isize, status (0), unit_crc */
+        size_t un64 = 0, un32 = 0;
+        uint64_t *d64 = nullptr;
+        uint32_t *d32 = nullptr;
+        CK(grow(&d64, &un64, 2 * nu));
+        if (cudaError_t e = grow(&d32, &un32, 5 * nu)) { cudaFree(d64); return fail(ctx, e, "grow"); }
+        std::vector<uint64_t> h64(2 * nu, 0);
+        std::vector<uint32_t> h32(5 * nu, 0);
+        for (uint64_t u = 0; u < nu; u++) {
+            h64[nu + u] = u * kGzCrcPiece;
+            h32[2 * nu + u] = (uint32_t)std::min<uint64_t>(kGzCrcPiece, total - u * kGzCrcPiece);
+        }
+        cudaError_t e = cudaMemcpyAsync(d64, h64.data(), h64.size() * 8, cudaMemcpyHostToDevice, stream);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(d32, h32.data(), h32.size() * 4, cudaMemcpyHostToDevice, stream);
+        BgzfInflateArgs v;
+        memset(&v, 0, sizeof v);
+        v.in = d_out;
+        v.in_off = d64;
+        v.out_off = d64 + nu;
+        v.hdr_len = d32;
+        v.msize = d32 + nu;
+        v.unit_isize = d32 + 2 * nu;
+        v.status = d32 + 3 * nu;
+        v.unit_crc = d32 + 4 * nu;
+        v.nblocks = (uint32_t)nu;
+        v.out = d_out;
+        v.err_flag = a.err + 2;
+        v.verify_crc = 1;
+        v.crctab = ctx->d_crctab;
+        v.crcpow = ctx->d_crcpow;
+        if (e == cudaSuccess) e = bgzf_launch_verify(&v, stream);
+        ctx->launches += 1;
+        if (e == cudaSuccess) e = cudaMemcpyAsync(hcrc.data(), v.unit_crc, nu * 4, cudaMemcpyDeviceToHost, stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(stream);
+        cudaFree(d64);
+        cudaFree(d32);
+        if (e != cudaSuccess) return fail(ctx, e, "gzip verify");
+    }
+    CK(cudaMemcpyAsync(z.h + 5, a.err, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    if ((uint32_t)z.h[5]) return BGZF_GZIP_FALLBACK;    /* (a back-reference before the member start: the one-warp path reports it) */
+    if (verify) {
+        uint32_t crc = 0;
+        for (uint64_t u = 0; u < nu; u++) crc = u ? b200bgzf_crc32_combine(crc, hcrc[u], std::min<uint64_t>(kGzCrcPiece, total - u * kGzCrcPiece)) : hcrc[u];
+        if (crc != want_crc) return B200BGZF_E_CRC;
+    }
+    return B200BGZF_OK;
+}
+
+/* the checks the one-warp path makes of a member before decoding it (inflate_host_impl): 0 or B200BGZF_E_FORMAT */
+int gzip_member_check(size_t in_bytes, uint32_t hlen, uint32_t isize)
+{
+    if (!hlen || in_bytes < (size_t)hlen + 10 || in_bytes > 0xffffffffull || hlen > 0xffffu) return B200BGZF_E_FORMAT;
+    if (isize > 0x7fffffffu || isize > 1032ull * (in_bytes - hlen) + 1032u) return B200BGZF_E_FORMAT;
+    return 0;
+}
+
+}  // namespace
+
+extern "C" int b200bgzf_gzip_inflate_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, void *d_out, size_t out_cap,
+                                            size_t *out_bytes, unsigned flags, void *stream_)
+{
+    if (!ctx || !d_in || !out_bytes) return B200BGZF_E_ARG;
+    *out_bytes = 0;
+    if (in_bytes < 18) return B200BGZF_E_FORMAT;
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    int r = lane_reserve(ctx, l, 1, 0, 0, false);
+    if (r) return r;
+    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : l.stream;
+    GzWork &z = ctx->gz;
+    const uint8_t *in = (const uint8_t *)d_in;
+    /* the header (FEXTRA, FNAME, FCOMMENT, FHCRC) in small reads, growing while a field runs past what was read; the trailer */
+    std::vector<uint8_t> head;
+    uint8_t tr[8];
+    size_t hlen = 0, xoff, xlen;
+    for (size_t want = std::min<size_t>(in_bytes, 4096);; want = std::min(in_bytes, want * 4)) {
+        head.resize(want);
+        CK(cudaMemcpyAsync(head.data(), in, want, cudaMemcpyDeviceToHost, stream));
+        CK(cudaMemcpyAsync(tr, in + in_bytes - 8, 8, cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        hlen = bgzf_gz_header(head.data(), want, &xoff, &xlen);
+        if (hlen || want == in_bytes || head.size() < 10 || head[0] != 0x1f || head[1] != 0x8b) break;
+    }
+    const uint32_t want_crc = rd32(tr), isize = rd32(tr + 4);
+    if ((r = gzip_member_check(in_bytes, (uint32_t)hlen, isize))) return r;
+    size_t total = isize;
+    r = gzip_chain_inflate(ctx, in, in_bytes, (uint32_t)hlen, isize, want_crc, (uint8_t *)d_out, d_out ? out_cap : 0, &total, flags, stream,
+                           [](uint64_t, uint64_t) { return 0; });
+    *out_bytes = total;
+    if (r != BGZF_GZIP_FALLBACK) return r;
+    /* no usable flush points: one warp decodes the member, as b200bgzf_inflate_units_host does */
+    *out_bytes = isize;
+    if (isize > out_cap || (!d_out && isize)) return B200BGZF_E_NOSPACE;
+    size_t c64 = z.small64 ? 8 : 0, c32 = z.small32 ? 8 : 0, hc = z.h_cap;
+    CK(grow(&z.small64, &c64, 8));
+    CK(grow(&z.small32, &c32, 8));
+    CK(grow(&z.h, &hc, 8, true));
+    z.h_cap = hc;
+    uint32_t *h32 = (uint32_t *)z.h;
+    z.h[0] = 0;                                          /* in_off, out_off */
+    z.h[1] = 0;
+    h32[4] = (uint32_t)hlen;                             /* hdr_len, msize, status, err_flag */
+    h32[5] = (uint32_t)in_bytes;
+    h32[6] = 0;
+    h32[7] = 0;
+    CK(cudaMemcpyAsync(z.small64, z.h, 2 * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+    CK(cudaMemcpyAsync(z.small32, h32 + 4, 4 * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    BgzfInflateArgs a;
+    memset(&a, 0, sizeof a);
+    a.in = in;
+    a.in_off = z.small64;
+    a.out_off = z.small64 + 1;
+    a.hdr_len = z.small32;
+    a.msize = z.small32 + 1;
+    a.status = z.small32 + 2;
+    a.err_flag = z.small32 + 3;
+    a.nblocks = 1;
+    a.out = (uint8_t *)d_out;
+    a.crctab = ctx->d_crctab;
+    a.crcpow = ctx->d_crcpow;
+    a.verify_crc = (flags & B200BGZF_VERIFY) ? 1 : 0;
+    CK(bgzf_launch_inflate(&a, stream));
+    ctx->launches += 1 + a.verify_crc;
+    CK(cudaMemcpyAsync(z.h + 2, a.err_flag, sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    const uint32_t ef = (uint32_t)z.h[2];
+    return (ef & 1u) ? B200BGZF_E_FORMAT : (ef & 2u) ? B200BGZF_E_CRC : B200BGZF_OK;
+}
+
+/* the GZIP container reader's route (host/containers.c): the member goes to the device, finished batches come back while the
+ * next ones decode; BGZF_GZIP_FALLBACK hands the member to the one-warp path */
+extern "C" int bgzf_gzip_inflate_host(b200bgzf_ctx *ctx, const void *in_, size_t in_bytes, uint32_t hlen, void *out, size_t out_cap,
+                                      size_t *out_bytes, unsigned flags)
+{
+    const uint8_t *in = (const uint8_t *)in_;
+    if (!ctx || !in || !out_bytes || in_bytes < (size_t)hlen + 10) return BGZF_GZIP_FALLBACK;
+    const uint32_t want_crc = rd32(in + in_bytes - 8), isize = rd32(in + in_bytes - 4);
+    if (gzip_member_check(in_bytes, hlen, isize) || isize > out_cap || (!out && isize)) return BGZF_GZIP_FALLBACK;
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    int r = lane_reserve(ctx, l, 1, 0, 0, false);
+    if (r) return r;
+    GzWork &z = ctx->gz;
+    if (!z.copy) CK(cudaStreamCreateWithFlags(&z.copy, cudaStreamNonBlocking));
+    if (!z.ev) CK(cudaEventCreateWithFlags(&z.ev, cudaEventDisableTiming));
+    CK(grow(&z.d_in, &z.in_cap, in_bytes + 64));
+    CK(grow(&z.d_out, &z.out_cap, (size_t)isize + 64));
+    CK(cudaMemcpyAsync(z.d_in, in, in_bytes, cudaMemcpyHostToDevice, l.stream));
+    size_t total = isize;
+    r = gzip_chain_inflate(ctx, z.d_in, in_bytes, hlen, isize, want_crc, z.d_out, isize, &total, flags, l.stream,
+                           [&](uint64_t base, uint64_t bytes) -> int {
+                               if (!bytes) return 0;
+                               CK(cudaEventRecord(z.ev, l.stream));
+                               CK(cudaStreamWaitEvent(z.copy, z.ev, 0));
+                               CK(cudaMemcpyAsync((uint8_t *)out + base, z.d_out + base, bytes, cudaMemcpyDeviceToHost, z.copy));
+                               return 0;
+                           });
+    const cudaError_t e = cudaStreamSynchronize(z.copy);
+    if (r == B200BGZF_E_NOSPACE) r = B200BGZF_E_FORMAT;   /* (more output than ISIZE: the one-warp path's overrun) */
+    if (r == B200BGZF_OK || r == B200BGZF_E_CRC) *out_bytes = isize;
+    if (e != cudaSuccess && r != BGZF_GZIP_FALLBACK) return fail(ctx, e, "gzip copy");
+    return r;
 }
 
 /* ------------------------------------------------------------------------------------------------ */

@@ -125,6 +125,31 @@ struct BgzfRangeGatherArgs {
     uint32_t nranges;
 };
 
+/* whole-stream gzip (bgzf_gzip.cu): one member inflated in chunks cut at its byte-aligned flush points (all device memory) */
+struct BgzfGzipArgs {
+    const uint8_t *data;       /* the member's DEFLATE data (after the header) */
+    uint64_t data_len;         /* its bytes up to the 8-byte trailer */
+    uint64_t max_in;           /* compressed bytes one chunk may span (a longer one ends the parallel attempt) */
+    uint32_t *tile_count;      /* [tiles] candidates per 32 KiB tile */
+    uint64_t *tile_off;        /* [tiles] their exclusive scan */
+    uint64_t *counts;          /* [4]: candidates found by the scan, candidates (+ the data start), chained chunks, output bytes */
+    const uint64_t *ncand, *nchunks;   /* counts + 1, counts + 2 */
+    uint64_t *total;           /* counts + 3 */
+    uint64_t *cand;            /* [ncand] candidate offsets in the DEFLATE data, ascending; cand[0] = 0 */
+    uint64_t *end;             /* [ncand] where each candidate's chunk ends */
+    uint32_t *olen, *status;   /* [ncand] its output bytes, how it ended */
+    uint32_t *jump, *jump2, *reach;   /* [ncand + 2] successor links (pointer doubling) and the chain from candidate 0 */
+    uint64_t *pick;            /* [ncand] exclusive scan of reach[] */
+    uint32_t *chain_status;    /* bit 0: the chain from candidate 0 does not reach the end of the data */
+    uint64_t *c_start;         /* [nchunks] the chained chunks: start in the DEFLATE data */
+    uint32_t *c_len;           /* [nchunks] output bytes */
+    uint64_t *c_off;           /* [nchunks] output offset in the member */
+    uint32_t *lastm, *anchor;  /* [nchunks] one past the last marker a chunk wrote; 1 = its preceding 32 KiB hold no marker */
+    uint16_t *scratch;         /* 32 KiB before the batch + the batch's output, one u16 per byte */
+    uint8_t *out;              /* the member's output */
+    uint32_t *err;             /* bit 0: a back-reference before the member start, bit 1: a chunk decoded differently */
+};
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -141,9 +166,21 @@ cudaError_t bgzf_launch_compact(const uint8_t *slots, const uint32_t *len, uint6
 cudaError_t bgzf_launch_deliver(const uint8_t *slots, const uint32_t *len, const uint64_t *out_off, uint8_t *host_out, uint32_t n,
                                 cudaStream_t stream);
 size_t bgzf_index_tiles(uint64_t in_bytes);
+size_t bgzf_gzip_tiles(uint64_t data_len);
+size_t bgzf_gzip_window(void);
+cudaError_t bgzf_launch_gzip_count(const BgzfGzipArgs *a, cudaStream_t stream);    /* counts[0] = flush points found */
+cudaError_t bgzf_launch_gzip_chain(const BgzfGzipArgs *a, uint32_t ncand, cudaStream_t stream);
+cudaError_t bgzf_launch_gzip_batch(const BgzfGzipArgs *a, uint32_t j0, uint32_t j1, uint64_t base, uint64_t bytes, cudaStream_t stream);
+#define BGZF_GZIP_CHAIN_LAUNCHES 8
+#define BGZF_GZIP_BATCH_LAUNCHES 5
 #define BGZF_INDEX_LAUNCHES 8
 cudaError_t bgzf_launch_index(const uint8_t *in, uint64_t in_bytes, const BgzfIndexWork *w, cudaStream_t stream);
 cudaError_t bgzf_launch_inflate(const BgzfInflateArgs *a, cudaStream_t stream);
+cudaError_t bgzf_launch_verify(const BgzfInflateArgs *a, cudaStream_t stream);   /* bgzf_verify_kernel alone */
+/* pointer doubling over successor links (bgzf_index_chain_kernel): reach[k] = 1 for every candidate on the chain from
+ * candidate 0 (which must lie at offset 0); status bit 0 = the chain does not end at node `count` ("the end") */
+cudaError_t bgzf_launch_chain(const uint64_t *cand_off, const uint64_t *count, uint32_t max_blocks, uint32_t *jump,
+                              uint32_t *jump2, uint32_t *reach, uint32_t *status, cudaStream_t stream);
 #ifdef __cplusplus
 }
 #endif

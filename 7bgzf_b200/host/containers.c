@@ -17,6 +17,7 @@
 #include <stdio.h>
 
 #include "../../include/b200bgzf.h"
+#include "../csrc/bgzf_gzip_route.h"
 
 #define PIECE_MAX 65280u          /* the BGZF rule (applet/7bgzf.c:146-147): a stored piece and its framing fit 64 KiB */
 #define DICTZIP_MAX_CHUNKS 32762u /* (0xffff - 10) / 2: the chunk table must fit XLEN (applet/7dictzip.c:178) */
@@ -343,6 +344,8 @@ static size_t gz_header(const uint8_t *p, size_t avail, size_t *xoff, size_t *xl
     return n <= avail ? n : 0;
 }
 
+size_t bgzf_gz_header(const uint8_t *p, size_t avail, size_t *xoff, size_t *xlen) { return gz_header(p, avail, xoff, xlen); }
+
 /* a member made of pieces: units [first, first + count) together must have the CRC-32 its trailer states */
 struct member_check {
     size_t first, count;
@@ -485,7 +488,8 @@ static int units_gzinga(const uint8_t *p, size_t n, struct unit_list *l)
     return start == idx ? B200BGZF_OK : B200BGZF_E_FORMAT;
 }
 
-/* plain gzip members one after another, each a single unit (no index: one warp per member) */
+/* plain gzip: one unit spanning the input (b200bgzf_container_inflate_host decodes it between its flush points where it has
+ * them, else on one warp) */
 static int units_gzip(const uint8_t *p, size_t n, struct unit_list *l)
 {
     /* without an index a member's end is only known once it is decoded: a single member is taken to span the input */
@@ -566,7 +570,13 @@ int b200bgzf_container_inflate_host(b200bgzf_ctx *ctx, int kind, const void *in,
          * (dictzip, RAZF) is combined here from those of its pieces (the reference's readers check neither) */
         if ((flags & B200BGZF_VERIFY) && l.nchk && !(crc = (uint32_t *)malloc(sizeof(uint32_t) * (l.n + 1)))) rc = B200BGZF_E_ARG;
         else if (l.out_bytes > out_cap) rc = B200BGZF_E_NOSPACE;
-        else rc = b200bgzf_inflate_units_host(ctx, in, in_bytes, l.u, l.n, out, out_cap, out_bytes, flags, crc);
+        else {
+            /* whole-stream gzip: in parallel between the member's flush points when it has a complete chain of them */
+            rc = kind == B200BGZF_CONTAINER_GZIP && l.n == 1
+                     ? bgzf_gzip_inflate_host(ctx, in, in_bytes, l.u[0].hdr_len, out, out_cap, out_bytes, flags)
+                     : BGZF_GZIP_FALLBACK;
+            if (rc == BGZF_GZIP_FALLBACK) rc = b200bgzf_inflate_units_host(ctx, in, in_bytes, l.u, l.n, out, out_cap, out_bytes, flags, crc);
+        }
     }
     if (rc == 0 && crc)
         for (size_t k = 0; k < l.nchk && rc == 0; k++) {

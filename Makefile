@@ -10,7 +10,7 @@ CSRC      := $(PKG)/csrc
 HOST      := $(PKG)/host
 OBJ       := build/obj
 
-CU_SRCS   := $(CSRC)/bgzf_compress.cu $(CSRC)/bgzf_inflate.cu $(CSRC)/bgzf_ranges.cu $(CSRC)/b200bgzf_api.cu
+CU_SRCS   := $(CSRC)/bgzf_compress.cu $(CSRC)/bgzf_inflate.cu $(CSRC)/bgzf_ranges.cu $(CSRC)/bgzf_gzip.cu $(CSRC)/b200bgzf_api.cu
 CU_OBJS   := $(patsubst $(CSRC)/%.cu,$(OBJ)/%.o,$(CU_SRCS))
 HDRS      := $(wildcard $(CSRC)/*.h) include/b200bgzf.h
 
@@ -21,7 +21,7 @@ $(OBJ)/%.o: $(CSRC)/%.cu $(HDRS)
 	@mkdir -p $(OBJ)
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> $(OBJ)/$*.ptxas.log || (cat $(OBJ)/$*.ptxas.log; false)
 
-$(OBJ)/%.o: $(HOST)/%.c include/b200bgzf.h
+$(OBJ)/%.o: $(HOST)/%.c include/b200bgzf.h $(CSRC)/bgzf_gzip_route.h
 	@mkdir -p $(OBJ)
 	$(CC) $(CFLAGS) -c $< -o $@
 

@@ -276,13 +276,34 @@ int b200bgzf_multi_container_compress_host(b200bgzf_multi *m, int kind, uint32_t
                                            void *out, size_t out_cap, size_t *out_bytes);
 
 /* The readers: the unit list of a dictzip / RAZF / GZinga file from its own index (a plain gzip member without an index is
- * one unit: one warp decodes it), to be released with b200bgzf_units_free; out_bytes = the decoded size.  No GPU involved.
+ * one unit spanning the input), to be released with b200bgzf_units_free; out_bytes = the decoded size.  No GPU involved.
  * b200bgzf_container_inflate_host = that list + b200bgzf_inflate_units_host (MiGz: b200bgzf_inflate_host, whose header
- * walk knows the "MZ" subfield). */
+ * walk knows the "MZ" subfield; GZIP: the member goes through b200bgzf_gzip_inflate_device's chunked decode, and only a
+ * member without a usable flush point is decoded by one warp, as the unit list says). */
 int b200bgzf_container_units(int kind, const void *in, size_t in_bytes, b200bgzf_unit **units, size_t *nunits, size_t *out_bytes);
 void b200bgzf_units_free(b200bgzf_unit *units);
 int b200bgzf_container_inflate_host(b200bgzf_ctx *ctx, int kind, const void *in, size_t in_bytes, void *out, size_t out_cap,
                                     size_t *out_bytes, unsigned flags);   /* flags: 0 or B200BGZF_VERIFY (CRC-32 of every member) */
+/*
+ * Whole-stream gzip on the device: one gzip member (RFC 1952; FEXTRA, FNAME, FCOMMENT and FHCRC accepted) in d_in[0, in_bytes),
+ * decoded into d_out.  Every block that follows a byte-aligned flush point — the empty stored block (00 00 ff ff) that our GZIP
+ * writer puts after every piece, that pigz puts after every chunk and that zlib's Z_SYNC_FLUSH / Z_FULL_FLUSH write — starts a
+ * chunk; the chunks are decoded side by side (one warp each) and their back-references across chunk starts resolved after.
+ * The chunks are accepted only when they chain from the data start to the trailer exactly as a sequential decoder walks them;
+ * otherwise (no flush point, a chunk of more than 4 MiB of compressed data or one whose output alone is over the scratch
+ * budget, a stream that does not end at the trailer, e.g. several members) one warp decodes the member, as
+ * b200bgzf_inflate_units_host does.  Either way the bytes, or the error, are those of that one-warp decode.
+ *   Output   *out_bytes = the decoded size; out_cap too small (or d_out NULL with a non-empty result): B200BGZF_E_NOSPACE with
+ *            *out_bytes = the size needed, before anything is decoded.  The decoded size must equal ISIZE (mod 2^32), else
+ *            B200BGZF_E_FORMAT.
+ *   Verify   B200BGZF_VERIFY checks the CRC-32 against the trailer (B200BGZF_E_CRC); without it a damaged stored byte decodes
+ *            silently, as in the one-warp path.
+ *   Memory   the header is read with small device-to-host copies.  Device scratch: 2 bytes per output byte of the chunks in
+ *            flight, in batches of at most 1 GiB (B200BGZF_GZIP_BUDGET, in bytes from 1 MiB, lowers it), plus ~50 bytes per
+ *            flush-point candidate.  Synchronises before returning.
+ */
+int b200bgzf_gzip_inflate_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, void *d_out, size_t out_cap, size_t *out_bytes,
+                                 unsigned flags, void *stream);
 /* decoded size (and number of units) of a container, to size the output: MiGz — and gzip input that turns out to be a
  * stream of members carrying their own size (BGZF, MiGz, mgzip) — by the header walk, the others by their index */
 int b200bgzf_container_inflate_size(int kind, const void *in, size_t in_bytes, size_t *out_bytes, size_t *nunits);
