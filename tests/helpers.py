@@ -61,6 +61,28 @@ def emul_block(payload, level=6, order=0):
     return rc, dst.raw[: dl.value]
 
 
+def emul_trees():
+    """the trees of the last emulated block's final pass: {btype, (used symbols, overflow) of "litlen", "dist", "precode"};
+    overflow = nodes deeper than the code's length limit (15, 15, 7), what the code-length repair starts from"""
+    lib = _emul()
+    lib.bgemul_last_trees.argtypes = [ctypes.POINTER(ctypes.c_uint32)]
+    lib.bgemul_last_trees.restype = None
+    v = (ctypes.c_uint32 * 7)()
+    lib.bgemul_last_trees(v)
+    return {"btype": v[0], "litlen": (v[1], v[2]), "dist": (v[3], v[4]), "precode": (v[5], v[6])}
+
+
+def emul_ties():
+    """ties in the last emulated block's distance and precode trees: {"dist" / "precode": (leaves of the same weight as
+    the leaf before them, merge picks where the lightest leaf and the lightest merged node weigh the same)}"""
+    lib = _emul()
+    lib.bgemul_last_ties.argtypes = [ctypes.POINTER(ctypes.c_uint32)]
+    lib.bgemul_last_ties.restype = None
+    v = (ctypes.c_uint32 * 4)()
+    lib.bgemul_last_ties(v)
+    return {"dist": (v[0], v[1]), "precode": (v[2], v[3])}
+
+
 def emul_piece(payload, level=6, head_gap=0, tail_gap=0, final=True, order=0, history=b""):
     """One block in piece mode (raw DEFLATE between `head_gap` and `tail_gap` free bytes): (slot bytes, CRC-32 of payload).
     history: the input right before the payload that matches may reach into (a multiple of 272 bytes, at most 32640)."""

@@ -5,6 +5,7 @@
 //
 //   emul compress <level> <in> <out.bgz> [order]   order: 0 forward, 1 reverse, 2 shuffled
 //   library: int bgemul_compress_block(const uint8_t* src, uint32_t n, int level, int order, uint8_t* dst /*65536*/, uint32_t* dlen)
+//            void bgemul_last_trees(uint32_t out[7]), bgemul_last_ties(uint32_t out[4])   the Huffman trees of the last block (see below)
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -41,7 +42,41 @@ void run(phase_fn f, const BgCtx &c, int order, uint32_t seed)
     }
     for (uint32_t t : idx) f(c, t, T);
 }
+
+/* the tree over the m ascending keys (m <= 32), built by the kernel's merge on copies: out[0] = the overflow the code-length
+ * repair of bg_huff_lengths() starts from (nodes deeper than maxbits), out[1] = leaves of the same weight as the leaf
+ * before them, out[2] = picks of the merge where the lightest leaf and the lightest merged node weigh the same (the leaf
+ * goes first) */
+void tree_stats(const uint32_t *keys, uint32_t m, uint32_t maxbits, uint32_t out[3])
+{
+    out[0] = out[1] = out[2] = 0;
+    if (m < 2) return;
+    uint32_t w[64];
+    uint16_t par[64];
+    for (uint32_t i = 0; i < m; i++) w[i] = keys[i] >> 9;
+    bg_huff_merge(m, w, par);
+    const uint32_t root = 2 * m - 2;
+    for (uint32_t i = 0; i < root; i++) {
+        uint32_t d = 0;
+        for (uint32_t x = i; x != root; x = par[x]) d++;
+        out[0] += d > maxbits;
+    }
+    for (uint32_t i = 1; i < m; i++) out[1] += w[i] == w[i - 1];
+    for (uint32_t a = 0, b = m, e = m; e < 2 * m - 1; e++)     /* the picks again, from the weights the merge left */
+        for (int k = 0; k < 2; k++) {
+            if (a < m && b < e && w[a] == w[b]) out[2]++;
+            if (a < m && (b >= e || w[a] <= w[b])) a++; else b++;
+        }
+}
 }  // namespace
+
+/* statistics of the trees of the last bgemul_compress_block call's final pass (the one it emits):
+ * BTYPE, then used symbols and overflow (nodes deeper than the length limit) of the litlen, distance and precode codes */
+static uint32_t g_emul_trees[7];
+extern "C" void bgemul_last_trees(uint32_t out[7]) { memcpy(out, g_emul_trees, sizeof g_emul_trees); }
+/* ties of the same call's distance and precode trees: equal leaf weights, then leaf / merged-node ties, of each (tree_stats) */
+static uint32_t g_emul_ties[4];
+extern "C" void bgemul_last_ties(uint32_t out[4]) { memcpy(out, g_emul_ties, sizeof g_emul_ties); }
 
 static uint32_t g_emul_hdr = 18;
 /* member framing of the following bgemul_compress_block calls: 18 = BGZF (default), 20 = MiGz */
@@ -92,6 +127,8 @@ extern "C" int bgemul_compress_block(const uint8_t *src, uint32_t n, int level, 
     if (g_emul_hist % BG_HISTORY_STEP || g_emul_hist > BG_MAX_HISTORY || g_emul_hist > n) return -3;
     c.frame = g_emul_piece ? bg_frame(g_emul_head, g_emul_tail, g_emul_final, 1u, g_emul_hist) : bg_frame(g_emul_hdr, 8u, 1u, 0u);
     c.prm = bg_level_params(level);
+    memset(g_emul_trees, 0, sizeof g_emul_trees);
+    memset(g_emul_ties, 0, sizeof g_emul_ties);
     uint32_t k = 0;
     run(bg_phase_init, c, order, k++);
     run(bg_phase_scan, c, order, k++);
@@ -132,7 +169,17 @@ extern "C" int bgemul_compress_block(const uint8_t *src, uint32_t n, int level, 
         }
         run(bg_phase_huff_prep, c, order, k++);
         run(bg_phase_huff, c, order, k++);
+        {
+            uint32_t st[3];
+            tree_stats((const uint32_t *)(c.regb + BG_B_DKEYS), c.scal[BG_S_DM], 15, st);
+            g_emul_trees[3] = c.scal[BG_S_DM];
+            g_emul_trees[4] = st[0];
+            g_emul_ties[0] = st[1];
+            g_emul_ties[1] = st[2];
+        }
         run(bg_phase_huff_depth, c, order, k++);
+        g_emul_trees[1] = c.scal[BG_S_HM];
+        g_emul_trees[2] = c.scal[BG_S_HOVF];
         run(bg_phase_huff_fix, c, order, k++);
         run(bg_phase_huff_assign, c, order, k++);
     }
@@ -146,6 +193,14 @@ extern "C" int bgemul_compress_block(const uint8_t *src, uint32_t n, int level, 
     }
     run(bg_phase_hdr4, c, order, k++);
     run(bg_phase_hdr4b, c, order, k++);
+    {
+        uint32_t st[3];
+        tree_stats((const uint32_t *)(c.regb + BG_B_PKEYS), c.scal[BG_S_PM], 7, st);
+        g_emul_trees[5] = c.scal[BG_S_PM];
+        g_emul_trees[6] = st[0];
+        g_emul_ties[2] = st[1];
+        g_emul_ties[3] = st[2];
+    }
     for (uint32_t t = 0; t < BG_THREADS; t++) bg_phase_hdr5(c, t, BG_THREADS, nitems);
     {   // cross-check against the sequential rule
         static uint16_t ref_items[400]; uint32_t ref_pf[19];
@@ -156,6 +211,7 @@ extern "C" int bgemul_compress_block(const uint8_t *src, uint32_t n, int level, 
         }
     }
     run(bg_phase_decide_b, c, order, k++);
+    g_emul_trees[0] = c.scal[BG_S_BTYPE];
     run(bg_phase_codes_a, c, order, k++);
     run(bg_phase_codes_b, c, order, k++);
     run(bg_phase_codes_c, c, order, k++);
