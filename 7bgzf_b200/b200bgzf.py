@@ -32,7 +32,8 @@ EXPORTS = [
     "b200bgzf_inflate_units_host", "b200bgzf_container_units", "b200bgzf_units_free", "b200bgzf_container_inflate_host",
     "b200bgzf_multi_container_bound", "b200bgzf_multi_container_compress_host", "b200bgzf_container_inflate_size",
     "b200bgzf_index_host", "b200bgzf_gzi_parse", "b200bgzf_inflate_ranges_host", "b200bgzf_inflate_ranges_device",
-    "b200bgzf_gzip_inflate_device",
+    "b200bgzf_gzip_inflate_device", "b200bgzf_gzip_index_host", "b200bgzf_gzip_index_device", "b200bgzf_gzip_inflate_ranges_host",
+    "b200bgzf_gzip_inflate_ranges_device",
 ]
 CONTAINER_GZIP, CONTAINER_MIGZ, CONTAINER_GZINGA, CONTAINER_DICTZIP, CONTAINER_RAZF = 1, 2, 3, 4, 5
 
@@ -129,6 +130,10 @@ def load(path=LIB_PATH):
     prange = ctypes.POINTER(Range)
     lib.b200bgzf_inflate_ranges_host.argtypes = [vp, vp, sz, pu64, pu64, sz, prange, sz, vp, sz, psz, pu64, ctypes.c_uint]
     lib.b200bgzf_inflate_ranges_device.argtypes = [vp, vp, sz, prange, sz, vp, sz, psz, pu64, ctypes.c_uint, vp]
+    lib.b200bgzf_gzip_index_host.argtypes = [vp, vp, sz, u32, vp, sz, psz]
+    lib.b200bgzf_gzip_index_device.argtypes = [vp, vp, sz, u32, vp, sz, psz, vp]
+    lib.b200bgzf_gzip_inflate_ranges_host.argtypes = [vp, vp, sz, vp, sz, prange, sz, vp, sz, psz, pu64, ctypes.c_uint]
+    lib.b200bgzf_gzip_inflate_ranges_device.argtypes = [vp, vp, sz, vp, sz, prange, sz, vp, sz, psz, pu64, ctypes.c_uint, vp]
     return lib
 
 
@@ -347,6 +352,45 @@ class Codec:
         got, off = ctypes.c_size_t(), (ctypes.c_uint64 * max(n, 1))()
         self._check(self.lib.b200bgzf_inflate_ranges_device(self.h, d_in, nbytes, arr, n, d_out, out_cap, ctypes.byref(got), off,
                                                             flags | (RANGE_VOFFSET if voffsets else 0), stream))
+        return got.value, list(off[:n])
+
+    # ---- whole-stream gzip: random access through a checkpoint index ----
+    def _sized(self, fn):
+        """fn(buffer, cap, byref(size)) once to learn the size (E_NOSPACE), then into a buffer of that size"""
+        need = ctypes.c_size_t()
+        self._check(fn(None, 0, ctypes.byref(need)), ok=(0, E_NOSPACE))
+        out = bytearray(max(need.value, 1))
+        self._check(fn(_addr(out), len(out), ctypes.byref(need)))
+        return bytes(out[: need.value])
+
+    def gzip_index(self, blob, span=0):
+        """the checkpoint index of one gzip member (bytes) — b200bgzf_gzip_index_host (the member is decoded twice: size, then bytes)"""
+        return self._sized(lambda buf, cap, n: self.lib.b200bgzf_gzip_index_host(self.h, _addr(blob), len(blob), span, buf, cap, n))
+
+    def gzip_index_device(self, d_in, nbytes, span=0, stream=None):
+        """b200bgzf_gzip_index_device: the index (bytes, host) of the member at device address d_in"""
+        return self._sized(lambda buf, cap, n: self.lib.b200bgzf_gzip_index_device(self.h, d_in, nbytes, span, buf, cap, n, stream))
+
+    def gzip_inflate_ranges(self, blob, index, ranges, flags=0):
+        """(the ranges' bytes back to back, where each range starts) — b200bgzf_gzip_inflate_ranges_host"""
+        n = len(ranges)
+        arr = (Range * max(n, 1))(*[Range(b, e) for b, e in ranges])
+        need, off = ctypes.c_size_t(), (ctypes.c_uint64 * max(n, 1))()
+        self._check(self.lib.b200bgzf_gzip_inflate_ranges_host(self.h, _addr(blob), len(blob), _addr(index), len(index), arr, n, None, 0,
+                                                               ctypes.byref(need), off, flags), ok=(0, E_NOSPACE))
+        out = bytearray(max(need.value, 1))
+        got = ctypes.c_size_t()
+        self._check(self.lib.b200bgzf_gzip_inflate_ranges_host(self.h, _addr(blob), len(blob), _addr(index), len(index), arr, n, _addr(out),
+                                                               len(out), ctypes.byref(got), off, flags))
+        return bytes(out[: got.value]), list(off[:n])
+
+    def gzip_inflate_ranges_device(self, d_in, nbytes, index, ranges, d_out, out_cap, flags=0, stream=None):
+        """(output bytes, where each range starts) — b200bgzf_gzip_inflate_ranges_device (device addresses in and out, host index)"""
+        n = len(ranges)
+        arr = (Range * max(n, 1))(*[Range(b, e) for b, e in ranges])
+        got, off = ctypes.c_size_t(), (ctypes.c_uint64 * max(n, 1))()
+        self._check(self.lib.b200bgzf_gzip_inflate_ranges_device(self.h, d_in, nbytes, _addr(index), len(index), arr, n, d_out, out_cap,
+                                                                 ctypes.byref(got), off, flags, stream))
         return got.value, list(off[:n])
 
     def profile(self, enable=True, reset=True, slots=32):

@@ -120,6 +120,12 @@ struct GzWork {
     size_t tiles_cap = 0, tileoff_cap = 0, u32_cap = 0, u64_cap = 0, scratch_cap = 0, in_cap = 0, out_cap = 0, h_cap = 0;
     cudaStream_t copy = nullptr;      /* D2H of finished batches (host reader), behind the batch's event */
     cudaEvent_t ev = nullptr;
+    /* random access through a checkpoint index: windows, the u8 image of a batch's layout, the window carried over a cut run,
+     * per-batch chunk / window / gather lists */
+    uint8_t *d_win = nullptr, *d_img = nullptr, *d_rout = nullptr;
+    uint16_t *d_carry = nullptr;
+    uint64_t *d_meta = nullptr;
+    size_t win_cap = 0, img_cap = 0, rout_cap = 0, carry_cap = 0, meta_cap = 0;
 };
 
 }  // namespace
@@ -452,6 +458,7 @@ extern "C" void b200bgzf_destroy(b200bgzf_ctx *ctx)
         GzWork &z = ctx->gz;
         cudaFree(z.tile_count); cudaFree(z.u32); cudaFree(z.small32); cudaFree(z.tile_off); cudaFree(z.u64); cudaFree(z.small64);
         cudaFree(z.scratch); cudaFree(z.d_in); cudaFree(z.d_out);
+        cudaFree(z.d_win); cudaFree(z.d_img); cudaFree(z.d_rout); cudaFree(z.d_carry); cudaFree(z.d_meta);
         if (z.h) cudaFreeHost(z.h);
         if (z.copy) cudaStreamDestroy(z.copy);
         if (z.ev) cudaEventDestroy(z.ev);
@@ -1468,9 +1475,16 @@ constexpr uint32_t kGzCrcPiece = 1u << 20;       /* B200BGZF_VERIFY: output byte
  * Returns BGZF_GZIP_FALLBACK when the member has no complete chain (no flush point, a chunk over the caps, a chain that ends
  * anywhere but at the trailer, a decode that differs from the boundary pass): the one-warp path then gives the outcome.
  * on_batch(base, bytes) is called after the launches that write output [base, base + bytes). */
+/* the chain the index builder keeps: the chunk arrays of BgzfGzipArgs (c_start, c_off, c_len), valid until the next gzip call */
+struct GzChain {
+    BgzfGzipArgs a;
+    uint64_t nchunks;
+};
+
 template <typename F>
 int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, uint32_t hlen, uint32_t isize, uint32_t want_crc,
-                       uint8_t *d_out, size_t out_cap, size_t *total_out, unsigned flags, cudaStream_t stream, F on_batch)
+                       uint8_t *d_out, size_t out_cap, size_t *total_out, unsigned flags, cudaStream_t stream, F on_batch,
+                       GzChain *keep = nullptr)
 {
     GzWork &z = ctx->gz;
     const uint64_t data_len = in_bytes - hlen - 8;
@@ -1505,7 +1519,8 @@ int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, 
     CK(cudaMemcpyAsync(z.h, z.small64, sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
     CK(cudaStreamSynchronize(stream));
     const uint64_t nc = z.h[0] + 1;
-    if (nc < 2 || nc > 0xfffffff0ull) return BGZF_GZIP_FALLBACK;
+    /* (the index builder takes a member without flush points as one chunk when its data is within the chunk cap) */
+    if ((nc < 2 && !(keep && data_len <= kGzMaxChunkIn)) || nc > 0xfffffff0ull) return BGZF_GZIP_FALLBACK;
     /* u64: cand, end, pick, c_start, c_off; u32: olen, status, c_len, lastm, anchor, jump, jump2, reach */
     CK(grow(&z.u64, &z.u64_cap, 5 * nc));
     CK(grow(&z.u32, &z.u32_cap, 8 * (nc + 2)));
@@ -1526,6 +1541,7 @@ int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, 
     *total_out = (size_t)total;
     if ((uint32_t)total != isize) return B200BGZF_E_FORMAT;
     if (total > out_cap || (!d_out && total)) return B200BGZF_E_NOSPACE;
+    if (keep) *keep = { a, nchunks };
     /* 3. batches of chained chunks whose scratch fits the budget */
     const uint64_t win = bgzf_gzip_window(), budget = gzip_budget();
     std::vector<uint64_t> cut;                      /* batch boundaries (chunk indices) */
@@ -1627,6 +1643,23 @@ int gzip_member_check(size_t in_bytes, uint32_t hlen, uint32_t isize)
     return 0;
 }
 
+/* the header (FEXTRA, FNAME, FCOMMENT, FHCRC) of a member in device memory, in small reads that grow while a field runs past
+ * what was read (*hlen = 0: not a gzip header); the trailer */
+int gzip_device_header(b200bgzf_ctx *ctx, const uint8_t *in, size_t in_bytes, cudaStream_t stream, size_t *hlen, uint8_t tr[8])
+{
+    std::vector<uint8_t> head;
+    size_t xoff, xlen;
+    for (size_t want = std::min<size_t>(in_bytes, 4096);; want = std::min(in_bytes, want * 4)) {
+        head.resize(want);
+        CK(cudaMemcpyAsync(head.data(), in, want, cudaMemcpyDeviceToHost, stream));
+        CK(cudaMemcpyAsync(tr, in + in_bytes - 8, 8, cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        *hlen = bgzf_gz_header(head.data(), want, &xoff, &xlen);
+        if (*hlen || want == in_bytes || head.size() < 10 || head[0] != 0x1f || head[1] != 0x8b) break;
+    }
+    return B200BGZF_OK;
+}
+
 }  // namespace
 
 extern "C" int b200bgzf_gzip_inflate_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, void *d_out, size_t out_cap,
@@ -1643,18 +1676,9 @@ extern "C" int b200bgzf_gzip_inflate_device(b200bgzf_ctx *ctx, const void *d_in,
     cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : l.stream;
     GzWork &z = ctx->gz;
     const uint8_t *in = (const uint8_t *)d_in;
-    /* the header (FEXTRA, FNAME, FCOMMENT, FHCRC) in small reads, growing while a field runs past what was read; the trailer */
-    std::vector<uint8_t> head;
     uint8_t tr[8];
-    size_t hlen = 0, xoff, xlen;
-    for (size_t want = std::min<size_t>(in_bytes, 4096);; want = std::min(in_bytes, want * 4)) {
-        head.resize(want);
-        CK(cudaMemcpyAsync(head.data(), in, want, cudaMemcpyDeviceToHost, stream));
-        CK(cudaMemcpyAsync(tr, in + in_bytes - 8, 8, cudaMemcpyDeviceToHost, stream));
-        CK(cudaStreamSynchronize(stream));
-        hlen = bgzf_gz_header(head.data(), want, &xoff, &xlen);
-        if (hlen || want == in_bytes || head.size() < 10 || head[0] != 0x1f || head[1] != 0x8b) break;
-    }
+    size_t hlen = 0;
+    if ((r = gzip_device_header(ctx, in, in_bytes, stream, &hlen, tr))) return r;
     const uint32_t want_crc = rd32(tr), isize = rd32(tr + 4);
     if ((r = gzip_member_check(in_bytes, (uint32_t)hlen, isize))) return r;
     size_t total = isize;
@@ -2138,4 +2162,549 @@ extern "C" int b200bgzf_inflate_ranges_device(b200bgzf_ctx *ctx, const void *d_i
     CK(cudaStreamSynchronize(stream));
     const uint32_t ef = (uint32_t)ctx->h_idx[3];
     return (ef & 1u) ? B200BGZF_E_FORMAT : (ef & 2u) ? B200BGZF_E_CRC : B200BGZF_OK;
+}
+
+/* ------------------------------------------------------------------------------------------------ */
+/* whole-stream gzip: random access through a checkpoint index (the format: include/b200bgzf.h)    */
+
+namespace {
+
+constexpr size_t kGzIxHead = 48;                 /* magic, in_bytes, hdr_len, crc32, isize, out_bytes, span, nchunks, npoints */
+constexpr uint64_t kGzIxChunk = 20, kGzIxPoint = 8;
+constexpr uint32_t kGzIxSpan = 1u << 20;         /* span 0 */
+
+uint64_t rd64(const uint8_t *p) { return (uint64_t)rd32(p) | (uint64_t)rd32(p + 4) << 32; }
+void wr32(uint8_t *p, uint32_t v) { for (int k = 0; k < 4; k++) p[k] = (uint8_t)(v >> (8 * k)); }
+void wr64(uint8_t *p, uint64_t v) { wr32(p, (uint32_t)v); wr32(p + 4, (uint32_t)(v >> 32)); }
+
+/* CRC-32 on the host, eight bytes per step (an index carries up to 32 KiB of window per access point) */
+uint32_t host_crc32(const uint8_t *p, size_t n)
+{
+    static const std::vector<uint32_t> tab = [] {
+        std::vector<uint32_t> t(8 * 256);
+        bg_make_crc_table(t.data());
+        for (int k = 1; k < 8; k++)
+            for (int i = 0; i < 256; i++) t[k * 256 + i] = (t[(k - 1) * 256 + i] >> 8) ^ t[t[(k - 1) * 256 + i] & 0xffu];
+        return t;
+    }();
+    const uint32_t *t = tab.data();
+    uint32_t c = 0xffffffffu;
+    for (; n >= 8; p += 8, n -= 8) {
+        const uint32_t a = rd32(p) ^ c, b = rd32(p + 4);
+        c = t[7 * 256 + (a & 0xffu)] ^ t[6 * 256 + ((a >> 8) & 0xffu)] ^ t[5 * 256 + ((a >> 16) & 0xffu)] ^ t[4 * 256 + (a >> 24)] ^
+            t[3 * 256 + (b & 0xffu)] ^ t[2 * 256 + ((b >> 8) & 0xffu)] ^ t[256 + ((b >> 16) & 0xffu)] ^ t[b >> 24];
+    }
+    while (n--) c = t[(c ^ *p++) & 0xffu] ^ (c >> 8);
+    return ~c;
+}
+
+/* a parsed index: every field checked, the windows left in place */
+struct GzIx {
+    uint64_t in_bytes = 0, out_bytes = 0;
+    uint32_t hdr_len = 0, crc = 0, isize = 0, span = 0;
+    std::vector<uint64_t> cs, uo;        /* per chunk: file offset, output offset */
+    std::vector<uint32_t> ccrc;          /* per chunk: CRC-32 of its output */
+    std::vector<uint32_t> pchunk, wlen;  /* per access point: its chunk, its window's length */
+    std::vector<uint64_t> woff;          /* per access point: where its window starts in `win` */
+    const uint8_t *win = nullptr;
+    size_t n() const { return cs.size(); }
+    uint64_t uend(size_t k) const { return k + 1 < cs.size() ? uo[k + 1] : out_bytes; }
+    uint64_t cend(size_t k) const { return k + 1 < cs.size() ? cs[k + 1] : in_bytes - 8; }
+};
+
+int gz_index_parse(const void *index, size_t bytes, GzIx &ix)
+{
+    const uint8_t *x = (const uint8_t *)index;
+    if (bytes < kGzIxHead + 4 || memcmp(x, "B2GZIX01", 8) || rd32(x + bytes - 4) != host_crc32(x, bytes - 4)) return B200BGZF_E_FORMAT;
+    ix.in_bytes = rd64(x + 8);
+    ix.hdr_len = rd32(x + 16);
+    ix.crc = rd32(x + 20);
+    ix.isize = rd32(x + 24);
+    ix.out_bytes = rd64(x + 28);
+    ix.span = rd32(x + 36);
+    const uint64_t n = rd32(x + 40), np = rd32(x + 44);
+    if (!n || !np || np > n || ix.span < 32768 || ix.hdr_len < 10 || ix.in_bytes < (uint64_t)ix.hdr_len + 10 ||
+        ix.out_bytes > 0x7fffffffu || (uint32_t)ix.out_bytes != ix.isize)
+        return B200BGZF_E_FORMAT;
+    const uint64_t fixed = kGzIxHead + kGzIxChunk * n + kGzIxPoint * np + 4;
+    if (fixed > bytes) return B200BGZF_E_FORMAT;
+    ix.cs.resize(n);
+    ix.uo.resize(n);
+    ix.ccrc.resize(n);
+    for (uint64_t k = 0; k < n; k++) {
+        const uint8_t *c = x + kGzIxHead + kGzIxChunk * k;
+        const uint64_t s = rd64(c), u = rd64(c + 8);
+        if (k == 0 ? (s != ix.hdr_len || u != 0) : (s <= ix.cs[k - 1] || u < ix.uo[k - 1])) return B200BGZF_E_FORMAT;
+        if (s >= ix.in_bytes - 8 || u > ix.out_bytes) return B200BGZF_E_FORMAT;
+        ix.cs[k] = s;
+        ix.uo[k] = u;
+        ix.ccrc[k] = rd32(c + 16);
+    }
+    uint64_t wsum = 0;
+    for (uint64_t p = 0; p < np; p++) {
+        const uint8_t *q = x + kGzIxHead + kGzIxChunk * n + kGzIxPoint * p;
+        const uint32_t k = rd32(q), w = rd32(q + 4);
+        if (p == 0 ? k != 0 : k <= ix.pchunk.back()) return B200BGZF_E_FORMAT;
+        if (k >= n || w != std::min<uint64_t>(32768, ix.uo[k])) return B200BGZF_E_FORMAT;
+        ix.pchunk.push_back(k);
+        ix.wlen.push_back(w);
+        ix.woff.push_back(wsum);
+        wsum += w;
+    }
+    if (fixed + wsum != bytes) return B200BGZF_E_FORMAT;
+    ix.win = x + kGzIxHead + kGzIxChunk * n + kGzIxPoint * np;
+    return B200BGZF_OK;
+}
+
+/* Builds the index of the member d_in[0, in_bytes) (header of hlen bytes, trailer tr): its flush-point chain decoded once into
+ * the context's output buffer, the chunks' CRC-32 (bgzf_verify_kernel, one unit per chunk), the access points' windows
+ * (gathered on the device, copied back in one piece). */
+int gzip_index_build(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, uint32_t hlen, const uint8_t tr[8], uint32_t span,
+                     void *index, size_t index_cap, size_t *index_bytes, cudaStream_t stream)
+{
+    const uint32_t want_crc = rd32(tr), isize = rd32(tr + 4);
+    int r = gzip_member_check(in_bytes, hlen, isize);
+    if (r) return r;
+    GzWork &z = ctx->gz;
+    CK(grow(&z.d_out, &z.out_cap, (size_t)isize + 64));
+    size_t total = isize;
+    GzChain ch;
+    r = gzip_chain_inflate(ctx, d_in, in_bytes, hlen, isize, want_crc, z.d_out, isize, &total, 0, stream,
+                           [](uint64_t, uint64_t) { return 0; }, &ch);
+    if (r == BGZF_GZIP_FALLBACK || r == B200BGZF_E_NOSPACE) return B200BGZF_E_FORMAT;   /* not indexable */
+    if (r) return r;
+    const uint64_t n = ch.nchunks;
+    std::vector<uint64_t> cs(n), uo(n);
+    CK(cudaMemcpyAsync(uo.data(), ch.a.c_off, n * 8, cudaMemcpyDeviceToHost, stream));
+    CK(cudaMemcpyAsync(cs.data(), ch.a.c_start, n * 8, cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    /* access points: chunk 0, then every chunk at least `span` bytes of output past the previous point */
+    std::vector<uint32_t> pts{ 0 };
+    for (uint64_t k = 1; k < n; k++)
+        if (uo[k] - uo[pts.back()] >= span) pts.push_back((uint32_t)k);
+    const uint64_t np = pts.size();
+    std::vector<uint64_t> wl(np), wo(np);
+    uint64_t wsum = 0;
+    for (uint64_t p = 0; p < np; p++) {
+        wl[p] = std::min<uint64_t>(32768, uo[pts[p]]);
+        wo[p] = wsum;
+        wsum += wl[p];
+    }
+    const uint64_t size = kGzIxHead + kGzIxChunk * n + kGzIxPoint * np + wsum + 4;
+    *index_bytes = (size_t)size;
+    if (!index || index_cap < size) return B200BGZF_E_NOSPACE;
+    /* chunk CRCs: bgzf_verify_kernel over pieces of the output (in_off / hdr_len / msize / status unused: zeros) */
+    uint32_t *zero = ch.a.olen, *ucrc = ch.a.status;     /* (per-candidate arrays the chain no longer needs, >= n entries) */
+    CK(cudaMemsetAsync(zero, 0, n * 4, stream));
+    BgzfInflateArgs v;
+    memset(&v, 0, sizeof v);
+    v.in = z.d_out;
+    v.in_off = ch.a.c_off;
+    v.out_off = ch.a.c_off;
+    v.hdr_len = zero;
+    v.msize = zero;
+    v.unit_isize = ch.a.c_len;
+    v.status = zero;
+    v.unit_crc = ucrc;
+    v.nblocks = (uint32_t)n;
+    v.out = z.d_out;
+    v.err_flag = ch.a.err + 2;
+    v.verify_crc = 1;
+    v.crctab = ctx->d_crctab;
+    v.crcpow = ctx->d_crcpow;
+    CK(bgzf_launch_verify(&v, stream));
+    ctx->launches += 1;
+    /* windows: bgzf_range_gather_kernel cuts them out of the output, back to back */
+    std::vector<uint8_t> out(size);
+    if (wsum) {
+        std::vector<uint64_t> g(4 * np);
+        uint64_t tiles = 0;
+        for (uint64_t p = 0; p < np; p++) {
+            g[p] = uo[pts[p]] - wl[p];
+            g[np + p] = wo[p];
+            g[2 * np + p] = wl[p];
+            g[3 * np + p] = tiles;
+            tiles += (wl[p] + BGZF_GATHER_TILE - 1) / BGZF_GATHER_TILE;
+        }
+        CK(grow(&z.d_meta, &z.meta_cap, 4 * np));
+        CK(grow(&z.d_win, &z.win_cap, wsum + 64));
+        CK(cudaMemcpyAsync(z.d_meta, g.data(), g.size() * 8, cudaMemcpyHostToDevice, stream));
+        BgzfRangeGatherArgs ga;
+        ga.scratch = z.d_out;
+        ga.win_lo = 0;
+        ga.win_hi = ~0ull;
+        ga.out = z.d_win;
+        ga.src = z.d_meta;
+        ga.range_off = z.d_meta + np;
+        ga.len = z.d_meta + 2 * np;
+        ga.tile_off = z.d_meta + 3 * np;
+        ga.nranges = (uint32_t)np;
+        CK(bgzf_launch_range_gather(&ga, tiles, stream));
+        ctx->launches += 1;
+        CK(cudaMemcpyAsync(out.data() + kGzIxHead + kGzIxChunk * n + kGzIxPoint * np, z.d_win, wsum, cudaMemcpyDeviceToHost, stream));
+    }
+    std::vector<uint32_t> crc(n);
+    CK(cudaMemcpyAsync(crc.data(), ucrc, n * 4, cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    uint8_t *x = out.data();
+    memcpy(x, "B2GZIX01", 8);
+    wr64(x + 8, in_bytes);
+    wr32(x + 16, hlen);
+    wr32(x + 20, want_crc);
+    wr32(x + 24, isize);
+    wr64(x + 28, total);
+    wr32(x + 36, span);
+    wr32(x + 40, (uint32_t)n);
+    wr32(x + 44, (uint32_t)np);
+    for (uint64_t k = 0; k < n; k++) {
+        uint8_t *c = x + kGzIxHead + kGzIxChunk * k;
+        wr64(c, cs[k] + hlen);
+        wr64(c + 8, uo[k]);
+        wr32(c + 16, crc[k]);
+    }
+    for (uint64_t p = 0; p < np; p++) {
+        uint8_t *q = x + kGzIxHead + kGzIxChunk * n + kGzIxPoint * p;
+        wr32(q, pts[p]);
+        wr32(q + 4, (uint32_t)wl[p]);
+    }
+    wr32(x + size - 4, host_crc32(x, size - 4));
+    memcpy(index, x, size);
+    return B200BGZF_OK;
+}
+
+int gzip_span(uint32_t *span)
+{
+    if (*span == 0) *span = kGzIxSpan;
+    return *span < 32768 ? B200BGZF_E_ARG : B200BGZF_OK;
+}
+
+/* a run: chunks [s, e] decoded from the access point s */
+struct GzRun {
+    uint32_t s, e;
+};
+
+/* Checks the index against the file (size, trailer) and the ranges against the index; the merged runs the ranges touch, in
+ * order, range_off and the output size.  Returns E_FORMAT / E_ARG / E_NOSPACE as the public calls do. */
+int gz_ranges_plan(const GzIx &ix, size_t in_bytes, const uint8_t tr[8], const b200bgzf_range *ranges, size_t nranges, size_t out_cap,
+                   bool have_out, size_t *out_bytes, uint64_t *range_off, std::vector<GzRun> &runs)
+{
+    if (ix.in_bytes != in_bytes || ix.crc != rd32(tr) || ix.isize != rd32(tr + 4)) return B200BGZF_E_FORMAT;
+    uint64_t out_total = 0;
+    for (size_t i = 0; i < nranges; i++) {
+        const uint64_t b = ranges[i].beg, e = ranges[i].end;
+        if (b > e || e > ix.out_bytes) return B200BGZF_E_ARG;
+        if (range_off) range_off[i] = out_total;
+        out_total += e - b;
+        if (b == e) continue;
+        const uint32_t f = (uint32_t)last_le(ix.uo.data(), ix.n(), b), l = (uint32_t)last_le(ix.uo.data(), ix.n(), e - 1);
+        const size_t p = (size_t)(std::upper_bound(ix.pchunk.begin(), ix.pchunk.end(), f) - ix.pchunk.begin()) - 1;
+        runs.push_back({ ix.pchunk[p], l });
+    }
+    *out_bytes = (size_t)out_total;
+    if (out_total > out_cap || (!have_out && out_total)) return B200BGZF_E_NOSPACE;
+    std::sort(runs.begin(), runs.end(), [](const GzRun &a, const GzRun &b) { return a.s < b.s || (a.s == b.s && a.e > b.e); });
+    size_t m = 0;
+    for (size_t i = 0; i < runs.size(); i++) {
+        if (m && runs[i].s <= runs[m - 1].e + 1) runs[m - 1].e = std::max(runs[m - 1].e, runs[i].e);
+        else runs[m++] = runs[i];
+    }
+    runs.resize(m);
+    return B200BGZF_OK;
+}
+
+/* Decodes the runs and cuts the ranges out of them into d_out.  The compressed bytes are in d_data[0, data_len), chunk k at
+ * cstart[k] (indexed by chunk number, only touched chunks are read).  A batch holds consecutive runs (or parts of one run cut at
+ * a chunk boundary) whose u16 layout fits the budget: per part 32 KiB of window, then its chunks.  A part that continues a run
+ * takes its window from the last 32 KiB of the batch before it, resolved in scratch (as gzip_chain_inflate's prefix does). */
+int gz_ranges_decode(b200bgzf_ctx *ctx, const GzIx &ix, const uint8_t *d_data, uint64_t data_len, const std::vector<uint64_t> &cstart,
+                     const std::vector<GzRun> &runs, const b200bgzf_range *ranges, size_t nranges, const uint64_t *range_off,
+                     uint8_t *d_out, unsigned flags, cudaStream_t stream)
+{
+    GzWork &z = ctx->gz;
+    const uint64_t win = bgzf_gzip_window(), half = gzip_budget() / 2;
+    struct Part { uint32_t run, k0, k1; bool cont; uint64_t pos; };    /* chunks [k0, k1); pos: its window's place in the layout */
+    std::vector<std::vector<Part>> batches(1);
+    std::vector<uint64_t> bytes_of;                                    /* per batch: image bytes (layout after the first window) */
+    uint64_t used = 0;
+    auto close = [&]() { bytes_of.push_back(used - win); batches.emplace_back(); used = 0; };
+    for (uint32_t r = 0; r < runs.size(); r++) {
+        bool cont = false;
+        for (uint32_t k = runs[r].s; k <= runs[r].e;) {
+            if (win + ix.uend(k) - ix.uo[k] > half - used) {
+                if (!used) return B200BGZF_E_FORMAT;                   /* one chunk alone is over the budget */
+                close();
+                continue;
+            }
+            uint32_t k1 = k + 1;
+            while (k1 <= runs[r].e && win + ix.uend(k1) - ix.uo[k] <= half - used) k1++;
+            batches.back().push_back({ r, k, k1, cont, used });
+            used += win + ix.uo[k1 - 1] - ix.uo[k] + (ix.uend(k1 - 1) - ix.uo[k1 - 1]);
+            if (k1 <= runs[r].e) { close(); cont = true; }
+            k = k1;
+        }
+    }
+    if (used) close();
+    batches.pop_back();
+    /* image coordinates of every touched chunk over all batches, then the gather lists of the ranges */
+    std::vector<uint64_t> gbase(batches.size()), gpos(ix.n());
+    uint64_t g = 0, most = 0;
+    for (size_t b = 0; b < batches.size(); b++) {
+        gbase[b] = g;
+        for (const Part &p : batches[b])
+            for (uint32_t k = p.k0; k < p.k1; k++) gpos[k] = g + p.pos + ix.uo[k] - ix.uo[p.k0];
+        g += bytes_of[b];
+        most = std::max(most, bytes_of[b]);
+    }
+    const uint64_t R = nranges;
+    std::vector<uint64_t> rl(4 * R);
+    uint64_t tiles = 0;
+    for (uint64_t i = 0; i < R; i++) {
+        const uint64_t b = ranges[i].beg, len = ranges[i].end - b;
+        rl[i] = len ? gpos[last_le(ix.uo.data(), ix.n(), b)] + b - ix.uo[last_le(ix.uo.data(), ix.n(), b)] : 0;
+        rl[R + i] = range_off[i];
+        rl[2 * R + i] = len;
+        rl[3 * R + i] = tiles;
+        tiles += (len + BGZF_GATHER_TILE - 1) / BGZF_GATHER_TILE;
+    }
+    size_t maxj = 0, maxw = 0;
+    for (auto &parts : batches) {
+        size_t j = 0;
+        for (const Part &p : parts) j += p.k1 - p.k0;
+        maxj = std::max(maxj, j);
+        maxw = std::max(maxw, parts.size());
+    }
+    /* u64 meta: the gather lists [4R], then per batch c_start, c_off, m_off [J], win_src, win_dst [W]; u32 after it: c_len,
+     * lastm, anchor, zero, unit_crc [J], win_len [W], err */
+    const size_t m64 = 4 * R + 3 * maxj + 2 * maxw, m32 = 5 * maxj + maxw + 4;
+    CK(grow(&z.d_meta, &z.meta_cap, m64 + (m32 + 1) / 2));
+    CK(grow(&z.scratch, &z.scratch_cap, win + most + 16));
+    CK(grow(&z.d_img, &z.img_cap, most + 64));
+    CK(grow(&z.d_carry, &z.carry_cap, win));
+    size_t wcap = 0;
+    for (auto &parts : batches) {
+        size_t w = 0;
+        for (const Part &p : parts) w += p.cont ? 0 : 32768;
+        wcap = std::max(wcap, w);
+    }
+    CK(grow(&z.d_win, &z.win_cap, wcap + 64));
+    uint64_t *d_rl = z.d_meta, *d64 = z.d_meta + 4 * R;
+    uint32_t *d32 = (uint32_t *)(z.d_meta + m64);
+    uint32_t *d_err = d32 + 5 * maxj + maxw;
+    CK(cudaMemcpyAsync(d_rl, rl.data(), rl.size() * 8, cudaMemcpyHostToDevice, stream));
+    CK(cudaMemsetAsync(d_err, 0, 4, stream));
+    const bool verify = (flags & B200BGZF_VERIFY) != 0;
+    bool badcrc = false;
+    std::vector<uint64_t> h64;
+    std::vector<uint32_t> h32, hcrc, want;
+    std::vector<uint8_t> hwin;
+    for (size_t b = 0; b < batches.size(); b++) {
+        const std::vector<Part> &parts = batches[b];
+        size_t J = 0, W = 0;
+        for (const Part &p : parts) { J += p.k1 - p.k0; W += p.cont ? 0 : 1; }
+        h64.assign(3 * J + 2 * W, 0);
+        h32.assign(J + W, 0);
+        hwin.clear();
+        want.clear();
+        uint64_t *c_start = h64.data(), *c_off = c_start + J, *m_off = c_off + J, *wsrc = m_off + J, *wdst = wsrc + W;
+        uint32_t *c_len = h32.data(), *wlen = c_len + J;
+        size_t j = 0, w = 0;
+        for (const Part &p : parts) {
+            for (uint32_t k = p.k0; k < p.k1; k++, j++) {
+                c_start[j] = cstart[k];
+                c_off[j] = p.pos + ix.uo[k] - ix.uo[p.k0];
+                m_off[j] = ix.uo[k];
+                c_len[j] = (uint32_t)(ix.uend(k) - ix.uo[k]);
+                want.push_back(ix.ccrc[k]);
+            }
+            if (p.cont) continue;
+            const size_t pt = (size_t)(std::lower_bound(ix.pchunk.begin(), ix.pchunk.end(), p.k0) - ix.pchunk.begin());
+            wsrc[w] = hwin.size();
+            wdst[w] = p.pos;
+            wlen[w] = ix.wlen[pt];
+            hwin.insert(hwin.end(), ix.win + ix.woff[pt], ix.win + ix.woff[pt] + ix.wlen[pt]);
+            w++;
+        }
+        CK(cudaMemcpyAsync(d64, h64.data(), h64.size() * 8, cudaMemcpyHostToDevice, stream));
+        CK(cudaMemcpyAsync(d32, h32.data(), J * 4, cudaMemcpyHostToDevice, stream));
+        CK(cudaMemcpyAsync(d32 + 5 * maxj, wlen, W * 4, cudaMemcpyHostToDevice, stream));
+        if (!hwin.empty()) CK(cudaMemcpyAsync(z.d_win, hwin.data(), hwin.size(), cudaMemcpyHostToDevice, stream));
+        if (parts[0].cont) CK(cudaMemcpyAsync(z.scratch, z.d_carry, win * 2, cudaMemcpyDeviceToDevice, stream));
+        BgzfGzipArgs a;
+        memset(&a, 0, sizeof a);
+        a.data = d_data;
+        a.data_len = data_len;
+        a.max_in = kGzMaxChunkIn;
+        a.c_start = d64;
+        a.c_off = d64 + J;
+        a.c_len = d32;
+        a.lastm = d32 + maxj;
+        a.anchor = d32 + 2 * maxj;
+        a.scratch = z.scratch;
+        a.out = z.d_img;
+        a.err = d_err;
+        BgzfGzipRunArgs ra;
+        ra.nchunks = (uint32_t)J;
+        ra.m_off = d64 + 2 * J;
+        ra.nwin = (uint32_t)W;
+        ra.win = z.d_win;
+        ra.win_src = d64 + 3 * J;
+        ra.win_len = d32 + 5 * maxj;
+        ra.win_dst = d64 + 3 * J + W;
+        CK(bgzf_launch_gzip_runs(&a, &ra, bytes_of[b], stream));
+        ctx->launches += 4 + (W ? 1 : 0) + (bytes_of[b] ? 1 : 0);
+        if (verify) {
+            uint32_t *zero = d32 + 3 * maxj, *ucrc = d32 + 4 * maxj;
+            CK(cudaMemsetAsync(zero, 0, J * 4, stream));
+            BgzfInflateArgs v;
+            memset(&v, 0, sizeof v);
+            v.in = z.d_img;
+            v.in_off = a.c_off;
+            v.out_off = a.c_off;
+            v.hdr_len = zero;
+            v.msize = zero;
+            v.unit_isize = a.c_len;
+            v.status = zero;
+            v.unit_crc = ucrc;
+            v.nblocks = (uint32_t)J;
+            v.out = z.d_img;
+            v.err_flag = d_err + 1;
+            v.verify_crc = 1;
+            v.crctab = ctx->d_crctab;
+            v.crcpow = ctx->d_crcpow;
+            CK(bgzf_launch_verify(&v, stream));
+            ctx->launches += 1;
+            hcrc.resize(J);
+            CK(cudaMemcpyAsync(hcrc.data(), ucrc, J * 4, cudaMemcpyDeviceToHost, stream));
+        }
+        BgzfRangeGatherArgs ga;
+        ga.scratch = z.d_img;
+        ga.win_lo = gbase[b];
+        ga.win_hi = gbase[b] + bytes_of[b];
+        ga.out = d_out;
+        ga.src = d_rl;
+        ga.range_off = d_rl + R;
+        ga.len = d_rl + 2 * R;
+        ga.tile_off = d_rl + 3 * R;
+        ga.nranges = (uint32_t)R;
+        CK(bgzf_launch_range_gather(&ga, tiles, stream));
+        ctx->launches += 1;
+        if (parts.back().k1 <= runs[parts.back().run].e)   /* the last run goes on in the next batch: its window */
+            CK(cudaMemcpyAsync(z.d_carry, z.scratch + bytes_of[b], win * 2, cudaMemcpyDeviceToDevice, stream));
+        if (verify) {
+            CK(cudaStreamSynchronize(stream));
+            if (hcrc != want) badcrc = true;
+        }
+    }
+    uint32_t err = 0;
+    CK(cudaMemcpyAsync(&err, d_err, 4, cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    return err ? B200BGZF_E_FORMAT : badcrc ? B200BGZF_E_CRC : B200BGZF_OK;
+}
+
+}  // namespace
+
+extern "C" int b200bgzf_gzip_index_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, uint32_t span, void *index,
+                                          size_t index_cap, size_t *index_bytes, void *stream_)
+{
+    if (!ctx || !d_in || !index_bytes || gzip_span(&span)) return B200BGZF_E_ARG;
+    *index_bytes = 0;
+    if (in_bytes < 18) return B200BGZF_E_FORMAT;
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    int r = lane_reserve(ctx, l, 1, 0, 0, false);
+    if (r) return r;
+    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : l.stream;
+    uint8_t tr[8];
+    size_t hlen = 0;
+    if ((r = gzip_device_header(ctx, (const uint8_t *)d_in, in_bytes, stream, &hlen, tr))) return r;
+    return gzip_index_build(ctx, (const uint8_t *)d_in, in_bytes, (uint32_t)hlen, tr, span, index, index_cap, index_bytes, stream);
+}
+
+extern "C" int b200bgzf_gzip_index_host(b200bgzf_ctx *ctx, const void *in_, size_t in_bytes, uint32_t span, void *index, size_t index_cap,
+                                        size_t *index_bytes)
+{
+    const uint8_t *in = (const uint8_t *)in_;
+    if (!ctx || !in || !index_bytes || gzip_span(&span)) return B200BGZF_E_ARG;
+    *index_bytes = 0;
+    if (in_bytes < 18) return B200BGZF_E_FORMAT;
+    size_t xoff, xlen;
+    const size_t hlen = bgzf_gz_header(in, in_bytes, &xoff, &xlen);
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    int r = lane_reserve(ctx, l, 1, 0, 0, false);
+    if (r) return r;
+    GzWork &z = ctx->gz;
+    CK(grow(&z.d_in, &z.in_cap, in_bytes + 64));
+    CK(cudaMemcpyAsync(z.d_in, in, in_bytes, cudaMemcpyHostToDevice, l.stream));
+    return gzip_index_build(ctx, z.d_in, in_bytes, (uint32_t)hlen, in + in_bytes - 8, span, index, index_cap, index_bytes, l.stream);
+}
+
+extern "C" int b200bgzf_gzip_inflate_ranges_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, const void *index, size_t index_bytes,
+                                                   const b200bgzf_range *ranges, size_t nranges, void *d_out, size_t out_cap,
+                                                   size_t *out_bytes, uint64_t *range_off, unsigned flags, void *stream_)
+{
+    if (!ctx || !d_in || !index || !out_bytes || (!ranges && nranges) || nranges > 0x7fffffffu || (flags & B200BGZF_RANGE_VOFFSET))
+        return B200BGZF_E_ARG;
+    *out_bytes = 0;
+    GzIx ix;
+    int r = gz_index_parse(index, index_bytes, ix);
+    if (r) return r;
+    if (in_bytes != ix.in_bytes) return B200BGZF_E_FORMAT;
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    if ((r = lane_reserve(ctx, l, 1, 0, 0, false))) return r;
+    cudaStream_t stream = stream_ ? (cudaStream_t)stream_ : l.stream;
+    uint8_t tr[8];
+    CK(cudaMemcpyAsync(tr, (const uint8_t *)d_in + in_bytes - 8, 8, cudaMemcpyDeviceToHost, stream));
+    CK(cudaStreamSynchronize(stream));
+    std::vector<uint64_t> roff(nranges);
+    std::vector<GzRun> runs;
+    r = gz_ranges_plan(ix, in_bytes, tr, ranges, nranges, out_cap, d_out != nullptr, out_bytes, roff.data(), runs);
+    if (range_off && (r == B200BGZF_OK || r == B200BGZF_E_NOSPACE)) memcpy(range_off, roff.data(), nranges * 8);
+    if (r || runs.empty()) return r;
+    return gz_ranges_decode(ctx, ix, (const uint8_t *)d_in, in_bytes - 8, ix.cs, runs, ranges, nranges, roff.data(), (uint8_t *)d_out,
+                            flags, stream);
+}
+
+extern "C" int b200bgzf_gzip_inflate_ranges_host(b200bgzf_ctx *ctx, const void *in_, size_t in_bytes, const void *index, size_t index_bytes,
+                                                 const b200bgzf_range *ranges, size_t nranges, void *out, size_t out_cap,
+                                                 size_t *out_bytes, uint64_t *range_off, unsigned flags)
+{
+    const uint8_t *in = (const uint8_t *)in_;
+    if (!ctx || !in || !index || !out_bytes || (!ranges && nranges) || nranges > 0x7fffffffu || (flags & B200BGZF_RANGE_VOFFSET))
+        return B200BGZF_E_ARG;
+    *out_bytes = 0;
+    GzIx ix;
+    int r = gz_index_parse(index, index_bytes, ix);
+    if (r) return r;
+    if (in_bytes != ix.in_bytes) return B200BGZF_E_FORMAT;
+    std::vector<uint64_t> roff(nranges);
+    std::vector<GzRun> runs;
+    r = gz_ranges_plan(ix, in_bytes, in + in_bytes - 8, ranges, nranges, out_cap, out != nullptr, out_bytes, roff.data(), runs);
+    if (range_off && (r == B200BGZF_OK || r == B200BGZF_E_NOSPACE)) memcpy(range_off, roff.data(), nranges * 8);
+    if (r || runs.empty()) return r;
+    DeviceGuard g(ctx->device);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    Lane &l = ctx->lanes[0];
+    if ((r = lane_reserve(ctx, l, 1, 0, 0, false))) return r;
+    GzWork &z = ctx->gz;
+    /* only the compressed bytes of the touched runs are read: packed back to back on the device */
+    std::vector<uint64_t> cstart(ix.n());
+    uint64_t packed = 0;
+    for (const GzRun &u : runs) {
+        for (uint32_t k = u.s; k <= u.e; k++) cstart[k] = packed + ix.cs[k] - ix.cs[u.s];
+        packed += ix.cend(u.e) - ix.cs[u.s];
+    }
+    CK(grow(&z.d_in, &z.in_cap, packed + 64));
+    CK(grow(&z.d_rout, &z.rout_cap, *out_bytes + 64));
+    for (const GzRun &u : runs)
+        CK(cudaMemcpyAsync(z.d_in + cstart[u.s], in + ix.cs[u.s], ix.cend(u.e) - ix.cs[u.s], cudaMemcpyHostToDevice, l.stream));
+    r = gz_ranges_decode(ctx, ix, z.d_in, packed, cstart, runs, ranges, nranges, roff.data(), z.d_rout, flags, l.stream);
+    if (r) return r;
+    CK(cudaMemcpyAsync(out, z.d_rout, *out_bytes, cudaMemcpyDeviceToHost, l.stream));
+    CK(cudaStreamSynchronize(l.stream));
+    return B200BGZF_OK;
 }

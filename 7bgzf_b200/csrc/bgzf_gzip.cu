@@ -440,6 +440,48 @@ gz_narrow_kernel(BgzfGzipArgs a, uint32_t j0, uint32_t j1, uint64_t base, uint64
     }
 }
 
+/* ---- random access through a checkpoint index: runs of chunks, each from an access point, each behind its own window ----
+ * A batch lays its runs out back to back in scratch: 32 KiB of window (u16 bytes), then the run's chunks.  c_off[j] is a
+ * chunk's place in that layout (so the anchor, resolve and narrow passes work unchanged: the window is a run of bytes that
+ * separates a run from the markers of the one before it), m_off[j] its offset in the member (the "reference before the
+ * member start" check). */
+
+/* scratch[dst[r], + GZ_WIN) = window r, widened and right-aligned; zeros before a window shorter than 32 KiB (the member start) */
+__global__ void __launch_bounds__(256)
+gz_window_kernel(uint16_t *scratch, const uint8_t *win, const uint64_t *src, const uint32_t *len, const uint64_t *dst)
+{
+    const uint32_t r = blockIdx.x, n = len[r], pad = GZ_WIN - n;
+    uint16_t *d = scratch + dst[r];
+    for (uint32_t i = threadIdx.x; i < GZ_WIN; i += blockDim.x) d[i] = i >= pad ? win[src[r] + (i - pad)] : 0;
+}
+
+/* gz_marker_kernel for a run layout (chunks [0, gridDim.x) of the batch) */
+__global__ void __launch_bounds__(32, 32)
+gz_run_marker_kernel(BgzfGzipArgs a, const uint64_t *m_off)
+{
+    __shared__ InfSmem sm;
+    const uint32_t lane = threadIdx.x, j = blockIdx.x;
+    const uint64_t s = a.c_start[j], o = a.c_off[j];
+    const uint8_t *lim = a.data + (a.data_len - s > a.max_in ? s + a.max_in : a.data_len);
+    const GzChunk c = gz_decode_chunk<true>(sm, a.data, a.data + s, lim, false, a.scratch + GZ_WIN + o, a.c_len[j], m_off[j], lane);
+    if (lane == 0) {
+        a.lastm[j] = c.lastm;
+        if (c.status == GZ_FAIL || c.olen != a.c_len[j]) atomicOr(a.err, c.dist_err ? 1u : 2u);
+    }
+}
+
+extern "C" cudaError_t bgzf_launch_gzip_runs(const BgzfGzipArgs *a, const BgzfGzipRunArgs *r, uint64_t bytes, cudaStream_t stream)
+{
+    if (r->nchunks == 0) return cudaSuccess;
+    if (r->nwin) gz_window_kernel<<<r->nwin, 256, 0, stream>>>(a->scratch, r->win, r->win_src, r->win_len, r->win_dst);
+    gz_run_marker_kernel<<<r->nchunks, 32, 0, stream>>>(*a, r->m_off);
+    gz_anchor_kernel<<<1, 1024, 0, stream>>>(*a, 0, r->nchunks, 0);
+    gz_resolve_kernel<<<r->nchunks, GZ_RESOLVE_THREADS, 0, stream>>>(*a, 0, r->nchunks, 0);
+    const uint64_t threads = (bytes + GZ_NARROW - 1) / GZ_NARROW;
+    if (threads) gz_narrow_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(*a, 0, r->nchunks, 0, bytes);
+    return cudaGetLastError();
+}
+
 extern "C" size_t bgzf_gzip_tiles(uint64_t data_len) { return (size_t)((data_len + GZ_TILE - 1) / GZ_TILE); }
 extern "C" size_t bgzf_gzip_window(void) { return GZ_WIN; }
 

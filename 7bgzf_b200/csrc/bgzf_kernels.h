@@ -150,6 +150,17 @@ struct BgzfGzipArgs {
     uint32_t *err;             /* bit 0: a back-reference before the member start, bit 1: a chunk decoded differently */
 };
 
+/* random access through a gzip checkpoint index (bgzf_launch_gzip_runs): the batch's chunks lie in runs, each behind its window */
+struct BgzfGzipRunArgs {
+    uint32_t nchunks;          /* chunks of the batch (c_start, c_off, c_len of BgzfGzipArgs, from index 0) */
+    const uint64_t *m_off;     /* [nchunks] each chunk's output offset in the member */
+    uint32_t nwin;             /* windows to place */
+    const uint8_t *win;        /* their bytes */
+    const uint64_t *win_src;   /* [nwin] where window r starts in win */
+    const uint32_t *win_len;   /* [nwin] its length (<= 32 KiB) */
+    const uint64_t *win_dst;   /* [nwin] scratch offset of its 32 KiB slot (it is right-aligned there) */
+};
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -171,6 +182,7 @@ size_t bgzf_gzip_window(void);
 cudaError_t bgzf_launch_gzip_count(const BgzfGzipArgs *a, cudaStream_t stream);    /* counts[0] = flush points found */
 cudaError_t bgzf_launch_gzip_chain(const BgzfGzipArgs *a, uint32_t ncand, cudaStream_t stream);
 cudaError_t bgzf_launch_gzip_batch(const BgzfGzipArgs *a, uint32_t j0, uint32_t j1, uint64_t base, uint64_t bytes, cudaStream_t stream);
+cudaError_t bgzf_launch_gzip_runs(const BgzfGzipArgs *a, const BgzfGzipRunArgs *r, uint64_t bytes, cudaStream_t stream);
 #define BGZF_GZIP_CHAIN_LAUNCHES 8
 #define BGZF_GZIP_BATCH_LAUNCHES 5
 #define BGZF_INDEX_LAUNCHES 8

@@ -5,6 +5,8 @@
  *   7bgzf -d [-@ N] < in.bgz > out            decompress
  *   7bgzf -d --offset=N [--size=M] [--gzi=F] < in.bgz > out    decompress bytes [N, N+M) only (bgzip -b N -s M)
  *   7bgzf --reindex --gzi=F < in.bgz          write the .gzi of an existing stream (bgzip -r)
+ *   7gzip --reindex --index=F < in.gz         write the checkpoint index of a whole-stream gzip member
+ *   7gzip -d --offset=N [--size=M] --index=F < in.gz > out    decompress bytes [N, N+M) only, through that index
  *
  * Same flags as the reference's popt table (7bgzf.c:379-398): -l[N]/--libdeflate[=N] (1-12, default 6),
  * -z -m -s -S -n -C -i -K -T [N] and -Z N (the other method flags: each selects a level for the one GPU codec,
@@ -68,6 +70,7 @@ static void usage(const char *argv0)
             "      --offset=N            (extension, with -d) decompress from byte N of the data on (read --gzi=FILE if given)\n"
             "      --size=M              (extension, with --offset) at most M bytes\n"
             "      --reindex             (extension) write the .gzi of the stream on stdin to --gzi=FILE, nothing to stdout\n"
+            "      --index=FILE          (extension, 7gzip) the checkpoint index: written by --reindex, read by -d --offset (required)\n"
             "      --devices=N           (extension) spread the blocks over N GPUs (contiguous block ranges, same output)\n"
             "      --independent         (extension, 7gzip) pieces without the 16 KiB of history before them: faster, 2-3 %% larger\n"
             "      --primed              (extension, 7migz) pieces of a member see the 32 KiB before them: slower, 2 %% smaller\n"
@@ -472,6 +475,22 @@ static void input_free(struct input_map *im)
     else free(im->p);
 }
 
+/* the whole of an index file */
+static int read_file(const char *path, unsigned char **buf, size_t *len)
+{
+    *buf = NULL;
+    *len = 0;
+    FILE *f = fopen(path, "rb");
+    if (!f) { fprintf(stderr, "cannot read the index %s\n", path); return 1; }
+    size_t cap = 4096;
+    *buf = (unsigned char *)malloc(cap);
+    for (size_t r; *buf && (r = fread(*buf + *len, 1, cap - *len, f)) > 0;)
+        if ((*len += r) == cap) *buf = (unsigned char *)realloc(*buf, cap *= 2);
+    fclose(f);
+    if (!*buf) { fprintf(stderr, "out of memory\n"); return 1; }
+    return 0;
+}
+
 /* (caddr, uaddr) of every member: from a .gzi, or by a header walk of the input */
 static int load_index(const struct input_map *im, const char *gzi_path, uint64_t **c, uint64_t **u, size_t *n)
 {
@@ -479,16 +498,7 @@ static int load_index(const struct input_map *im, const char *gzi_path, uint64_t
     *n = 0;
     unsigned char *buf = NULL;
     size_t len = 0;
-    if (gzi_path) {
-        FILE *f = fopen(gzi_path, "rb");
-        if (!f) { fprintf(stderr, "cannot read the index %s\n", gzi_path); return 1; }
-        size_t cap = 4096;
-        buf = (unsigned char *)malloc(cap);
-        for (size_t r; buf && (r = fread(buf + len, 1, cap - len, f)) > 0;)
-            if ((len += r) == cap) buf = (unsigned char *)realloc(buf, cap *= 2);
-        fclose(f);
-        if (!buf) { fprintf(stderr, "out of memory\n"); return 1; }
-    }
+    if (gzi_path && read_file(gzi_path, &buf, &len)) return 1;
     int r = gzi_path ? b200bgzf_gzi_parse(buf, len, NULL, NULL, 0, n) : b200bgzf_index_host(im->p, im->n, NULL, NULL, 0, n);
     if (r == 0 || r == B200BGZF_E_NOSPACE) {
         *c = (uint64_t *)malloc((*n + 1) * sizeof(uint64_t));
@@ -569,6 +579,73 @@ static int reindex_applet(const char *gzi_path)
     return ret;
 }
 
+static b200bgzf_ctx *applet_ctx(void)
+{
+    b200bgzf_ctx *ctx = NULL;
+    const char *dev = getenv("B200BGZF_DEVICE");
+    const int r = b200bgzf_create(&ctx, dev && *dev ? atoi(dev) : -1);
+    if (r) fprintf(stderr, "b200bgzf: cannot initialise the GPU codec: %s\n", b200bgzf_strerror(r));
+    return r ? NULL : ctx;
+}
+
+/* 7gzip -d --offset=N [--size=M] --index=F: bytes [N, N+M) of a whole-stream gzip member (the decoded size is the index's
+ * out_bytes field, include/b200bgzf.h) */
+static int gzip_range_applet(uint64_t offset, uint64_t size, int have_size, const char *index_path)
+{
+    struct input_map im;
+    if (input_load(&im)) { fprintf(stderr, "cannot read stdin\n"); return 1; }
+    unsigned char *ix = NULL;
+    size_t ixn = 0;
+    uint64_t total = 0;
+    int ret = read_file(index_path, &ix, &ixn);
+    if (!ret && (ixn < 52 || memcmp(ix, "B2GZIX01", 8))) { fprintf(stderr, "%s: not a gzip index\n", index_path); ret = 1; }
+    for (int k = 7; !ret && k >= 0; k--) total = total << 8 | ix[28 + k];
+    if (!ret && offset > total) { fprintf(stderr, "offset %llu is past the end of the data (%llu bytes)\n", (unsigned long long)offset, (unsigned long long)total); ret = 1; }
+    if (!ret) {
+        const uint64_t end = !have_size || size > total - offset ? total : offset + size;
+        b200bgzf_range rg = { offset, end };
+        unsigned char *out = (unsigned char *)malloc(end - offset + 1);
+        b200bgzf_ctx *ctx = out ? applet_ctx() : NULL;
+        size_t got = 0;
+        int r = ctx ? b200bgzf_gzip_inflate_ranges_host(ctx, im.p, im.n, ix, ixn, &rg, 1, out, end - offset + 1, &got, NULL, 0) : B200BGZF_E_ARG;
+        if (r && ctx) fprintf(stderr, "%s: %s\n", index_path, b200bgzf_strerror(r));
+        if (!r && got && fwrite(out, 1, got, stdout) != got) r = 1;
+        ret = r ? 1 : 0;
+        b200bgzf_destroy(ctx);
+        free(out);
+    }
+    free(ix);
+    input_free(&im);
+    return ret;
+}
+
+/* 7gzip --reindex --index=F: the checkpoint index of the member on stdin (span 1 MiB) */
+static int gzip_reindex_applet(const char *index_path)
+{
+    struct input_map im;
+    if (input_load(&im)) { fprintf(stderr, "cannot read stdin\n"); return 1; }
+    b200bgzf_ctx *ctx = applet_ctx();
+    size_t cap = ((size_t)1 << 20) + im.n / 8, need = 0;   /* (a first guess: 32 KiB of window per MiB of output) */
+    unsigned char *ix = (unsigned char *)malloc(cap);
+    int r = !ctx || !ix ? B200BGZF_E_ARG : b200bgzf_gzip_index_host(ctx, im.p, im.n, 0, ix, cap, &need);
+    if (r == B200BGZF_E_NOSPACE) {
+        free(ix);
+        ix = (unsigned char *)malloc(cap = need);
+        r = ix ? b200bgzf_gzip_index_host(ctx, im.p, im.n, 0, ix, cap, &need) : B200BGZF_E_ARG;
+    }
+    if (r && ctx) fprintf(stderr, "cannot index this input: %s\n", b200bgzf_strerror(r));
+    if (!r) {
+        FILE *f = fopen(index_path, "wb");
+        if (!f || fwrite(ix, 1, need, f) != need) r = 1;
+        if (f && fclose(f)) r = 1;
+        if (r) fprintf(stderr, "cannot write the index %s\n", index_path);
+    }
+    b200bgzf_destroy(ctx);
+    free(ix);
+    input_free(&im);
+    return r ? 1 : 0;
+}
+
 int container_applet(const char *name, int kind, int decompress, int level, unsigned param, int ndevices, int nfiles, char **files);   /* applet_containers.c */
 
 static const struct { const char *name; int kind; } k_personas[] = {
@@ -583,7 +660,7 @@ int main(int argc, char **argv)
     int have_offset = 0, have_size = 0, reindex = 0;
     unsigned long long range_offset = 0, range_size = 0;
     unsigned piece_flags = 0;    /* 7gzip --independent: pieces without dictionary priming; 7migz --primed: with it */
-    const char *gzi_path = NULL, *persona = "7bgzf";
+    const char *gzi_path = NULL, *index_path = NULL, *persona = "7bgzf";
     memset(levels, 0, sizeof levels);
     /* allow `cielbox 7bgzf ...` style invocation.  As `7migz` (applet/7migz.c) with -b N <= 63 the same pipeline writes MiGz
      * members of N KiB (one member = one 64 KiB GPU slot); larger members (the reference's default is 512 KiB) and the
@@ -611,6 +688,7 @@ int main(int argc, char **argv)
         { "extreme", no_argument, 0, 'X' },      { "independent", no_argument, 0, 1002 },
         { "primed", no_argument, 0, 1003 },      { "offset", required_argument, 0, 1004 },
         { "size", required_argument, 0, 1005 },  { "reindex", no_argument, 0, 1006 },
+        { "index", required_argument, 0, 1007 },
         { 0, 0, 0, 0 },
     };
     int opt;
@@ -632,6 +710,7 @@ int main(int argc, char **argv)
             continue;
         }
         if (opt == 1006) { reindex = 1; continue; }
+        if (opt == 1007) { index_path = optarg; continue; }
         if (opt == 'h' || opt == '?') { bad = 1; continue; }
         for (size_t k = 0; k < NFLAGS; k++)
             if (k_flags[k].short_opt == opt)
@@ -640,9 +719,11 @@ int main(int argc, char **argv)
     int chosen = -1, nchosen = 0, level_sum = 0;
     for (size_t k = 0; k < NFLAGS; k++)
         if (levels[k]) { chosen = (int)k; nchosen++; level_sum += levels[k]; }
-    /* random access (7bgzf only): -d --offset [--size] [--gzi], and --reindex --gzi */
-    if ((have_offset || have_size || reindex) && !bad) {
-        if (kind || (reindex && (decompress || nchosen || have_offset || have_size || !gzi_path)) ||
+    /* random access: 7bgzf -d --offset [--size] [--gzi], and --reindex --gzi; 7gzip the same with --index (required) */
+    const int gz = kind == B200BGZF_CONTAINER_GZIP;
+    if ((have_offset || have_size || reindex || index_path) && !bad) {
+        if ((kind && !gz) || (gz ? !index_path || gzi_path : index_path != NULL) ||
+            (reindex && (decompress || nchosen || have_offset || have_size || !(gz || gzi_path))) ||
             (!reindex && (!decompress || nchosen || !have_offset))) {
             usage(argv[0]);
             return 1;
@@ -651,6 +732,7 @@ int main(int argc, char **argv)
             usage(argv[0]);
             return -1;
         }
+        if (gz) return reindex ? gzip_reindex_applet(index_path) : gzip_range_applet(range_offset, range_size, have_size, index_path);
         return reindex ? reindex_applet(gzi_path) : range_applet(range_offset, range_size, have_size, gzi_path);
     }
     if (bad || (!decompress && nchosen != 1) || (decompress && nchosen != 0)) {

@@ -304,6 +304,60 @@ int b200bgzf_container_inflate_host(b200bgzf_ctx *ctx, int kind, const void *in,
  */
 int b200bgzf_gzip_inflate_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, void *d_out, size_t out_cap, size_t *out_bytes,
                                  unsigned flags, void *stream);
+
+/*
+ * Random access into one whole-stream gzip member through a checkpoint index (the gzip counterpart of zran / indexed_gzip).
+ * The chunks between the member's flush points, chained as b200bgzf_gzip_inflate_device chains them, are its natural access
+ * points: a decoder can start at a chunk's byte offset with the 32 KiB of output before it.
+ *
+ * b200bgzf_gzip_index_host / _device decode the member (same header handling as b200bgzf_gzip_inflate_device) once and write
+ * its index to host memory `index`.  index NULL or index_cap too small: B200BGZF_E_NOSPACE with *index_bytes = the size
+ * needed (known only once the chain is built: the member is decoded to find it).  Every chained chunk is listed with its
+ * CRC-32; chunk 0 is an access point, and so is every chunk whose output offset is at least `span` past the previous access
+ * point (span 0 = 1 MiB; 0 < span < 32 KiB: B200BGZF_E_ARG).  An access point stores its window, the min(32768, u_off) output
+ * bytes before it.  B200BGZF_E_FORMAT, with nothing more decoded: a chain from the data start that does not reach the
+ * trailer (several members, damage), a chunk of more than 4 MiB of compressed data or over the scratch budget, a reference
+ * before the member start, a decoded size other than ISIZE.  A member without any flush point is indexable as one chunk
+ * when its DEFLATE data is at most 4 MiB.  The same input and span give the same bytes from either variant.
+ *
+ * Index format (public, little endian; "B2GZIX01"):
+ *   offset  0  u8[8]  magic "B2GZIX01"
+ *           8  u64    in_bytes    size of the gzip file                      \
+ *          16  u32    hdr_len     its header length (= the data start)        | bind the index to its file
+ *          20  u32    crc32       trailer CRC-32                              |
+ *          24  u32    isize       trailer ISIZE                              /
+ *          28  u64    out_bytes   decoded size
+ *          36  u32    span
+ *          40  u32    nchunks
+ *          44  u32    npoints
+ *          48  nchunks x { u64 c_start (file offset of the chunk: hdr_len, or right after a 00 00 ff ff); u64 u_off; u32 crc }
+ *              npoints x { u32 chunk; u32 window_len (= min(32768, u_off of that chunk)) }
+ *              the windows, back to back, in point order
+ *              u32    CRC-32 of everything above
+ *
+ * b200bgzf_gzip_inflate_ranges_host / _device decode byte ranges [beg, end) of the member, as b200bgzf_inflate_ranges_* do
+ * for BGZF: the ranges' bytes back to back in the caller's order, range_off[i] (optional) where range i starts; ranges
+ * unsorted, overlapping or empty; beg <= end <= out_bytes, else B200BGZF_E_ARG; out_cap too small (or out NULL with a
+ * non-empty result): B200BGZF_E_NOSPACE with *out_bytes = the size needed, before any decode.  B200BGZF_RANGE_VOFFSET:
+ * B200BGZF_E_ARG.  A damaged index (magic, self-CRC, sizes that do not add up, chunks not ascending) or one of another file
+ * (in_bytes or trailer differ) is B200BGZF_E_FORMAT before any decode.  A range touches the chunks from the access point at or
+ * before its first byte to the chunk of its last byte; overlapping runs are merged and every touched chunk is decoded once
+ * per call, the runs side by side, each behind its window (2 bytes of device scratch per output byte of the runs in flight,
+ * in batches under the budget of b200bgzf_gzip_inflate_device; a longer run is cut at a chunk boundary).  A touched chunk
+ * that fails to decode or decodes to another length: B200BGZF_E_FORMAT; B200BGZF_VERIFY checks every decoded chunk against
+ * its CRC-32 in the index (B200BGZF_E_CRC).  The host variant reads only the compressed bytes of the touched runs and the
+ * trailer (not the header: hdr_len comes from the index).  Synchronises before returning.
+ */
+int b200bgzf_gzip_index_host(b200bgzf_ctx *ctx, const void *in, size_t in_bytes, uint32_t span, void *index, size_t index_cap,
+                             size_t *index_bytes);
+int b200bgzf_gzip_index_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, uint32_t span, void *index, size_t index_cap,
+                               size_t *index_bytes, void *stream);
+int b200bgzf_gzip_inflate_ranges_host(b200bgzf_ctx *ctx, const void *in, size_t in_bytes, const void *index, size_t index_bytes,
+                                      const b200bgzf_range *ranges, size_t nranges, void *out, size_t out_cap, size_t *out_bytes,
+                                      uint64_t *range_off, unsigned flags);
+int b200bgzf_gzip_inflate_ranges_device(b200bgzf_ctx *ctx, const void *d_in, size_t in_bytes, const void *index, size_t index_bytes,
+                                        const b200bgzf_range *ranges, size_t nranges, void *d_out, size_t out_cap, size_t *out_bytes,
+                                        uint64_t *range_off, unsigned flags, void *stream);
 /* decoded size (and number of units) of a container, to size the output: MiGz — and gzip input that turns out to be a
  * stream of members carrying their own size (BGZF, MiGz, mgzip) — by the header walk, the others by their index */
 int b200bgzf_container_inflate_size(int kind, const void *in, size_t in_bytes, size_t *out_bytes, size_t *nunits);
