@@ -19,6 +19,7 @@
 #include <algorithm>
 #include <atomic>
 #include <condition_variable>
+#include <map>
 #include <mutex>
 #include <thread>
 #include <vector>
@@ -1482,6 +1483,10 @@ struct GzChain {
 };
 
 template <typename F>
+int gzip_batches(b200bgzf_ctx *ctx, BgzfGzipArgs a, uint64_t nchunks, uint64_t total, uint32_t want_crc, unsigned flags,
+                 cudaStream_t stream, F on_batch, const uint64_t *bit_end);
+
+template <typename F>
 int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, uint32_t hlen, uint32_t isize, uint32_t want_crc,
                        uint8_t *d_out, size_t out_cap, size_t *total_out, unsigned flags, cudaStream_t stream, F on_batch,
                        GzChain *keep = nullptr)
@@ -1542,6 +1547,17 @@ int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, 
     if ((uint32_t)total != isize) return B200BGZF_E_FORMAT;
     if (total > out_cap || (!d_out && total)) return B200BGZF_E_NOSPACE;
     if (keep) *keep = { a, nchunks };
+    return gzip_batches(ctx, a, nchunks, total, want_crc, flags, stream, on_batch, nullptr);
+}
+
+/* Steps 3 and 4 of both parallel routes: the chained chunks of `a` (c_start, c_len, c_off; nchunks of them, total bytes) are
+ * decoded in batches under the scratch budget, then checked (B200BGZF_VERIFY).  bit_end: NULL for flush-point chunks, else
+ * the searched route's chunk ends (c_start in bits). */
+template <typename F>
+int gzip_batches(b200bgzf_ctx *ctx, BgzfGzipArgs a, uint64_t nchunks, uint64_t total, uint32_t want_crc, unsigned flags,
+                 cudaStream_t stream, F on_batch, const uint64_t *bit_end)
+{
+    GzWork &z = ctx->gz;
     /* 3. batches of chained chunks whose scratch fits the budget */
     const uint64_t win = bgzf_gzip_window(), budget = gzip_budget();
     std::vector<uint64_t> cut;                      /* batch boundaries (chunk indices) */
@@ -1577,7 +1593,7 @@ int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, 
     CK(grow(&z.scratch, &z.scratch_cap, win + most + 16));
     a.scratch = z.scratch;
     for (size_t i = 0; i + 1 < cut.size(); i++) {
-        CK(bgzf_launch_gzip_batch(&a, (uint32_t)cut[i], (uint32_t)cut[i + 1], base[i], base[i + 1] - base[i], stream));
+        CK(bgzf_launch_gzip_batch(&a, (uint32_t)cut[i], (uint32_t)cut[i + 1], base[i], base[i + 1] - base[i], bit_end, stream));
         ctx->launches += BGZF_GZIP_BATCH_LAUNCHES;
         if (int r = on_batch(base[i], base[i + 1] - base[i])) return r;
     }
@@ -1602,7 +1618,7 @@ int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, 
         if (e == cudaSuccess) e = cudaMemcpyAsync(d32, h32.data(), h32.size() * 4, cudaMemcpyHostToDevice, stream);
         BgzfInflateArgs v;
         memset(&v, 0, sizeof v);
-        v.in = d_out;
+        v.in = a.out;
         v.in_off = d64;
         v.out_off = d64 + nu;
         v.hdr_len = d32;
@@ -1611,7 +1627,7 @@ int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, 
         v.status = d32 + 3 * nu;
         v.unit_crc = d32 + 4 * nu;
         v.nblocks = (uint32_t)nu;
-        v.out = d_out;
+        v.out = a.out;
         v.err_flag = a.err + 2;
         v.verify_crc = 1;
         v.crctab = ctx->d_crctab;
@@ -1633,6 +1649,131 @@ int gzip_chain_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, 
         if (crc != want_crc) return B200BGZF_E_CRC;
     }
     return B200BGZF_OK;
+}
+
+constexpr int kGzRepairRounds = 8;   /* searched route: chain repairs before the member goes to one warp */
+
+/* The searched route (DESIGN §6g), for a member whose flush-point chain is unusable: chunk starts at bit offsets proposed by
+ * gz_search_kernel (one per region after the first), a boundary pass from each up to the next proposal, and a chain walk
+ * here from the data start.  A chunk on the walk ends at a true block boundary; when that end is no candidate, it becomes
+ * one, and the boundary pass runs again on the new candidates only.  The chained chunks are the sequential decoder's exact
+ * bit path, decoded by gzip_batches.  Returns BGZF_GZIP_FALLBACK for a member within one region, a chain that breaks (a
+ * failed chunk: an error, a reference before the member start, over the caps) or does not end 8 bytes before the input end,
+ * or more than kGzRepairRounds repairs: the one-warp path then gives the outcome. */
+template <typename F>
+int gzip_search_inflate(b200bgzf_ctx *ctx, const uint8_t *d_in, size_t in_bytes, uint32_t hlen, uint32_t isize, uint32_t want_crc,
+                        uint8_t *d_out, size_t out_cap, size_t *total_out, unsigned flags, cudaStream_t stream, F on_batch)
+{
+    GzWork &z = ctx->gz;
+    const uint64_t data_len = in_bytes - hlen - 8, region = bgzf_gzip_region();
+    const uint64_t nreg = (data_len + region - 1) / region;
+    if (nreg < 2) return BGZF_GZIP_FALLBACK;
+    size_t c32 = z.small32 ? 8 : 0, hc = z.h_cap;
+    CK(grow(&z.small32, &c32, 8));
+    CK(grow(&z.h, &hc, 8, true));
+    z.h_cap = hc;
+    CK(cudaMemsetAsync(z.small32, 0, 8 * sizeof(uint32_t), stream));
+    BgzfGzipArgs a;
+    memset(&a, 0, sizeof a);
+    a.data = d_in + hlen;
+    a.data_len = data_len;
+    a.max_in = kGzMaxChunkIn;
+    a.err = z.small32 + 1;
+    a.out = d_out;
+    /* 1. candidates (bit offsets, ascending): the data start, then what the search proposes */
+    std::vector<uint64_t> cand{ 0 };
+    {
+        CK(grow(&z.u64, &z.u64_cap, nreg));
+        CK(bgzf_launch_gzip_search(&a, (uint32_t)nreg, z.u64, stream));
+        ctx->launches += 1;
+        std::vector<uint64_t> found(nreg - 1);
+        CK(cudaMemcpyAsync(found.data(), z.u64, found.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        for (uint64_t f : found)
+            if (f != ~0ull) cand.push_back(f);
+    }
+    /* 2. rounds of the boundary pass over the new candidates and the walk from the data start */
+    struct Bound {
+        uint64_t end;
+        uint32_t olen, status;
+    };
+    std::map<uint64_t, Bound> bound;              /* every candidate's chunk, by its start */
+    std::vector<uint64_t> todo = cand, chain;
+    for (int round = 0;; round++) {
+        const size_t n = todo.size();
+        CK(grow(&z.u64, &z.u64_cap, 3 * n));
+        CK(grow(&z.u32, &z.u32_cap, 2 * n));
+        std::vector<uint64_t> h64(2 * n);         /* start, stop (the next candidate; none: decode up to the final block) */
+        for (size_t k = 0; k < n; k++) {
+            const auto next = std::upper_bound(cand.begin(), cand.end(), todo[k]);
+            h64[k] = todo[k];
+            h64[n + k] = next == cand.end() ? ~0ull : *next;
+        }
+        a.cand = z.u64;
+        a.end = z.u64 + 2 * n;
+        a.olen = z.u32;
+        a.status = z.u32 + n;
+        CK(cudaMemcpyAsync(z.u64, h64.data(), h64.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+        CK(bgzf_launch_gzip_bit_bound(&a, z.u64 + n, (uint32_t)n, stream));
+        ctx->launches += 1;
+        std::vector<uint64_t> end(n);
+        std::vector<uint32_t> h32(2 * n);
+        CK(cudaMemcpyAsync(end.data(), a.end, n * sizeof(uint64_t), cudaMemcpyDeviceToHost, stream));
+        CK(cudaMemcpyAsync(h32.data(), a.olen, 2 * n * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream));
+        CK(cudaStreamSynchronize(stream));
+        for (size_t k = 0; k < n; k++) bound[todo[k]] = { end[k], h32[k], h32[n + k] };
+        chain.clear();
+        bool done = false;
+        for (uint64_t at = 0;;) {
+            const Bound &c = bound.at(at);
+            if (c.status == GZ_FAIL) return BGZF_GZIP_FALLBACK;
+            chain.push_back(at);
+            if (c.status == GZ_END_FINAL) {
+                if ((c.end + 7) / 8 != data_len) return BGZF_GZIP_FALLBACK;
+                done = true;
+                break;
+            }
+            if (!bound.count(c.end)) break;       /* a true block boundary the search did not propose */
+            at = c.end;
+        }
+        if (done) break;
+        if (round == kGzRepairRounds) return BGZF_GZIP_FALLBACK;
+        /* repair: the unmatched ends of all chunks become candidates (those of chunks from false starts cost a warp each) */
+        todo.clear();
+        for (const auto &kv : bound)
+            if (kv.second.status == GZ_END_FLUSH && !bound.count(kv.second.end)) todo.push_back(kv.second.end);
+        std::sort(todo.begin(), todo.end());
+        todo.erase(std::unique(todo.begin(), todo.end()), todo.end());
+        std::vector<uint64_t> merged(cand.size() + todo.size());
+        std::merge(cand.begin(), cand.end(), todo.begin(), todo.end(), merged.begin());
+        cand.swap(merged);
+    }
+    /* 3. the chained chunks: start and end (bits), output offset and length */
+    const uint64_t nchunks = chain.size();
+    std::vector<uint64_t> h64(3 * nchunks);
+    std::vector<uint32_t> h32(nchunks);
+    uint64_t total = 0;
+    for (uint64_t j = 0; j < nchunks; j++) {
+        const Bound &c = bound.at(chain[j]);
+        h64[j] = chain[j];
+        h64[nchunks + j] = total;
+        h64[2 * nchunks + j] = c.end;
+        h32[j] = c.olen;
+        total += c.olen;
+    }
+    *total_out = (size_t)total;
+    if ((uint32_t)total != isize) return B200BGZF_E_FORMAT;
+    if (total > out_cap || (!d_out && total)) return B200BGZF_E_NOSPACE;
+    CK(grow(&z.u64, &z.u64_cap, 3 * nchunks));
+    CK(grow(&z.u32, &z.u32_cap, 3 * nchunks));
+    a.c_start = z.u64;
+    a.c_off = z.u64 + nchunks;
+    a.c_len = z.u32;
+    a.lastm = z.u32 + nchunks;
+    a.anchor = z.u32 + 2 * nchunks;
+    CK(cudaMemcpyAsync(z.u64, h64.data(), h64.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, stream));
+    CK(cudaMemcpyAsync(z.u32, h32.data(), h32.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    return gzip_batches(ctx, a, nchunks, total, want_crc, flags, stream, on_batch, z.u64 + 2 * nchunks);
 }
 
 /* the checks the one-warp path makes of a member before decoding it (inflate_host_impl): 0 or B200BGZF_E_FORMAT */
@@ -1682,13 +1823,23 @@ extern "C" int b200bgzf_gzip_inflate_device(b200bgzf_ctx *ctx, const void *d_in,
     const uint32_t want_crc = rd32(tr), isize = rd32(tr + 4);
     if ((r = gzip_member_check(in_bytes, (uint32_t)hlen, isize))) return r;
     size_t total = isize;
+    bool batched = false;                   /* (a fallback after the flush-point route decoded a batch goes to one warp) */
+    const auto on_batch = [&](uint64_t, uint64_t) { batched = true; return 0; };
     r = gzip_chain_inflate(ctx, in, in_bytes, (uint32_t)hlen, isize, want_crc, (uint8_t *)d_out, d_out ? out_cap : 0, &total, flags, stream,
-                           [](uint64_t, uint64_t) { return 0; });
+                           on_batch);
     *out_bytes = total;
     if (r != BGZF_GZIP_FALLBACK) return r;
-    /* no usable flush points: one warp decodes the member, as b200bgzf_inflate_units_host does */
     *out_bytes = isize;
     if (isize > out_cap || (!d_out && isize)) return B200BGZF_E_NOSPACE;
+    /* no usable flush points: chunks from a search for block headers, else one warp, as b200bgzf_inflate_units_host decodes */
+    if (!batched) {
+        total = isize;
+        r = gzip_search_inflate(ctx, in, in_bytes, (uint32_t)hlen, isize, want_crc, (uint8_t *)d_out, out_cap, &total, flags, stream,
+                                on_batch);
+        *out_bytes = total;
+        if (r != BGZF_GZIP_FALLBACK) return r;
+        *out_bytes = isize;
+    }
     size_t c64 = z.small64 ? 8 : 0, c32 = z.small32 ? 8 : 0, hc = z.h_cap;
     CK(grow(&z.small64, &c64, 8));
     CK(grow(&z.small32, &c32, 8));
@@ -1746,14 +1897,20 @@ extern "C" int bgzf_gzip_inflate_host(b200bgzf_ctx *ctx, const void *in_, size_t
     CK(grow(&z.d_out, &z.out_cap, (size_t)isize + 64));
     CK(cudaMemcpyAsync(z.d_in, in, in_bytes, cudaMemcpyHostToDevice, l.stream));
     size_t total = isize;
-    r = gzip_chain_inflate(ctx, z.d_in, in_bytes, hlen, isize, want_crc, z.d_out, isize, &total, flags, l.stream,
-                           [&](uint64_t base, uint64_t bytes) -> int {
-                               if (!bytes) return 0;
-                               CK(cudaEventRecord(z.ev, l.stream));
-                               CK(cudaStreamWaitEvent(z.copy, z.ev, 0));
-                               CK(cudaMemcpyAsync((uint8_t *)out + base, z.d_out + base, bytes, cudaMemcpyDeviceToHost, z.copy));
-                               return 0;
-                           });
+    bool batched = false;
+    const auto on_batch = [&](uint64_t base, uint64_t bytes) -> int {
+        batched = true;
+        if (!bytes) return 0;
+        CK(cudaEventRecord(z.ev, l.stream));
+        CK(cudaStreamWaitEvent(z.copy, z.ev, 0));
+        CK(cudaMemcpyAsync((uint8_t *)out + base, z.d_out + base, bytes, cudaMemcpyDeviceToHost, z.copy));
+        return 0;
+    };
+    r = gzip_chain_inflate(ctx, z.d_in, in_bytes, hlen, isize, want_crc, z.d_out, isize, &total, flags, l.stream, on_batch);
+    if (r == BGZF_GZIP_FALLBACK && !batched) {
+        total = isize;
+        r = gzip_search_inflate(ctx, z.d_in, in_bytes, hlen, isize, want_crc, z.d_out, isize, &total, flags, l.stream, on_batch);
+    }
     const cudaError_t e = cudaStreamSynchronize(z.copy);
     if (r == B200BGZF_E_NOSPACE) r = B200BGZF_E_FORMAT;   /* (more output than ISIZE: the one-warp path's overrun) */
     if (r == B200BGZF_OK || r == B200BGZF_E_CRC) *out_bytes = isize;

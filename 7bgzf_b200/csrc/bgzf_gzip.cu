@@ -95,10 +95,6 @@ gz_cand_scan_kernel(const uint8_t *d, uint64_t n, uint32_t *tile_count, const ui
 
 /* ---- decoding one chunk ---- */
 
-#define GZ_END_FLUSH 0u   /* ended right after a non-final empty stored block */
-#define GZ_END_FINAL 1u   /* ended with the final block */
-#define GZ_FAIL 2u        /* not a chunk a sequential decoder could produce without an error (or over the caps) */
-
 struct GzChunk {
     uint64_t end;       /* byte offset (in the DEFLATE data) one past the chunk */
     uint32_t olen;      /* output bytes */
@@ -111,10 +107,12 @@ struct GzChunk {
  * EMIT: writes u16 symbols to out[0..olen) — bytes, or 256 + j for byte j of the 32 KiB before the chunk; abs0 = the chunk's
  * output offset in the member (a reference further back is INF_E_DIST).  Without EMIT only the lengths are counted, and a
  * reference before the chunk is an error only for the chunk at the member start (first).  Reading stops at `lim` (the
- * trailer, or the compressed-length cap): more input is GZ_FAIL, and so is more output than max_out. */
-template <bool EMIT>
+ * trailer, or the compressed-length cap): more input is GZ_FAIL, and so is more output than max_out.
+ * BITS (the searched route): the chunk starts `skip` bits into byte p, ends at the first block boundary at or after bit `stop`
+ * of the DEFLATE data, or with the final block, and c.end is a bit offset; an empty stored block ends nothing. */
+template <bool EMIT, bool BITS = false>
 __device__ GzChunk gz_decode_chunk(InfSmem &sm, const uint8_t *data, const uint8_t *p, const uint8_t *lim, bool first, uint16_t *out,
-                                   uint32_t max_out, uint64_t abs0, uint32_t lane)
+                                   uint32_t max_out, uint64_t abs0, uint32_t lane, uint32_t skip = 0, uint64_t stop = 0)
 {
     GzChunk c;
     c.end = 0;
@@ -126,6 +124,7 @@ __device__ GzChunk gz_decode_chunk(InfSmem &sm, const uint8_t *data, const uint8
     bool fail = false;
     BitReader r;
     br_init(r, p, lim, lane);
+    if (BITS) br_consume(r, skip);
     for (;;) {
         const bool last = br_take(r, 1);
         const uint32_t btype = br_take(r, 2);
@@ -139,7 +138,14 @@ __device__ GzChunk gz_decode_chunk(InfSmem &sm, const uint8_t *data, const uint8
             if (EMIT)
                 for (uint32_t k = lane; k < len; k += 32) out[pos + k] = raw[k];
             pos += len;
-            if (last || len == 0) {
+            if (BITS) {
+                const uint64_t eb = 8ull * (uint64_t)(raw + len - data);
+                if (last || eb >= stop) {
+                    c.end = eb;
+                    c.status = last ? GZ_END_FINAL : GZ_END_FLUSH;
+                    break;
+                }
+            } else if (last || len == 0) {
                 c.end = (uint64_t)(raw + len - data);
                 c.status = last ? GZ_END_FINAL : GZ_END_FLUSH;
                 break;
@@ -235,7 +241,14 @@ __device__ GzChunk gz_decode_chunk(InfSmem &sm, const uint8_t *data, const uint8
         }
         if (fail) break;
         if (br_overrun(r)) { fail = true; break; }
-        if (last) {
+        if (BITS) {
+            const uint64_t eb = 8ull * (uint64_t)((const uint8_t *)r.base - data) + r.wi * 32u + r.bit;
+            if (last || eb >= stop) {
+                c.end = eb;
+                c.status = last ? GZ_END_FINAL : GZ_END_FLUSH;
+                break;
+            }
+        } else if (last) {
             c.end = (uint64_t)((const uint8_t *)r.base - data) + (r.wi * 32u + r.bit + 7u) / 8u;
             c.status = GZ_END_FINAL;
             break;
@@ -327,6 +340,159 @@ gz_marker_kernel(BgzfGzipArgs a, uint32_t j0, uint64_t base)
     if (lane == 0) {
         a.lastm[j] = c.lastm;
         if (c.status == GZ_FAIL || c.olen != a.c_len[j]) atomicOr(a.err, c.dist_err ? 1u : 2u);
+    }
+}
+
+/* ---- members without flush points (DESIGN §6g): chunk starts at bit offsets, found by a search for block headers ----
+ * Region r >= 1 (GZ_REGION compressed bytes each) proposes the first bit offset inside it whose bits read as a dynamic block
+ * header gz_decode_chunk would accept: BTYPE 2, a precode, code lengths and litlen / distance codes that build_table takes, and
+ * a code for end-of-block.  The search only proposes: a missed start merges two regions, a false one costs a repair round of
+ * the host's chain walk.  The boundary and marker passes then decode chunks between bit offsets. */
+#ifndef GZ_REGION
+#define GZ_REGION (256u << 10)
+#endif
+#define GZ_SEARCH_WARPS 4u
+
+/* 32 bits of the stream from bit b of the word-aligned base w (words from nwords on read as zeros) */
+__device__ __forceinline__ uint32_t gz_bits_at(const uint32_t *w, uint32_t nwords, uint64_t b)
+{
+    const uint64_t i = b >> 5;
+    const uint32_t lo = i < nwords ? __ldg(w + i) : 0u, hi = i + 1 < nwords ? __ldg(w + i + 1) : 0u;
+    return __funnelshift_r(lo, hi, (uint32_t)b & 31u);
+}
+
+/* where precode symbol s stands in the header's length list (the inverse of bg_precode_order) */
+__device__ __forceinline__ uint32_t gz_precode_pos(uint32_t s)
+{
+    const uint64_t lo = 3ull | 17ull << 5 | 15ull << 10 | 13ull << 15 | 11ull << 20 | 9ull << 25 | 7ull << 30 | 5ull << 35 |
+                        4ull << 40 | 6ull << 45 | 8ull << 50 | 10ull << 55;
+    const uint64_t hi = 12ull | 14ull << 5 | 16ull << 10 | 18ull << 15 | 0ull << 20 | 1ull << 25 | 2ull << 30;
+    return (uint32_t)((s < 12 ? lo >> (5 * s) : hi >> (5 * (s - 12))) & 31u);
+}
+
+/* one lane: does a dynamic block header the decoder accepts start at bit b?  srt: this lane's 19 bytes of shared memory */
+__device__ bool gz_dynamic_header(const uint32_t *w, uint32_t nwords, uint64_t b, uint8_t *srt)
+{
+    const uint32_t x = gz_bits_at(w, nwords, b);
+    if (((x >> 1) & 3u) != 2u) return false;
+    const uint32_t nl = ((x >> 3) & 31u) + 257, nd = ((x >> 8) & 31u) + 1, np = ((x >> 13) & 15u) + 4;
+    b += 17;
+    const uint64_t pc = ((uint64_t)gz_bits_at(w, nwords, b) | (uint64_t)gz_bits_at(w, nwords, b + 32) << 32) &
+                        ((1ull << (3 * np)) - 1ull);
+    b += 3 * np;
+    /* the precode: complete, or one 1-bit codeword (build_table's rule; an empty one leaves end-of-block without a code) */
+    uint32_t kraft = 0, ncodes = 0;
+    uint64_t cnt = 0;                                   /* 5 bits per length */
+    for (uint32_t i = 0; i < np; i++) {
+        const uint32_t l = (uint32_t)(pc >> (3 * i)) & 7u;
+        if (!l) continue;
+        kraft += 128u >> l;
+        ncodes++;
+        cnt += 1ull << (5 * l);
+    }
+    const bool lone = ncodes == 1 && kraft == 64;
+    if (kraft != 128 && !lone) return false;
+    uint32_t lone_sym = 0;
+    {
+        uint32_t offs[8], at = 0;
+        for (uint32_t l = 1; l <= 7; l++) { offs[l] = at; at += (uint32_t)(cnt >> (5 * l)) & 31u; }
+        for (uint32_t s = 0; s < 19; s++) {
+            const uint32_t i = gz_precode_pos(s);
+            const uint32_t l = i < np ? (uint32_t)(pc >> (3 * i)) & 7u : 0u;
+            if (l) { srt[offs[l]++] = (uint8_t)s; lone_sym = s; }
+        }
+    }
+    /* the code lengths, decoded as gz_decode_chunk does; Kraft sums of the litlen and distance codes on the way */
+    const uint32_t total = nl + nd;
+    uint32_t i = 0, prev = 0, kl = 0, kd = 0, cl = 0, cd = 0, l1 = 0, d1 = 0, eob = 0;
+    while (i < total) {
+        uint32_t v = gz_bits_at(w, nwords, b), sym = lone_sym, nb = 1;
+        if (!lone) {
+            int code = 0, first = 0, index = 0;
+            for (nb = 1; nb <= 7; nb++) {
+                code |= (int)((v >> (nb - 1)) & 1u);
+                const int count = (int)((cnt >> (5 * nb)) & 31u);
+                if (code - count < first) { sym = srt[index + (code - first)]; break; }
+                index += count;
+                first = (first + count) << 1;
+                code <<= 1;
+            }
+        }
+        v >>= nb;
+        uint32_t rep, val, xb = 0;
+        if (sym < 16) { rep = 1; val = sym; prev = sym; }
+        else if (sym == 16) { if (i == 0) return false; xb = 2; rep = 3 + (v & 3u); val = prev; }
+        else if (sym == 17) { xb = 3; rep = 3 + (v & 7u); val = 0; prev = 0; }
+        else { xb = 7; rep = 11 + (v & 127u); val = 0; prev = 0; }
+        b += nb + xb;
+        if (i + rep > total) return false;
+        if (val) {
+            const uint32_t nlit = i < nl ? min(i + rep, nl) - i : 0u, ndist = rep - nlit;
+            kl += nlit << (15 - val);
+            kd += ndist << (15 - val);
+            cl += nlit;
+            cd += ndist;
+            if (val == 1) { l1 += nlit; d1 += ndist; }
+            if (i <= 256 && 256 < i + rep) eob = val;
+            if (kl > (1u << 15) || kd > (1u << 15)) return false;
+        }
+        i += rep;
+    }
+    if (!eob) return false;
+    if (kl != (1u << 15) && !(cl == 1 && l1 == 1)) return false;
+    return kd == (1u << 15) || cd == 0 || (cd == 1 && d1 == 1);
+}
+
+/* one warp per region r >= 1, one lane per bit offset: found[r - 1] = the first accepted offset (bits), or ~0 */
+__global__ void __launch_bounds__(GZ_SEARCH_WARPS * 32)
+gz_search_kernel(const uint8_t *data, uint64_t data_len, uint32_t nreg, uint64_t *found)
+{
+    __shared__ uint8_t srt[GZ_SEARCH_WARPS * 32][20];
+    const uint32_t lane = threadIdx.x & 31u, r = 1 + blockIdx.x * GZ_SEARCH_WARPS + (threadIdx.x >> 5);
+    if (r >= nreg) return;
+    const uint32_t mis = (uint32_t)((uintptr_t)data & 3u);
+    const uint32_t *w = (const uint32_t *)(data - mis);
+    const uint32_t nwords = (uint32_t)((data_len + mis + 3) >> 2);
+    const uint64_t b0 = 8ull * GZ_REGION * r, b1 = min(b0 + 8ull * GZ_REGION, 8ull * data_len);
+    uint64_t hit = ~0ull;
+    for (uint64_t b = b0; b < b1; b += 32) {
+        const bool ok = b + lane < b1 && gz_dynamic_header(w, nwords, 8ull * mis + b + lane, srt[threadIdx.x]);
+        const uint32_t m = __ballot_sync(0xffffffffu, ok);
+        if (m) { hit = b + __ffs(m) - 1; break; }
+    }
+    if (lane == 0) found[r - 1] = hit;
+}
+
+/* gz_bound_kernel between bit offsets: candidate k = cand[k] (bits) decodes up to the first block boundary at or after stop[k] */
+__global__ void __launch_bounds__(32, 32)
+gz_bit_bound_kernel(BgzfGzipArgs a, const uint64_t *stop)
+{
+    __shared__ InfSmem sm;
+    const uint32_t lane = threadIdx.x, k = blockIdx.x;
+    const uint64_t sb = a.cand[k], s = sb >> 3;
+    const uint8_t *lim = a.data + (a.data_len - s > a.max_in ? s + a.max_in : a.data_len);
+    const GzChunk c = gz_decode_chunk<false, true>(sm, a.data, a.data + s, lim, sb == 0, nullptr, GZ_MAX_CHUNK, 0, lane,
+                                                   (uint32_t)(sb & 7u), stop[k]);
+    if (lane == 0) {
+        a.end[k] = c.end;
+        a.olen[k] = c.olen;
+        a.status[k] = c.status;
+    }
+}
+
+/* gz_marker_kernel between bit offsets: chunk j runs from c_start[j] to exactly bit_end[j] */
+__global__ void __launch_bounds__(32, 32)
+gz_bit_marker_kernel(BgzfGzipArgs a, const uint64_t *bit_end, uint32_t j0, uint64_t base)
+{
+    __shared__ InfSmem sm;
+    const uint32_t lane = threadIdx.x, j = j0 + blockIdx.x;
+    const uint64_t sb = a.c_start[j], s = sb >> 3, o = a.c_off[j];
+    const uint8_t *lim = a.data + (a.data_len - s > a.max_in ? s + a.max_in : a.data_len);
+    const GzChunk c = gz_decode_chunk<true, true>(sm, a.data, a.data + s, lim, sb == 0, a.scratch + GZ_WIN + (o - base), a.c_len[j], o,
+                                                  lane, (uint32_t)(sb & 7u), bit_end[j]);
+    if (lane == 0) {
+        a.lastm[j] = c.lastm;
+        if (c.status == GZ_FAIL || c.olen != a.c_len[j] || c.end != bit_end[j]) atomicOr(a.err, c.dist_err ? 1u : 2u);
     }
 }
 
@@ -508,14 +674,31 @@ extern "C" cudaError_t bgzf_launch_gzip_chain(const BgzfGzipArgs *a, uint32_t nc
 }
 
 extern "C" cudaError_t bgzf_launch_gzip_batch(const BgzfGzipArgs *a, uint32_t j0, uint32_t j1, uint64_t base, uint64_t bytes,
-                                              cudaStream_t stream)
+                                              const uint64_t *bit_end, cudaStream_t stream)
 {
     if (j1 <= j0) return cudaSuccess;
     gz_prefix_kernel<<<32, 256, 0, stream>>>(*a, base);
-    gz_marker_kernel<<<j1 - j0, 32, 0, stream>>>(*a, j0, base);
+    if (bit_end) gz_bit_marker_kernel<<<j1 - j0, 32, 0, stream>>>(*a, bit_end, j0, base);
+    else gz_marker_kernel<<<j1 - j0, 32, 0, stream>>>(*a, j0, base);
     gz_anchor_kernel<<<1, 1024, 0, stream>>>(*a, j0, j1, base);
     gz_resolve_kernel<<<j1 - j0, GZ_RESOLVE_THREADS, 0, stream>>>(*a, j0, j1, base);
     const uint64_t threads = (bytes + GZ_NARROW - 1) / GZ_NARROW;
     if (threads) gz_narrow_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, stream>>>(*a, j0, j1, base, bytes);
+    return cudaGetLastError();
+}
+
+extern "C" size_t bgzf_gzip_region(void) { return GZ_REGION; }
+
+extern "C" cudaError_t bgzf_launch_gzip_search(const BgzfGzipArgs *a, uint32_t nreg, uint64_t *found, cudaStream_t stream)
+{
+    if (nreg < 2) return cudaSuccess;
+    gz_search_kernel<<<(nreg - 1 + GZ_SEARCH_WARPS - 1) / GZ_SEARCH_WARPS, GZ_SEARCH_WARPS * 32, 0, stream>>>(a->data, a->data_len, nreg, found);
+    return cudaGetLastError();
+}
+
+extern "C" cudaError_t bgzf_launch_gzip_bit_bound(const BgzfGzipArgs *a, const uint64_t *stop, uint32_t n, cudaStream_t stream)
+{
+    if (n == 0) return cudaSuccess;
+    gz_bit_bound_kernel<<<n, 32, 0, stream>>>(*a, stop);
     return cudaGetLastError();
 }

@@ -7,7 +7,7 @@
 
 #include "../../include/b200bgzf.h"
 
-#define BGZF_GZIP_FALLBACK 100   /* the member has no usable flush-point chain: decode it on one warp */
+#define BGZF_GZIP_FALLBACK 100   /* neither parallel route (flush points, searched block starts) takes the member: decode it on one warp */
 
 #ifdef __cplusplus
 extern "C" {

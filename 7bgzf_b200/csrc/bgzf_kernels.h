@@ -126,6 +126,9 @@ struct BgzfRangeGatherArgs {
 };
 
 /* whole-stream gzip (bgzf_gzip.cu): one member inflated in chunks cut at its byte-aligned flush points (all device memory) */
+#define GZ_END_FLUSH 0u   /* ended right after a non-final empty stored block (searched route: at a block boundary at or after its stop) */
+#define GZ_END_FINAL 1u   /* ended with the final block */
+#define GZ_FAIL 2u        /* not a chunk a sequential decoder could produce without an error (or over the caps) */
 struct BgzfGzipArgs {
     const uint8_t *data;       /* the member's DEFLATE data (after the header) */
     uint64_t data_len;         /* its bytes up to the 8-byte trailer */
@@ -181,7 +184,15 @@ size_t bgzf_gzip_tiles(uint64_t data_len);
 size_t bgzf_gzip_window(void);
 cudaError_t bgzf_launch_gzip_count(const BgzfGzipArgs *a, cudaStream_t stream);    /* counts[0] = flush points found */
 cudaError_t bgzf_launch_gzip_chain(const BgzfGzipArgs *a, uint32_t ncand, cudaStream_t stream);
-cudaError_t bgzf_launch_gzip_batch(const BgzfGzipArgs *a, uint32_t j0, uint32_t j1, uint64_t base, uint64_t bytes, cudaStream_t stream);
+/* bit_end: NULL for flush-point chunks (c_start in bytes); else c_start and bit_end[j] are the bit offsets of the searched route */
+cudaError_t bgzf_launch_gzip_batch(const BgzfGzipArgs *a, uint32_t j0, uint32_t j1, uint64_t base, uint64_t bytes,
+                                   const uint64_t *bit_end, cudaStream_t stream);
+/* members without flush points (DESIGN §6g): region size of the search (bytes); found[r - 1] = the proposed chunk start of
+ * region r in bits (~0: none), r = 1 .. nreg - 1; the boundary pass over cand[0, n) (bits), each up to the first block
+ * boundary at or after stop[k], into end (bits), olen and status */
+size_t bgzf_gzip_region(void);
+cudaError_t bgzf_launch_gzip_search(const BgzfGzipArgs *a, uint32_t nreg, uint64_t *found, cudaStream_t stream);
+cudaError_t bgzf_launch_gzip_bit_bound(const BgzfGzipArgs *a, const uint64_t *stop, uint32_t n, cudaStream_t stream);
 cudaError_t bgzf_launch_gzip_runs(const BgzfGzipArgs *a, const BgzfGzipRunArgs *r, uint64_t bytes, cudaStream_t stream);
 #define BGZF_GZIP_CHAIN_LAUNCHES 8
 #define BGZF_GZIP_BATCH_LAUNCHES 5

@@ -278,8 +278,9 @@ int b200bgzf_multi_container_compress_host(b200bgzf_multi *m, int kind, uint32_t
 /* The readers: the unit list of a dictzip / RAZF / GZinga file from its own index (a plain gzip member without an index is
  * one unit spanning the input), to be released with b200bgzf_units_free; out_bytes = the decoded size.  No GPU involved.
  * b200bgzf_container_inflate_host = that list + b200bgzf_inflate_units_host (MiGz: b200bgzf_inflate_host, whose header
- * walk knows the "MZ" subfield; GZIP: the member goes through b200bgzf_gzip_inflate_device's chunked decode, and only a
- * member without a usable flush point is decoded by one warp, as the unit list says). */
+ * walk knows the "MZ" subfield; GZIP: the member goes through b200bgzf_gzip_inflate_device's chunked decode, cut at its flush
+ * points or, without usable ones, at block starts found by a search; only a member neither route takes is decoded by one
+ * warp, as the unit list says). */
 int b200bgzf_container_units(int kind, const void *in, size_t in_bytes, b200bgzf_unit **units, size_t *nunits, size_t *out_bytes);
 void b200bgzf_units_free(b200bgzf_unit *units);
 int b200bgzf_container_inflate_host(b200bgzf_ctx *ctx, int kind, const void *in, size_t in_bytes, void *out, size_t out_cap,
@@ -289,10 +290,14 @@ int b200bgzf_container_inflate_host(b200bgzf_ctx *ctx, int kind, const void *in,
  * decoded into d_out.  Every block that follows a byte-aligned flush point — the empty stored block (00 00 ff ff) that our GZIP
  * writer puts after every piece, that pigz puts after every chunk and that zlib's Z_SYNC_FLUSH / Z_FULL_FLUSH write — starts a
  * chunk; the chunks are decoded side by side (one warp each) and their back-references across chunk starts resolved after.
- * The chunks are accepted only when they chain from the data start to the trailer exactly as a sequential decoder walks them;
- * otherwise (no flush point, a chunk of more than 4 MiB of compressed data or one whose output alone is over the scratch
- * budget, a stream that does not end at the trailer, e.g. several members) one warp decodes the member, as
- * b200bgzf_inflate_units_host does.  Either way the bytes, or the error, are those of that one-warp decode.
+ * The chunks are accepted only when they chain from the data start to the trailer exactly as a sequential decoder walks them.
+ * A member without such a chain (no flush point — GNU gzip, zlib's default deflate(), Python's gzip —, a chain that breaks,
+ * a chunk over the caps) whose DEFLATE data spans more than 256 KiB is cut instead at DEFLATE block starts at bit offsets:
+ * a search proposes one per 256 KiB of compressed data, decoding from the data start confirms or repairs them, and the
+ * confirmed chunks are decoded side by side as above.  A member neither route takes (a chunk of more than 4 MiB of
+ * compressed data or one whose output alone is over the scratch budget, a stream that does not end at the trailer, e.g.
+ * several members, more than 8 repairs) is decoded by one warp, as b200bgzf_inflate_units_host does.  Whatever the route,
+ * the bytes, or the error, are those of that one-warp decode.
  *   Output   *out_bytes = the decoded size; out_cap too small (or d_out NULL with a non-empty result): B200BGZF_E_NOSPACE with
  *            *out_bytes = the size needed, before anything is decoded.  The decoded size must equal ISIZE (mod 2^32), else
  *            B200BGZF_E_FORMAT.
